@@ -6,7 +6,7 @@ One step = k-mer counting (k=6) of every genome into 4^k frequency rows + Shanno
 followed by the order-preserving nmost (n=100) selection over the shuffled record order.
 Metric = whole-step throughput in Gbp/s (bases consumed / step time).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 N>1 is launched by torchrun (one rank per GPU); each rank counts its own 10.5k-genome shard (weak
 scaling) and pushes its frequency rows to every peer over NVLink while it is still counting; the nmost
@@ -17,6 +17,8 @@ runs the reference's -np semantics instead (select per GPU, final_nmost merge of
 `value` times the step with inputs already in HBM; `e2e` times the same step through
 the public host-buffer API (pinned host -> device copy + result read-back inside the timed region).
 `--impl reference` times the CPU restatement of the reference (oracle/) on the host cores.
+`--dump-outputs DIR` writes what the last timed step returned to its caller as DIR/<name>.npy (see
+dump_outputs); the inputs depend on the arguments alone, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -64,7 +66,14 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-ctree", action="store_true", help="skip the ctree pairs/s side measurements (N=1 only)")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="target wall time of one CPU sample")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step as DIR/<name>.npy (float64, < 64 MB in all)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs is not None and a.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
+    return a
 
 
 def workload_config(a, world):
@@ -429,6 +438,34 @@ def side_metrics(a, ctx, comm, rank, world, device, barrier, hbm_peak):
     kf12.close(); ss.close()
     return out
 
+
+# ------------------------------------------------------------------------ --dump-outputs ----
+DUMP_ROWS = 512              # frequency rows in the seeded sample ...
+DUMP_FREQ_BYTES = 16 << 20   # ... and their size at most (columns are sampled too when rows are wider)
+
+
+def dump_outputs(out_dir, kf, idx, delta, stats):
+    """What one step hands its caller, as float64 .npy files: the selection (`selected_indices` in Vec order,
+    `delta_jsd`, `selection_stats` = total_jsd, mean, std and cov of delta_jsd, summed entropies) and, of the
+    frequency rows it leaves on the device, every record's `entropies` and `valid` flag plus `freqs_sample`,
+    the rows `freqs_sample_rows` x columns `freqs_sample_cols` drawn with a fixed seed."""
+    out = pathlib.Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    nrec, dim = kf.nrec, kf.dim
+    rng = np.random.default_rng(SEED)
+    rows = np.sort(rng.choice(nrec, size=min(nrec, DUMP_ROWS), replace=False))
+    ncols = min(dim, DUMP_FREQ_BYTES // (8 * max(rows.size, 1)))
+    cols = np.arange(dim) if ncols == dim else np.sort(rng.choice(dim, size=ncols, replace=False))
+    sample = np.empty((rows.size, cols.size), dtype=np.float64)
+    for i, r in enumerate(rows):
+        sample[i] = kf.download(int(r), 1, counts=False)[1][0, cols]
+    _, _, ent, valid = kf.download(counts=False, freqs=False)
+    arrays = {"selected_indices": idx, "delta_jsd": delta, "selection_stats": stats, "entropies": ent, "valid": valid,
+              "freqs_sample": sample, "freqs_sample_rows": rows, "freqs_sample_cols": cols}
+    for name, arr in arrays.items():
+        np.save(out / f"{name}.npy", np.asarray(arr, dtype=np.float64))
+
+
 # ------------------------------------------------------------------------ B200 leg ----
 _REAL_STDOUT = None
 
@@ -494,21 +531,28 @@ def main():
         torch.cuda.synchronize(device)
 
     phase = {}
+    kept = []  # the frequency rows of a step run with keep=True (--dump-outputs: the last timed step)
 
-    def step(ss):
+    def release(kf, keep):
+        if keep:
+            kept.append(kf)
+        else:
+            kf.close()
+
+    def step(ss, keep=False):
         t0 = time.perf_counter()
         if world > 1 and a.multi == "sharded":
             kf, _ = shard.count_sharded(ctx, comm, ss, a.k)
             t1 = time.perf_counter()
             idx, delta, stats = shard.select_sharded(ctx, comm, kf, order, _lib.MODE_NMOST, a.n)
-            kf.close()
+            release(kf, keep)
         else:
             if world == 1 and a.overlap == "on":
                 # counting with the nmost rounds trailing it (dvs_count_select): one call, two streams
                 kf, idx, delta, stats = _lib.KFreqs.count_select(ctx, ss, a.k, order, _lib.MODE_NMOST, a.n, a.n,
                                                                  chunks=a.chunks)
                 t1 = time.perf_counter()
-                kf.close()
+                release(kf, keep)
                 phase["trail_accepts"] = int(ctx._lib.dvs_select_last_trail_accepts(ctx.handle))
                 phase["count_ms"] = ctx.phase_ms(_lib.PHASE_COUNT_LAUNCHES)  # the counting launches alone, summed
                 phase["count_region_ms"] = ctx.phase_ms(_lib.PHASE_COUNT_KERNEL)  # first launch .. last entropy launch
@@ -523,6 +567,7 @@ def main():
                 idx = np.array([r * a.nrec + i for r, i in idx], dtype=np.uint32)
             else:
                 idx, delta, stats = kf.select(order, _lib.MODE_NMOST, a.n)
+            release(kf, keep)
         t3 = time.perf_counter()
         phase["count_ms"] = ctx.phase_ms(_lib.PHASE_COUNT_KERNEL)
         phase["freq_entropy_ms"] = ctx.phase_ms(_lib.PHASE_FREQ_ENTROPY)
@@ -555,13 +600,17 @@ def main():
     count_ms, fe_ms, sel_ms = [], [], []
 
     def step_resident():
-        r = step(seqset)
+        r = step(seqset, keep=a.dump_outputs is not None and len(count_ms) == a.steps - 1)
         count_ms.append(phase["count_ms"]); fe_ms.append(phase["freq_entropy_ms"]); sel_ms.append(phase["select_ms"])
         return r
 
     ms_step, (idx, delta, stats) = timed(step_resident, a.steps)
     launches = ctx.launch_count - launches0  # kernels of libdvs_b200.so launched inside the timed region (all K steps)
     accepts = int(ctx._lib.dvs_select_last_accepts(ctx.handle))
+    if kept:  # before any further step: the peer window of the sharded path holds the rows of one step only
+        if rank == 0:
+            dump_outputs(a.dump_outputs, kept[0], idx, delta, stats)
+        kept.pop().close()
     # NVML sometimes answers only once or twice inside a 70 ms timed region: keep the load on with further identical
     # (untimed) steps until the sampler has a usable number of readings; every rank runs the same number of steps
     in_region = len(sampler.samples) if rank == 0 else 0
