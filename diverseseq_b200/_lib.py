@@ -21,6 +21,7 @@ PHASE_PREP = 7
 PHASE_CLUSTER = 8
 PHASE_SPARSE = 9
 PHASE_COUNT_LAUNCHES = 10
+PHASE_EUCLID_SPARSE = 11
 
 _vp = C.c_void_p
 _u32, _u64, _i32, _f64 = C.c_uint32, C.c_uint64, C.c_int, C.c_double
@@ -69,6 +70,7 @@ SIGNATURES = {
     "dvs_ksparse_stats": (_i32, [_vp, _vp, _vp, _vp, _vp, _vp]),
     "dvs_ksparse_download": (_i32, [_vp, _vp, _u32, _vp, _vp, _u64, C.POINTER(_u64)]),
     "dvs_ksparse_free": (None, [_vp]),
+    "dvs_euclid_distances_sparse": (_i32, [_vp, _vp, _u32, _u32, _vp]),
     "dvs_select": (_i32, [_vp, _vp, _vp, _u32, _i32, _u32, _u32, _vp, _vp, _vp, C.POINTER(_u32)]),
     "dvs_count_select": (_i32, [_vp, _vp, _i32, _i32, _vp, _u32, _i32, _u32, _u32, _u32, C.POINTER(_vp), _vp, _vp, _vp,
                                 C.POINTER(_u32)]),
@@ -110,6 +112,7 @@ SIGNATURES = {
     "dvs_debug_log2": (_i32, [_vp, _vp, _vp, _u64]),
     "dvs_debug_fast_terms": (_i32, [_vp, _vp, _vp, _vp, _vp, _vp, _u64]),
     "dvs_debug_entropy": (_i32, [_vp, _vp, _u32, _u64, _vp, _vp]),
+    "dvs_debug_euclid_sparse_pairs": (_i32, [_vp, _vp, _vp, _u32, _vp]),
 }
 
 _lib = None
@@ -600,6 +603,27 @@ class KSparse(_Handle):
             check(self.ctx._lib.dvs_ksparse_download(self.ctx.handle, self.handle, int(rec), ptr(idx), ptr(cnt), n.value,
                                                      C.byref(n)))
         return idx, cnt
+
+    def euclidean(self, row_begin: int = 0, row_end: int | None = None) -> np.ndarray:
+        """rows [row_begin, row_end) of the Euclidean distance matrix of the frequency rows (dvs_euclid_distances_sparse)"""
+        row_end = self.nrec if row_end is None else row_end
+        out = np.zeros((max(row_end - row_begin, 0), self.nrec), dtype=np.float64)
+        check(self.ctx._lib.dvs_euclid_distances_sparse(self.ctx.handle, self.handle, row_begin, row_end, ptr(out)))
+        return out
+
+    def euclidean_into(self, device_ptr: int, row_begin: int = 0, row_end: int | None = None) -> None:
+        """same matrix written to device memory at `device_ptr` ((row_end-row_begin) x nrec f64)"""
+        row_end = self.nrec if row_end is None else row_end
+        check(self.ctx._lib.dvs_euclid_distances_sparse(self.ctx.handle, self.handle, row_begin, row_end,
+                                                        _vp(device_ptr)))
+
+    def debug_euclid_pairs(self, pairs) -> np.ndarray:
+        """difference-form distances of the given (a, b) record pairs (dvs_debug_euclid_sparse_pairs)"""
+        pairs = np.ascontiguousarray(pairs, dtype=np.uint32).reshape(-1, 2)
+        out = np.zeros(pairs.shape[0], dtype=np.float64)
+        check(self.ctx._lib.dvs_debug_euclid_sparse_pairs(self.ctx.handle, self.handle, ptr(pairs) if pairs.size else None,
+                                                          pairs.shape[0], ptr(out)))
+        return out
 
 
 class Comm:

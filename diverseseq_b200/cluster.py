@@ -17,6 +17,7 @@ from collections.abc import Sequence
 import numpy as np
 
 from . import _lib
+from .distance import counts_sparse_for_euclidean
 
 
 class ClusterTree:
@@ -111,6 +112,8 @@ class dvs_ctree:
         if self._distance_mode == "mash":
             sk = _lib.Sketches.sketch(ctx, ss, self._k, int(self._sketch_size), self._num_states, self._mash_canonical)
             sk.distances_into(dmat.ptr, self._k, int(self._sketch_size))
+        elif counts_sparse_for_euclidean(self._k, self._num_states):
+            _lib.KSparse.count(ctx, ss, self._k, self._num_states).euclidean_into(dmat.ptr)
         else:
             kf = _lib.KFreqs.count(ctx, ss, self._k, self._num_states)
             kf.euclidean_into(dmat.ptr)

@@ -28,11 +28,10 @@
 
 #include "common.cuh"
 #include "entropy.cuh"
+#include "sparse.cuh"
 
 namespace dvs {
 
-constexpr int kSpLowBits = 12;
-constexpr uint32_t kSpLowBins = 1u << kSpLowBits;
 constexpr uint32_t kSpItemBytes = 32768;  // <= 32768 k-mers per item: u16 item histograms cannot overflow
 constexpr int kSpThreads = 1024;
 constexpr int kSpBucketThreads = 256;
@@ -543,22 +542,6 @@ k_sp_compact(const uint32_t* __restrict__ out_idx, const uint32_t* __restrict__ 
 }  // namespace dvs
 
 using namespace dvs;
-
-struct dvs_ksparse {
-    int device = 0;
-    uint32_t nrec = 0, nb = 0;
-    int k = 0;
-    uint64_t dim = 0, slots = 0;
-    bool has_entropy = false;
-    std::vector<uint64_t> h_offsets;   // record base (slot index) = byte offset of the record
-    DevBuf<uint64_t> offsets;          // the same on the device
-    DevBuf<uint32_t> idx, cnt;         // [slots] bucket-major, ascending index inside a record, count 0 = no entry
-    DevBuf<uint32_t> bucket_ptr;       // [nrec][nb + 1] first slot of each bucket inside the record's region
-    DevBuf<uint32_t> bucket_nnz;       // [nrec][nb] entries in use
-    DevBuf<uint64_t> totals, nnz;      // [nrec] valid k-mers, distinct k-mers
-    DevBuf<double> entropy, err_total; // [nrec]
-    DevBuf<uint8_t> valid, err;        // [nrec]
-};
 
 extern "C" {
 

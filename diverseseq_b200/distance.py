@@ -66,11 +66,23 @@ def mash_distances(seq_arrays, k: int, sketch_size: int, num_states: int, *, mas
     return NamedDistances.from_array_names(dist, [s.seqid for s in seq_arrays])
 
 
+def counts_sparse_for_euclidean(k: int, num_states: int) -> bool:
+    """Whether the Euclidean matrix is formed from sparse k-mer rows (dvs_count_kmers_sparse +
+    dvs_euclid_distances_sparse) instead of dense frequency rows: for DNA at 10 <= k <= 12, where a dense row
+    takes 4^k x 12 bytes and a pair 2 x 4^k flops.  At k = 9 the dense rows (3 MB) were measured ahead on
+    4 Mbp genomes (13 against 18 ms for 256 of them, DESIGN.md §5.11) and stay."""
+    return num_states == 4 and 10 <= k <= 12
+
+
 def euclidean_distances(seq_arrays, k: int, moltype: str = "dna", *, progress=None) -> NamedDistances:
     num_states = seq_arrays[0].num_states if len(seq_arrays) and hasattr(seq_arrays[0], "num_states") else 4
     ctx = _lib.default_context()
-    kf = _lib.KFreqs.count(ctx, _seqset(ctx, seq_arrays), k, num_states)
-    return NamedDistances.from_array_names(kf.euclidean(), [s.seqid for s in seq_arrays])
+    ss = _seqset(ctx, seq_arrays)
+    if counts_sparse_for_euclidean(k, num_states):
+        dist = _lib.KSparse.count(ctx, ss, k, num_states).euclidean()
+    else:
+        dist = _lib.KFreqs.count(ctx, ss, k, num_states).euclidean()
+    return NamedDistances.from_array_names(dist, [s.seqid for s in seq_arrays])
 
 
 def euclidean_distance(freq_1: np.ndarray, freq_2: np.ndarray) -> float:

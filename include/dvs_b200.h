@@ -78,6 +78,7 @@ uint64_t dvs_ctx_launch_count(dvs_ctx* ctx);
 #define DVS_PHASE_SPARSE 9         /* the partition passes of one dvs_count_kmers_sparse (without the optional entropies) */
 #define DVS_PHASE_COUNT_LAUNCHES 10 /* chunked counting (sharded / dvs_count_select): sum of the counting launches alone */
 #define DVS_PHASE_PREP 7           /* all device work of one dvs_prep_fasta (k_prep x2 + k_prep_carry) */
+#define DVS_PHASE_EUCLID_SPARSE 11 /* all device work of one dvs_euclid_distances_sparse (without the output copy) */
 /* bytes that actually crossed PCIe during the last dvs_seqset_upload (2-bit packed + exceptions for
  * large uploads, see csrc/upload.cu; equal to the input size for the plain copy) */
 uint64_t dvs_ctx_last_upload_wire_bytes(dvs_ctx* ctx);
@@ -172,6 +173,14 @@ int dvs_ksparse_stats(dvs_ctx* ctx, const dvs_ksparse* sp, uint64_t* nnz, uint64
 int dvs_ksparse_download(dvs_ctx* ctx, const dvs_ksparse* sp, uint32_t rec, uint32_t* idx, uint32_t* cnt, uint64_t cap,
                          uint64_t* nnz_out);
 void dvs_ksparse_free(dvs_ksparse* sp);
+/* euclidean_distances over the sparse rows: the matrix dvs_euclid_distances gives for the dense rows of the same
+ * records (1e-9 relative; NaN for pairs with a record without valid k-mers, zero diagonal), rows
+ * [row_begin,row_end) x all columns, `dist` host or device memory; every pair is bit-identical whatever the row
+ * range.  A pair costs one product per k-mer both records hold (exact integer Gram form, DESIGN.md §5.11); the
+ * pairs that form cannot give to 1e-9 of the reference's rounded frequencies are recomputed in difference form
+ * (their number: dvs_euclid_last_fallback_pairs).  A matrix that does not fit the free device memory is refused
+ * with DVS_ERR_ARG: ask for fewer rows per call. */
+int dvs_euclid_distances_sparse(dvs_ctx* ctx, const dvs_ksparse* sp, uint32_t row_begin, uint32_t row_end, double* dist);
 
 /* ---- nmost / max selection ------------------------------------------------------------------
  * select_nmost_divergent / select_max_divergent and their *_final forms (src/records.rs:311-507)
@@ -240,7 +249,8 @@ int dvs_mash_sketch_host(dvs_ctx* ctx, const uint8_t* seq, uint64_t len, int k, 
  * frequency rows, rows [row_begin,row_end) x all columns, zero diagonal; `dist` may be host or device memory. */
 int dvs_euclid_distances(dvs_ctx* ctx, const dvs_kfreqs* f, uint32_t row_begin, uint32_t row_end, double* dist);
 /* pairs that the Gram-form kernel of the last dvs_euclid_distances(_sharded) on this ctx handed to the
- * difference form because |a|^2 + |b|^2 - 2 a.b would have cancelled too many digits (near-duplicate rows) */
+ * difference form because |a|^2 + |b|^2 - 2 a.b would have cancelled too many digits (near-duplicate rows);
+ * after dvs_euclid_distances_sparse, the pairs its difference-form kernel recomputed */
 uint32_t dvs_euclid_last_fallback_pairs(dvs_ctx* ctx);
 
 /* ---- `dvs ctree` tail: average-linkage tree of a precomputed distance matrix -----------------
@@ -340,6 +350,9 @@ int dvs_debug_fast_terms(dvs_ctx* ctx, const double* a, const double* b, double*
 /* exact (reference-order) entropy of each host row on the device; err[r]=1 when the reference
  * would panic (sum check, src/record.rs:101-104) */
 int dvs_debug_entropy(dvs_ctx* ctx, const double* rows, uint32_t nrec, uint64_t dim, double* out, uint8_t* err);
+/* the difference-form kernel of dvs_euclid_distances_sparse on the given pairs (pairs[2 p], pairs[2 p + 1]) of sp's
+ * records: out[p] = sum over the union of the two rows of (fl(c_a/T_a) - fl(c_b/T_b))^2, square-rooted */
+int dvs_debug_euclid_sparse_pairs(dvs_ctx* ctx, const dvs_ksparse* sp, const uint32_t* pairs, uint32_t n, double* out);
 
 #ifdef __cplusplus
 }
