@@ -566,6 +566,11 @@ class KFreqs(_Handle):
         row_end = self.nrec if row_end is None else row_end
         check(self.ctx._lib.dvs_euclid_distances(self.ctx.handle, self.handle, row_begin, row_end, _vp(device_ptr)))
 
+    def fallback_pairs(self) -> int:
+        """pairs that the last Euclidean call on this context took from the Gram form's list and recomputed in
+        difference form (dvs_euclid_last_fallback_pairs); 0 when the difference-form tile kernel did the whole call"""
+        return int(self.ctx._lib.dvs_euclid_last_fallback_pairs(self.ctx.handle))
+
 
 class KSparse(_Handle):
     """Sparse (index, count) k-mer rows for 9 <= k <= 12 (dvs_ksparse)."""

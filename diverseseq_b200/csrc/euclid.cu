@@ -57,9 +57,11 @@ k_euclid_tiles(const double* __restrict__ F, uint64_t dim, uint32_t n, uint32_t 
     }
     const uint32_t i0 = row_begin + ti * kEuT, j0 = tj * kEuT;
     if (i0 >= row_end) return;
-    // a tile strictly above the diagonal whose transpose is also produced by this launch is skipped
-    // (tiles of rows and columns only coincide when row_begin is tile aligned)
-    const bool mirror_in_range = (row_begin % kEuT == 0) && (j0 >= row_begin) && (j0 < row_end);
+    // a tile strictly above the diagonal is skipped when its transpose, produced by this launch, mirrors every entry
+    // of it: tiles of rows and columns only coincide when row_begin is tile aligned, and the transpose stores rows
+    // < row_end only, so all of the tile's columns j0 .. j0+127 must be rows of the call (or lie past n)
+    const bool mirror_in_range =
+        (row_begin % kEuT == 0) && (j0 >= row_begin) && (j0 + kEuT <= row_end || row_end == n);
     if (mirror_in_range && j0 > i0) return;
     const int t = threadIdx.x, tx = t & 15, ty = t >> 4;
     // loader mapping: a slab row segment is 16 doubles = one 128-byte line; chunk = 16 bytes (2 columns).
@@ -184,7 +186,9 @@ constexpr size_t kEuSmemBytes = 4ull * kEuK * (kEuT + kEuPad) * sizeof(double);
 // range or GPU, so partial-range calls, single-GPU and sharded calls return identical bits.
 constexpr int kEgT = 128, kEgSlab = 16, kEgStride = 20, kEgStages = 3, kEgThreads = 512;
 constexpr uint32_t kEgSlice = 2048;
-constexpr double kEgTau = 5e-4;  // >= 2 * (2048 + 64 + 16 + 8) * 1.11e-16 / 1e-9
+// relative error of a Gram-form d^2 <= (kEgSlice + #slices + log2 D + 8) u / kEgTau, of d half that: 2.3e-10 at
+// 32 slices (k=8), 2.9e-10 at 512 (D = 2^20), below 0.5e-9 up to about 2,400 slices (D ~ 4.9 M)
+constexpr double kEgTau = 5e-4;
 constexpr size_t kEgSmemBytes = (size_t)kEgStages * 2 * kEgT * kEgStride * sizeof(double);
 
 struct EgTile {
@@ -489,9 +493,10 @@ extern "C" int dvs_euclid_distances_sharded(dvs_ctx* ctx, dvs_comm* c, const dvs
         for (int r = 0; r < c->world; ++r) outs.p[r] = reinterpret_cast<double*>(c->peer[(c->rank + r) % c->world] + hoff);
         outs.count = c->world;
         PhaseTimer pt(ctx, DVS_PHASE_EUCLID);
-        // Gram form on this GPU's share of the lower-triangle tiles (t = rank, rank + world, ...); every rank must
-        // take the same decision, so the fallback to the difference form is decided per call by the data-independent
-        // checks only (row length, workspace) - a rank with many near-duplicate pairs lists them all
+        // Gram form on this GPU's share of the lower-triangle tiles (t = rank, rank + world, ...).  Each rank decides
+        // on its own whether to fall back to the difference form: row length and workspace are the same everywhere,
+        // but a rank whose list overflows runs the tile kernel over exactly its own tiles while the other ranks keep
+        // their Gram results, so the ranks need not agree
         bool fell_back = true;
         {
             std::vector<EgTile> my_tiles;
