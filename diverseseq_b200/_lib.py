@@ -622,6 +622,12 @@ class KSparse(_Handle):
         check(self.ctx._lib.dvs_euclid_distances_sparse(self.ctx.handle, self.handle, row_begin, row_end,
                                                         _vp(device_ptr)))
 
+    def fallback_pairs(self) -> int:
+        """pairs that the last Euclidean call on this context listed for the difference form
+        (dvs_euclid_last_fallback_pairs): 0 when the exact integer form gave every pair; after a list overflow, the
+        number of pairs that overflowed the list"""
+        return int(self.ctx._lib.dvs_euclid_last_fallback_pairs(self.ctx.handle))
+
     def debug_euclid_pairs(self, pairs) -> np.ndarray:
         """difference-form distances of the given (a, b) record pairs (dvs_debug_euclid_sparse_pairs)"""
         pairs = np.ascontiguousarray(pairs, dtype=np.uint32).reshape(-1, 2)

@@ -274,6 +274,8 @@ using namespace dvs;
 
 extern "C" int dvs_euclid_distances_sparse(dvs_ctx* ctx, const dvs_ksparse* sp, uint32_t row_begin, uint32_t row_end,
                                            double* dist) {
+    // the counter describes this call whatever its outcome; after a list overflow it holds the overflowing count
+    if (ctx) ctx->last_euclid_fallback_pairs = 0;
     if (!ctx || !sp || !dist || row_begin > row_end || row_end > sp->nrec) {
         set_error("dvs_euclid_distances_sparse: bad argument");
         return DVS_ERR_ARG;
@@ -349,6 +351,7 @@ extern "C" int dvs_euclid_distances_sparse(dvs_ctx* ctx, const dvs_ksparse* sp, 
     uint32_t h_cnt = 0;
     DVS_CUDA_TRY(cudaMemcpyAsync(&h_cnt, d_cnt.p, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
     DVS_CUDA_TRY(cudaStreamSynchronize(st));
+    ctx->last_euclid_fallback_pairs = h_cnt;
     if (h_cnt > flag_cap) {
         set_error("dvs_euclid_distances_sparse: %u pairs need the difference form, more than the %u one call can list; "
                   "ask for fewer rows at a time", h_cnt, flag_cap);
@@ -356,7 +359,6 @@ extern "C" int dvs_euclid_distances_sparse(dvs_ctx* ctx, const dvs_ksparse* sp, 
     }
     if (h_cnt) DVS_TRY(xs_launch_pairs(ctx, sp, d_flag.p, d_cnt.p, h_cnt, row_begin, row_end, out, nullptr));
     pt.stop();
-    ctx->last_euclid_fallback_pairs = h_cnt;
     if (!on_device)
         DVS_CUDA_TRY(cudaMemcpyAsync(dist, out, nrows * n * sizeof(double), cudaMemcpyDeviceToHost, st));
     DVS_CUDA_TRY(cudaStreamSynchronize(st));

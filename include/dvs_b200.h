@@ -250,7 +250,8 @@ int dvs_mash_sketch_host(dvs_ctx* ctx, const uint8_t* seq, uint64_t len, int k, 
 int dvs_euclid_distances(dvs_ctx* ctx, const dvs_kfreqs* f, uint32_t row_begin, uint32_t row_end, double* dist);
 /* pairs that the Gram-form kernel of the last dvs_euclid_distances(_sharded) on this ctx handed to the
  * difference form because |a|^2 + |b|^2 - 2 a.b would have cancelled too many digits (near-duplicate rows);
- * after dvs_euclid_distances_sparse, the pairs its difference-form kernel recomputed */
+ * after dvs_euclid_distances_sparse, the pairs it listed for its difference-form kernel (0 after an argument
+ * error or an empty range; after a list overflow, the number of pairs that overflowed the list) */
 uint32_t dvs_euclid_last_fallback_pairs(dvs_ctx* ctx);
 
 /* ---- `dvs ctree` tail: average-linkage tree of a precomputed distance matrix -----------------
