@@ -22,6 +22,7 @@ PHASE_CLUSTER = 8
 PHASE_SPARSE = 9
 PHASE_COUNT_LAUNCHES = 10
 PHASE_EUCLID_SPARSE = 11
+PHASE_EUCLID_SPARSE_ROWS = 12
 
 _vp = C.c_void_p
 _u32, _u64, _i32, _f64 = C.c_uint32, C.c_uint64, C.c_int, C.c_double
@@ -107,6 +108,7 @@ SIGNATURES = {
     "dvs_sketches_allgather": (_i32, [_vp, _vp, _vp, _vp, _u32, C.POINTER(_vp)]),
     "dvs_mash_distances_sharded": (_i32, [_vp, _vp, _vp, _i32, _u64, _vp]),
     "dvs_euclid_distances_sharded": (_i32, [_vp, _vp, _vp, _vp]),
+    "dvs_euclid_distances_sparse_sharded": (_i32, [_vp, _vp, _vp, _vp, _vp]),
     "dvs_select_sharded": (_i32, [_vp, _vp, _vp, _vp, _u32, _i32, _u32, _u32, _vp, _vp, _vp, C.POINTER(_u32)]),
     "dvs_debug_pack_host": (_i32, [_vp, _u64, _vp, _vp, _vp, _u32, C.POINTER(_u32)]),
     "dvs_debug_log2": (_i32, [_vp, _vp, _vp, _u64]),
@@ -622,10 +624,21 @@ class KSparse(_Handle):
         check(self.ctx._lib.dvs_euclid_distances_sparse(self.ctx.handle, self.handle, row_begin, row_end,
                                                         _vp(device_ptr)))
 
+    def euclidean_sharded(self, comm: "Comm", nrec_per_rank, device_ptr: int | None = None):
+        """whole matrix over the sparse rows of all ranks, each rank passing its own rows (collective,
+        dvs_euclid_distances_sparse_sharded); into device memory at `device_ptr` when given (returns None)"""
+        npr = np.ascontiguousarray(nrec_per_rank, dtype=np.uint32)
+        assert npr.size == comm.world
+        n = int(npr.sum())
+        out = None if device_ptr is not None else np.zeros((n, n), dtype=np.float64)
+        check(self.ctx._lib.dvs_euclid_distances_sparse_sharded(
+            self.ctx.handle, comm.handle, self.handle, ptr(npr), _vp(device_ptr) if device_ptr is not None else ptr(out)))
+        return out
+
     def fallback_pairs(self) -> int:
         """pairs that the last Euclidean call on this context listed for the difference form
         (dvs_euclid_last_fallback_pairs): 0 when the exact integer form gave every pair; after a list overflow, the
-        number of pairs that overflowed the list"""
+        number of pairs that overflowed the list.  After `euclidean_sharded`: the pairs this rank listed"""
         return int(self.ctx._lib.dvs_euclid_last_fallback_pairs(self.ctx.handle))
 
     def debug_euclid_pairs(self, pairs) -> np.ndarray:

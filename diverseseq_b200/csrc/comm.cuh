@@ -57,6 +57,14 @@ struct dvs_comm {
 };
 
 namespace dvs {
+// where a distance kernel's results go: one matrix (plain call) or the same place in the matrix of every GPU
+// (the *_sharded Euclidean calls: each kernel stores its results straight into every peer's window - compute and
+// all-gather in one kernel)
+struct EuOuts {
+    double* p[kCommMaxWorld];
+    int count;
+};
+
 // symmetric heap: every rank must call these in the same order with the same sizes
 int comm_heap_alloc(dvs_comm* c, uint64_t bytes, uint64_t* off);
 void comm_heap_free(dvs_comm* c, uint64_t off);

@@ -94,7 +94,7 @@ struct DevBuf {
 
 }  // namespace dvs
 
-constexpr int kNumPhases = 12;
+constexpr int kNumPhases = 13;
 
 struct dvs_ctx {
     int device = 0;
@@ -120,6 +120,7 @@ struct dvs_ctx {
     uint32_t last_exact_evals = 0;  // exact re-evaluations forced by the fast path's error bound
     uint64_t last_upload_wire_bytes = 0;
     uint32_t last_euclid_fallback_pairs = 0;  // pairs the Gram-form Euclid kernel handed to the difference form
+    double euclid_rows_ms = -1.0;  // peer row copies of the last dvs_euclid_distances_sparse_sharded (timing on)
     void* upload_stage = nullptr;  // pinned/device staging ring of the packed upload path (upload.cu)
     // pinned scratch for small device->host readbacks
     void* pinned = nullptr;

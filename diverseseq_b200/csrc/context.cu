@@ -137,6 +137,7 @@ double dvs_ctx_phase_ms(dvs_ctx* ctx, int phase) {
         }
         return sum;
     }
+    if (phase == DVS_PHASE_EUCLID_SPARSE_ROWS) return ctx->timing ? ctx->euclid_rows_ms : -1.0;  // (a sum)
     if (phase < 0 || phase >= kNumPhases || !ctx->ev_valid[phase]) return -1.0;
     if (cudaEventSynchronize(ctx->ev_stop[phase]) != cudaSuccess) return -1.0;
     float ms = -1.0f;

@@ -29,14 +29,6 @@ constexpr int kEuT = 128;  // tile edge (pairs)
 constexpr int kEuK = 16;   // columns per slab
 constexpr int kEuPad = 2;  // row padding of the [col][row] slabs (doubles)
 
-// where a tile's distances go: one matrix (plain call) or the same place in the matrix of every GPU
-// (dvs_euclid_distances_sharded: the tiles of the lower triangle are dealt over the GPUs and each kernel
-// stores its results straight into every peer's window - compute and all-gather in one kernel)
-struct EuOuts {
-    double* p[kCommMaxWorld];
-    int count;
-};
-
 // SHARDED: blockIdx.x enumerates this GPU's tiles t = tile_first + tile_step * blockIdx.x of the lower
 // triangle (t = ti (ti + 1) / 2 + tj, tj <= ti) of the whole n x n matrix
 template <bool SHARDED>

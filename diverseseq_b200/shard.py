@@ -11,7 +11,8 @@ library's own peer windows (include/dvs_b200.h, dvs_comm_*): no NCCL and no torc
   a different result by design) for callers that want to reproduce numprocs > 1 outputs.
 * distance matrices: sketches / rows are all-gathered, the lower triangle is dealt over the GPUs (pairs for
   mash, 128 x 128 tiles for Euclid) and every kernel stores its results straight into every peer's copy
-  of the matrix.
+  of the matrix.  Sparse k-mer rows (k = 9..12) are not gathered: each rank keeps its own and copies one peer's
+  at a time (`sharded_euclidean_sparse`).
 
 The only host-side exchange is the rendezvous below (window handles and a few integers over TCP on
 MASTER_ADDR:MASTER_PORT+1, or in-process for ranks that are threads of one process).
@@ -173,6 +174,22 @@ def window_bytes_for(nrec_total: int, dim: int, extra: int = 0) -> int:
     return int(nrec_total * (dim * 8 + 64) + extra + (64 << 20))
 
 
+def window_bytes_for_sparse(nrec_per_rank, bases_per_rank, k: int, extra: int = 0) -> int:
+    """the window `sharded_euclidean_sparse` needs (the formula dvs_euclid_distances_sparse_sharded checks): the
+    staged sparse rows of the largest shard - one slot per sequence byte, so known before counting; none on a single
+    rank - and the n x n matrix, plus `extra` bytes of other objects"""
+    def align(b):
+        return (int(b) + 255) // 256 * 256
+    nb = 4 ** (int(k) - 6)  # buckets per record (csrc/sparse.cu)
+    max_n = max((int(x) for x in nrec_per_rank), default=0)
+    max_slots = max((int(x) for x in bases_per_rank), default=0)
+    n = sum(int(x) for x in nrec_per_rank)
+    stage = (2 * align(max_slots * 4) + align((max_n + 1) * 8) + align(max_n * (nb + 1) * 4) + align(max_n * nb * 4)
+             + align(max_n * 8))
+    stage = max(stage, 256) if len(nrec_per_rank) > 1 else 0  # one rank stages nothing: no peer reads its rows
+    return 64 * 1024 + stage + max(align(n * n * 8), 256) + int(extra)
+
+
 # --------------------------------------------------------------------------------- counting ----
 def count_sharded(ctx, comm, seqset_local, k: int, num_states: int = 4):
     """(kfreqs with the rows of ALL ranks in rank-major order, records per rank)"""
@@ -239,6 +256,15 @@ def sharded_mash_distances(ctx, comm, seqset_local, k: int, sketch_size: int, nu
     allsk.close()
     sk.close()
     return out
+
+
+def sharded_euclidean_sparse(ctx, comm, ks_local, device_ptr: int | None = None):
+    """ctree Euclidean at 9 <= k <= 12 on N GPUs from each rank's own sparse rows (KSparse.count of its records):
+    the rows stay with their rank, a rank copies one peer's rows at a time and computes the pairs it owns, results
+    are stored into every peer's matrix; returns the full matrix (rank-major record order) on every rank, or writes
+    it to `device_ptr` (the window: `window_bytes_for_sparse`)"""
+    nrec = comm.rv.allgather(int(ks_local.nrec))
+    return ks_local.euclidean_sharded(comm, nrec, device_ptr)
 
 
 def sharded_euclidean(ctx, comm, kf_local=None, kf_all=None) -> np.ndarray:

@@ -78,7 +78,9 @@ uint64_t dvs_ctx_launch_count(dvs_ctx* ctx);
 #define DVS_PHASE_SPARSE 9         /* the partition passes of one dvs_count_kmers_sparse (without the optional entropies) */
 #define DVS_PHASE_COUNT_LAUNCHES 10 /* chunked counting (sharded / dvs_count_select): sum of the counting launches alone */
 #define DVS_PHASE_PREP 7           /* all device work of one dvs_prep_fasta (k_prep x2 + k_prep_carry) */
-#define DVS_PHASE_EUCLID_SPARSE 11 /* all device work of one dvs_euclid_distances_sparse (without the output copy) */
+#define DVS_PHASE_EUCLID_SPARSE 11 /* all device work of one dvs_euclid_distances_sparse (without the output copy);
+                                      * of dvs_euclid_distances_sparse_sharded: this rank's blocks, row copies included */
+#define DVS_PHASE_EUCLID_SPARSE_ROWS 12 /* dvs_euclid_distances_sparse_sharded: the copies of peer rows, summed */
 /* bytes that actually crossed PCIe during the last dvs_seqset_upload (2-bit packed + exceptions for
  * large uploads, see csrc/upload.cu; equal to the input size for the plain copy) */
 uint64_t dvs_ctx_last_upload_wire_bytes(dvs_ctx* ctx);
@@ -251,7 +253,9 @@ int dvs_euclid_distances(dvs_ctx* ctx, const dvs_kfreqs* f, uint32_t row_begin, 
 /* pairs that the Gram-form kernel of the last dvs_euclid_distances(_sharded) on this ctx handed to the
  * difference form because |a|^2 + |b|^2 - 2 a.b would have cancelled too many digits (near-duplicate rows);
  * after dvs_euclid_distances_sparse, the pairs it listed for its difference-form kernel (0 after an argument
- * error or an empty range; after a list overflow, the number of pairs that overflowed the list) */
+ * error or an empty range; after a list overflow, the number of pairs that overflowed the list); after
+ * dvs_euclid_distances_sparse_sharded, the pairs THIS rank listed over all of its blocks (reset on entry; after a
+ * list overflow on this rank, the overflowing count) */
 uint32_t dvs_euclid_last_fallback_pairs(dvs_ctx* ctx);
 
 /* ---- `dvs ctree` tail: average-linkage tree of a precomputed distance matrix -----------------
@@ -319,6 +323,21 @@ int dvs_sketches_allgather(dvs_ctx* ctx, dvs_comm* c, const dvs_sketches* local,
 int dvs_mash_distances_sharded(dvs_ctx* ctx, dvs_comm* c, const dvs_sketches* sk_all, int k, uint64_t sketch_size,
                                double* dist);
 int dvs_euclid_distances_sharded(dvs_ctx* ctx, dvs_comm* c, const dvs_kfreqs* f_all, double* dist);
+/* euclidean_distances over the sparse rows of ALL ranks.  Collective.  Each rank passes ITS OWN
+ * dvs_count_kmers_sparse result; the rows never leave their rank except one peer's at a time.
+ * nrec_per_rank[world] = records of every rank.  dist: n x n f64 (n = sum), host or device memory.
+ * Every rank receives the whole matrix in rank-major record order.  It is bit-identical to
+ * dvs_euclid_distances_sparse over the union of the records.
+ * Each rank stages its rows in its window and computes the pairs it owns: its own lower triangle, and at step
+ * d = 1 .. world/2 the pairs with rank (rank + d) % world, whose rows it copies into device memory of its own (at
+ * d = world/2 the two ranks split that block by the lower rank's first ceil(n/2) records); every distance is stored
+ * into every rank's matrix.  The window must hold the staged rows of the largest shard and the matrix
+ * (shard.window_bytes_for_sparse; a single rank stages nothing).  Every rank returns the same status: a different k
+ * on some rank or an nrec_per_rank that disagrees with any rank's records is DVS_ERR_ARG, a difference-form list
+ * overflow on any rank (more than 2^24 listed pairs on one rank) DVS_ERR_VALUE; when ranks fail differently, all return
+ * the worst class (DVS_ERR_CUDA before DVS_ERR_ARG before DVS_ERR_VALUE). */
+int dvs_euclid_distances_sparse_sharded(dvs_ctx* ctx, dvs_comm* c, const dvs_ksparse* local,
+                                        const uint32_t* nrec_per_rank, double* dist);
 int dvs_select_sharded(dvs_ctx* ctx, dvs_comm* c, const dvs_kfreqs* f_all, const uint32_t* order, uint32_t num,
                        int mode, uint32_t min_size, uint32_t max_size, uint32_t* sel_idx, double* sel_delta,
                        double* stats5, uint32_t* size_out);
