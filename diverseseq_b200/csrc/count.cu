@@ -133,13 +133,13 @@ __device__ __forceinline__ uint32_t pack16p(uint4 v) {
     return __byte_perm(lo, hi, 0x7610);
 }
 
-// SCR: bank scrambling.  The bank of a bin is its low 5 index bits = the last 2.5 bases, whose
-// distribution is as skewed as the genome's composition, so ATOMS bank conflicts grow with the skew
-// (ncu: 4.9 wavefronts per instruction on the benchmark set vs 2.6 for uniform bins).  Storing bin
+// Bank scrambling of the shared-memory tables.  The bank of a bin is its low 5 index bits = the last 2.5
+// bases, whose distribution is as skewed as the genome's composition, so ATOMS bank conflicts grow with the
+// skew (ncu: 4.9 wavefronts per instruction on the benchmark set vs 2.6 for uniform bins).  Storing bin
 // `idx` at slot `idx ^ (idx >> 5)` (a bijection) folds the next 2.5 bases into the bank bits.
 __device__ __forceinline__ uint32_t scr_word(uint32_t idx) { return idx ^ (idx >> 5); }
 
-template <int MODE, bool SCR, int THREADS>
+template <int MODE, int THREADS>
 __global__ void __launch_bounds__(THREADS)
 k_count(const uint8_t* __restrict__ seqs, const uint64_t* __restrict__ offsets, const CountWork* __restrict__ work,
         uint32_t nwork, uint32_t* __restrict__ next_item, int k, uint64_t dim, uint32_t part_bins,
@@ -175,13 +175,13 @@ k_count(const uint8_t* __restrict__ seqs, const uint64_t* __restrict__ offsets, 
         // idx4 = 4 * bin: one k-mer (MODE 0/1/2) or one (k+1)-mer (MODE 3)
         auto bump4 = [&](uint32_t idx4) {
             if (MODE == MODE_SMEM || MODE == MODE_SUPER) {
-                if (SCR) idx4 ^= (idx4 >> 5) & ~3u;
+                idx4 ^= (idx4 >> 5) & ~3u;
                 atomicAdd(reinterpret_cast<uint32_t*>(hist_b + idx4), 1u);
             } else if (MODE == MODE_SMEM_PARTS) {
                 // branch-free: bins of the other part wrap to huge offsets and are clamped onto one
                 // dummy word behind the table (same-address ATOMS are merged by the hardware)
                 uint32_t local4 = idx4 - (part_base << 2);
-                if (SCR) local4 ^= (local4 >> 5) & ~3u;  // (garbage for foreign bins, clamped next)
+                local4 ^= (local4 >> 5) & ~3u;  // (garbage for foreign bins, clamped next)
                 local4 = min(local4, part_bins << 2);
                 atomicAdd(reinterpret_cast<uint32_t*>(hist_b + local4), 1u);
             } else {
@@ -294,18 +294,18 @@ k_count(const uint8_t* __restrict__ seqs, const uint64_t* __restrict__ offsets, 
 #pragma unroll
                     for (uint32_t b = 0; b < 4; ++b) {  // x is the prefix k-mer
                         const uint32_t y = (x << 2) | b;
-                        c += hist[SCR ? scr_word(y) : y];
+                        c += hist[scr_word(y)];
                     }
 #pragma unroll
                     for (uint32_t a4 = 0; a4 < 4; ++a4) {  // x is the suffix k-mer
                         const uint32_t y = (a4 << (2 * k)) | x;
-                        c += hist[SCR ? scr_word(y) : y];
+                        c += hist[scr_word(y)];
                     }
                     if (c) atomicAdd(&grow[x], c);
                 }
             } else {
                 for (uint32_t i = tid; i < part_bins; i += THREADS) {
-                    uint32_t c = hist[SCR ? scr_word(i) : i];
+                    uint32_t c = hist[scr_word(i)];
                     if (c && (uint64_t)part_base + i < dim) atomicAdd(&grow[part_base + i], c);
                 }
             }
@@ -339,16 +339,13 @@ __device__ __forceinline__ uint32_t pack16w(uint32_t x, uint32_t y, uint32_t z, 
     return pack16p(make_uint4(x, y, z, w));
 }
 
-template <bool SCR, int THREADS, int PF>
-__device__ __forceinline__ void
-count_s3_body(const uint8_t* __restrict__ seqs, const uint64_t* __restrict__ offsets, const CountWork* __restrict__ work,
+template <int THREADS, int PF>
+__global__ void __launch_bounds__(THREADS, 1)
+k_count_s3(const uint8_t* __restrict__ seqs, const uint64_t* __restrict__ offsets, const CountWork* __restrict__ work,
            uint32_t nwork, uint32_t* __restrict__ next_item, int k, uint64_t dim, uint32_t* __restrict__ counts,
-           CountWork* __restrict__ retry, uint32_t* __restrict__ retry_count, uint32_t* resident) {
+           CountWork* __restrict__ retry, uint32_t* __restrict__ retry_count) {
     extern __shared__ uint32_t hist[];  // [4^(k+2) / 2] packed halves, then side[4^k]
     __shared__ uint32_t s_item, s_sum, s_inc;
-    // dvs_count_select: how many counting CTAs are resident right now (the trailing selection kernel is launched
-    // when every SM holds one, so that exactly one of its CTAs fits beside each)
-    if (resident && threadIdx.x == 0) atomicAdd(resident, 1u);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     constexpr int kWarps = THREADS / 32;
     constexpr uint32_t kFull = 0xffffffffu, kStep = 1024u;
@@ -383,9 +380,7 @@ count_s3_body(const uint8_t* __restrict__ seqs, const uint64_t* __restrict__ off
         uint32_t n_fast = 0;  // fast 16-base blocks of this thread: 5 (k+2)-mer increments each
         // v = (k+2)-mer << 1 with garbage above bit 2kk: byte offset of its counter word in bits [2kk:2], half in bit 1
         auto bump_v = [&](uint32_t v) {
-            uint32_t off = v & offmask;
-            if (SCR) off ^= (off >> 5) & ~3u;
-            atomicAdd(reinterpret_cast<uint32_t*>(hist_b + off), (v & 2u) ? 0x10000u : 1u);
+            atomicAdd(reinterpret_cast<uint32_t*>(hist_b + (v & offmask)), (v & 2u) ? 0x10000u : 1u);
         };
         // the five (k+2)-mers ending at block positions 2, 5, 8, 11, 14 and the k-mer ending at position 15
         auto fast_block = [&](uint32_t pc, uint32_t pp) {
@@ -481,12 +476,11 @@ count_s3_body(const uint8_t* __restrict__ seqs, const uint64_t* __restrict__ off
         __syncthreads();
         // fold: cnt[x] = side[x] + sum of the (k+2)-mers that hold x at offset 0, 1 or 2
         uint32_t pre_sum = 0;
-        auto word_at = [&](uint32_t wd) { return hist[SCR ? (wd ^ (wd >> 5)) : wd]; };
         for (uint32_t x = tid; x < (uint32_t)dim; x += THREADS) {
             uint32_t c = side[x], pre = 0;
 #pragma unroll
             for (uint32_t t = 0; t < 8; ++t) {  // x first: y = x * 16 + (0..15) = 8 whole words
-                const uint32_t v = word_at((x << 3) | t);
+                const uint32_t v = hist[(x << 3) | t];
                 pre += (v & 0xFFFFu) + (v >> 16);
             }
             c += pre;
@@ -495,13 +489,13 @@ count_s3_body(const uint8_t* __restrict__ seqs, const uint64_t* __restrict__ off
             for (uint32_t a4 = 0; a4 < 4; ++a4) {  // x in the middle: y = a | x | b
 #pragma unroll
                 for (uint32_t t = 0; t < 2; ++t) {
-                    const uint32_t v = word_at((a4 << (2 * k + 1)) | (x << 1) | t);
+                    const uint32_t v = hist[(a4 << (2 * k + 1)) | (x << 1) | t];
                     c += (v & 0xFFFFu) + (v >> 16);
                 }
             }
 #pragma unroll
             for (uint32_t t = 0; t < 16; ++t) {  // x last: y = t * 4^k + x
-                const uint32_t v = word_at((t << (2 * k - 1)) | (x >> 1));
+                const uint32_t v = hist[(t << (2 * k - 1)) | (x >> 1)];
                 c += (x & 1u) ? (v >> 16) : (v & 0xFFFFu);
             }
             side[x] = c;  // thread-private slot until the overflow check has passed
@@ -527,25 +521,6 @@ count_s3_body(const uint8_t* __restrict__ seqs, const uint64_t* __restrict__ off
         }
         __syncthreads();  // s_item / hist reuse
     }
-    if (resident && threadIdx.x == 0) atomicSub(resident, 1u);
-}
-
-template <bool SCR, int THREADS, int PF>
-__global__ void __launch_bounds__(THREADS, 1)
-k_count_s3(const uint8_t* __restrict__ seqs, const uint64_t* __restrict__ offsets, const CountWork* __restrict__ work,
-           uint32_t nwork, uint32_t* __restrict__ next_item, int k, uint64_t dim, uint32_t* __restrict__ counts,
-           CountWork* __restrict__ retry, uint32_t* __restrict__ retry_count) {
-    count_s3_body<SCR, THREADS, PF>(seqs, offsets, work, nwork, next_item, k, dim, counts, retry, retry_count, nullptr);
-}
-// the form dvs_count_select launches: 1,024 threads x 56 registers leave 8,192 registers - one CTA of the trailing
-// selection kernel - free on the SM
-template <int MAXR>
-__global__ void __maxnreg__(MAXR)
-k_count_s3_trail(const uint8_t* __restrict__ seqs, const uint64_t* __restrict__ offsets,
-                 const CountWork* __restrict__ work, uint32_t nwork, uint32_t* __restrict__ next_item, int k,
-                 uint64_t dim, uint32_t* __restrict__ counts, CountWork* __restrict__ retry,
-                 uint32_t* __restrict__ retry_count, uint32_t* resident) {
-    count_s3_body<false, 1024, 2>(seqs, offsets, work, nwork, next_item, k, dim, counts, retry, retry_count, resident);
 }
 
 // one block per record: total, validity, frequency row, exact entropy
@@ -688,9 +663,6 @@ struct CountDest {
     // optional: the sequence in which the records are counted (a permutation of 0..nrec-1; chunk c covers
     // rec_seq[rb..re)) - dvs_count_select counts in the selection's examination order so that the rounds can trail
     const uint32_t* rec_seq = nullptr;
-    int s3_shape = -1;  // >= 0 overrides DVS_COUNT_S3_SHAPE (the trailing selection needs the 56-register form)
-    uint32_t* resident = nullptr;  // device word: k_count_s3 CTAs resident right now
-    int trail_regs = 56;           // register cap of the counting kernel beside the trailing selection
     const uint32_t* weights = nullptr;  // [chunks] relative chunk sizes (NULL: equal)
 };
 
@@ -740,10 +712,6 @@ static int count_core(dvs_ctx* ctx, const dvs_seqset* s, int k, int num_states, 
         }
     }
     const bool smem = (mode != MODE_GLOBAL);
-    // bank scrambling needs a power-of-two table (always true for num_states == 4); DVS_COUNT_SCRAMBLE=0
-    // turns it off for A/B measurements
-    const char* scr_env = getenv("DVS_COUNT_SCRAMBLE");
-    const bool scramble = !(scr_env && scr_env[0] == '0');
 
     // ---- work list: (record, part, aligned range) ----
     int ctas_per_sm = 4;
@@ -874,42 +842,18 @@ static int count_core(dvs_ctx* ctx, const dvs_seqset* s, int k, int num_states, 
                 e = smem ? launch_generic(k_count_generic<true>) : launch_generic(k_count_generic<false>);
             else if (mode == MODE_SUPER3) {
                 // main pass + retry pass (items whose 16-bit halves overflowed, recounted with 32-bit counters).
-                // The 8-mer table spreads over 32,768 words: bank scrambling costs two instructions per atomic
-                // and buys nothing here unless asked for (DVS_COUNT_SCRAMBLE=1)
-                const bool scr3 = scr_env && scr_env[0] == '1';
-                // DVS_COUNT_S3_SHAPE (A/B measurements): 0 = 1024 threads x 3 KB-steps in flight per warp (8.78 ms on
-                // the bench set), 1 = 1024 threads x 2 steps (8.97 ms), 2 = 512 threads x 4 steps (9.03 ms)
-                const char* shape_env = getenv("DVS_COUNT_S3_SHAPE");
-                const int shape = dst.s3_shape >= 0 ? dst.s3_shape : (shape_env ? atoi(shape_env) : 0);
-                auto s3 = scr3 ? k_count_s3<true, 1024, 2>
-                               : (shape == 1 ? k_count_s3<false, 1024, 2>
-                                             : (shape == 2 ? k_count_s3<false, 512, 4> : k_count_s3<false, 1024, 3>));
-                const int s3_threads = (!scr3 && shape == 2) ? 512 : 1024;
-                auto rk = scramble ? k_count<MODE_SUPER, true, 512> : k_count<MODE_SUPER, false, 512>;
-                // DVS_COUNT_SMEM_PAD (A/B measurements): extra dynamic shared memory, i.e. a smaller L1 for the
-                // in-flight loads - what a co-resident kernel's shared memory costs the counting
-                const char* pad_env = getenv("DVS_COUNT_SMEM_PAD");
-                const size_t s3_bytes = hist_bytes + (pad_env ? (size_t)atoi(pad_env) : 0);
-                TRY_F(cudaFuncSetAttribute(s3, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s3_bytes));
+                // The 8-mer table spreads over 32,768 words: bank scrambling would cost two instructions per atomic
+                // and buy nothing here.  1024 threads x 3 KB-steps in flight per warp (8.78 ms on the bench set;
+                // 2 steps 8.97 ms, 512 threads x 4 steps 9.03 ms)
+                auto s3 = k_count_s3<1024, 3>;
+                auto rk = k_count<MODE_SUPER, 512>;
+                TRY_F(cudaFuncSetAttribute(s3, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hist_bytes));
                 const size_t retry_bytes = (size_t)dim * 20;
                 if (retry_bytes > 48 * 1024)
                     TRY_F(cudaFuncSetAttribute(rk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)retry_bytes));
                 uint32_t* rc2 = d_rc.p + 2 * ch;
-                if (dst.resident) {
-                    auto k_count_s3_trail = dst.trail_regs <= 40 ? dvs::k_count_s3_trail<40>
-                                            : (dst.trail_regs <= 48 ? dvs::k_count_s3_trail<48> : dvs::k_count_s3_trail<56>);
-                    TRY_F(cudaFuncSetAttribute(k_count_s3_trail, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s3_bytes));
-                    // the SM's shared-memory / L1 split cannot change while a CTA is resident: ask for the largest
-                    // split up front, or no selection CTA ever fits beside this one (tools/microbench/coresident.cu,
-                    // profiles/r2_coresident.txt); costs the counting ~3 % (28 KB of L1 for the loads in flight)
-                    TRY_F(cudaFuncSetAttribute(k_count_s3_trail, cudaFuncAttributePreferredSharedMemoryCarveout,
-                                               (int)cudaSharedmemCarveoutMaxShared));
-                    k_count_s3_trail<<<g, 1024, s3_bytes, st>>>(s->data(), s->offsets.p, d_work, n_work, d_nx, k, dim,
-                                                                d_counts, d_retry.p + ib, rc2, dst.resident);
-                } else {
-                    s3<<<g, s3_threads, s3_bytes, st>>>(s->data(), s->offsets.p, d_work, n_work, d_nx, k, dim, d_counts,
-                                                        d_retry.p + ib, rc2);
-                }
+                s3<<<g, 1024, hist_bytes, st>>>(s->data(), s->offsets.p, d_work, n_work, d_nx, k, dim, d_counts,
+                                                d_retry.p + ib, rc2);
                 ctx->launches++;
                 e = cudaGetLastError();
                 if (e == cudaSuccess) {
@@ -920,13 +864,13 @@ static int count_core(dvs_ctx* ctx, const dvs_seqset* s, int k, int num_states, 
                     e = cudaGetLastError();
                 }
             } else if (mode == MODE_SUPER)
-                e = scramble ? launch4(k_count<MODE_SUPER, true, 512>) : launch4(k_count<MODE_SUPER, false, 512>);
+                e = launch4(k_count<MODE_SUPER, 512>);
             else if (mode == MODE_SMEM)
-                e = scramble ? launch4(k_count<MODE_SMEM, true, 512>) : launch4(k_count<MODE_SMEM, false, 512>);
+                e = launch4(k_count<MODE_SMEM, 512>);
             else if (mode == MODE_SMEM_PARTS)  // one 128 KB CTA per SM: 1024 threads keep 32 warps resident
-                e = scramble ? launch4(k_count<MODE_SMEM_PARTS, true, 1024>) : launch4(k_count<MODE_SMEM_PARTS, false, 1024>);
+                e = launch4(k_count<MODE_SMEM_PARTS, 1024>);
             else
-                e = launch4(k_count<MODE_GLOBAL, false, 512>);
+                e = launch4(k_count<MODE_GLOBAL, 512>);
             pt.stop();
             if (chunk_ev) cudaEventRecord(ctx->ev_chunk[2 * ctx->n_chunk_ev++ + 1], st);
             if (e != cudaSuccess) {
@@ -1021,7 +965,7 @@ __global__ void k_set_word(unsigned* w, unsigned v) { *w = v; }
 
 // The records are counted on a second stream in `order`'s sequence, `chunks` launches; after each one the number of
 // positions whose rows / entropies / flags exist is published in a device word, and the nmost rounds (select.cu:
-// slim SM-replicated kernel, co-resident with the counting CTAs) only examine positions below it.  The result is
+// the SM-replicated kernel on DVS_TRAIL_SMS SMs of its own) only examine positions below it.  The result is
 // the one dvs_count_kmers + dvs_select give (same kernels' arithmetic; tests/test_gpu_fused.py).
 int dvs_count_select(dvs_ctx* ctx, const dvs_seqset* s, int k, int num_states, const uint32_t* order, uint32_t num,
                      int mode, uint32_t min_size, uint32_t max_size, uint32_t chunks, dvs_kfreqs** out,
@@ -1105,7 +1049,7 @@ int dvs_count_select(dvs_ctx* ctx, const dvs_seqset* s, int k, int num_states, c
         --chunks;
         weights.clear();
     }
-    // (only beside k_count_s3 - k = 4..6 over 4 states - whose CTA leaves room for exactly one selection CTA)
+    // (only beside k_count_s3: k = 4..6 over 4 states)
     const char* s3_env = getenv("DVS_COUNT_S3");
     const bool s3 = num_states == 4 && k >= 4 && k <= 6 && !(s3_env && s3_env[0] == '0');
     const bool trail = chunks > 1 && mode == DVS_MODE_NMOST && num > 0 && s3;
@@ -1122,18 +1066,13 @@ int dvs_count_select(dvs_ctx* ctx, const dvs_seqset* s, int k, int num_states, c
             rc = dvs::select_with_trail(ctx, f, order, num, mode, min_size, max_size, sel_idx, sel_delta, stats5,
                                         size_out, nullptr);
     } else {
-        dvs::TrailArgs ta{ctx->d_ready, 0, ctx->ev_first, ctx->ev_count_done, ctx->d_ready + 1};
-        DVS_CUDA_TRY(cudaMemsetAsync(ctx->d_ready, 0, 8, main_st));
+        dvs::TrailArgs ta{ctx->d_ready, 0, ctx->ev_first, ctx->ev_count_done};
+        DVS_CUDA_TRY(cudaMemsetAsync(ctx->d_ready, 0, sizeof(unsigned), main_st));
         DVS_CUDA_TRY(cudaEventRecord(ctx->ev_fork, main_st));
         DVS_CUDA_TRY(cudaStreamWaitEvent(ctx->stream2, ctx->ev_fork, 0));
         CountDest dst{f->freqs.p, f->totals.p, f->entropy.p, f->valid.p, f->err.p, f->err_total.p, chunks, nullptr};
         dst.rec_seq = seq.data();
         if (weights.size() == chunks) dst.weights = weights.data();
-        if (dvs::trail_shape() != 3) {  // co-resident forms: the counting CTA leaves registers / shared memory free
-            dst.s3_shape = 1;  // 56 registers: leaves 8,192 for the selection CTA on the same SM
-            dst.resident = ctx->d_ready + 1;
-            dst.trail_regs = dvs::trail_count_regs();
-        }
         bool first = true;
         cudaStream_t side = ctx->stream2;
         dst.after_chunk = [&](uint32_t, uint32_t re) -> int {

@@ -10,20 +10,11 @@ struct TrailArgs {
     unsigned limit0;           // its value once `first_ready` has happened
     cudaEvent_t first_ready;   // the first chunk of records has been published
     cudaEvent_t count_done;    // all of them have
-    const unsigned* d_resident;  // device word: counting CTAs resident right now (placement of the trailing kernel)
 };
-// DVS_TRAIL_SHAPE: how counting and the trailing selection share the GPU.
-//   0..2 = one selection CTA beside the counting CTA on every SM, the SM's 65,536 registers split as
-//          1,024 x 56 + 128 x 64 / 1,024 x 48 + 256 x 64 / 1,024 x 40 + 384 x 56;
-//   3    = the selection owns DVS_TRAIL_SMS whole SMs (default 36; measured 24..40 on the bench set): the stand-alone 512-thread kernel on a
-//          high-priority stream takes the SMs the counting CTAs of a finished launch leave, and the counting goes on
-//          with the rest (its CTAs are work-stealing loops, so the ones that find no SM just start late and exit).
-inline int trail_shape() {
-    const char* e = getenv("DVS_TRAIL_SHAPE");
-    const int v = e ? atoi(e) : 3;
-    return v < 0 || v > 3 ? 3 : v;
-}
-inline int trail_count_regs() { return 56 - 8 * (trail_shape() % 3); }
+// How counting and the trailing selection share the GPU: the selection owns DVS_TRAIL_SMS whole SMs (default 36;
+// measured 24..40 on the bench set).  The stand-alone 512-thread kernel on a high-priority stream takes the SMs the
+// counting CTAs of a finished launch leave, and the counting goes on with the rest (its CTAs are work-stealing loops,
+// so the ones that find no SM just start late and exit).
 inline unsigned trail_sms(int sm_count) {
     const char* e = getenv("DVS_TRAIL_SMS");
     const int v = e ? atoi(e) : 36;

@@ -19,6 +19,7 @@
 
 #include <algorithm>
 #include <limits>
+#include <optional>
 
 #include <cooperative_groups.h>
 
@@ -52,7 +53,7 @@ struct SelScal {
     unsigned pad0_;
     double std_bound;        // fast path: |stdv - reference std_delta_jsd| <= std_bound  (0 when exact)
     double cov_bound;        // fast path: same for cov (infinite when the mean is too close to 0)
-    // ---- device-driven rounds (k_sel_scan_dev / k_sel_round_dev) ----
+    // ---- device-driven rounds (k_sel_persist / k_sel_persist_sm_t) ----
     unsigned cursor;         // next position to examine
     unsigned window;         // candidates scored per round
     unsigned window_max;
@@ -303,26 +304,7 @@ k_sel_scan(const double* __restrict__ F, const double* __restrict__ H, uint64_t 
 #include "select_grow.cuh"
 #include "select_sm.cuh"
 
-// waits (bounded: ~150 us) until `want` counting CTAs are resident, or the counting is over
-__global__ void k_wait_resident(const unsigned* resident, unsigned want, const unsigned* ready, unsigned num) {
-    unsigned long long t0, t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t0));
-    for (;;) {
-        if (*reinterpret_cast<const volatile unsigned*>(resident) >= want) break;
-        if (*reinterpret_cast<const volatile unsigned*>(ready) >= num) break;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-        if (t - t0 > 150000ull) break;
-        __nanosleep(500);
-    }
-}
-
 constexpr auto k_sel_persist_sm_full = k_sel_persist_sm_t<kFastThreads, 1, kSmMaxN, kSmChunk>;
-// the trailing form: 128 threads x <= 64 registers and ~66 KB of shared memory fit beside one counting CTA
-// (1,024 threads x 56 registers, 144 KB) on every SM
-template <int NT>
-struct SlimKernel {
-    static constexpr auto fn = k_sel_persist_sm_t<NT, (1024 + NT - 1) / NT, kSmSlimMaxN, kSmSlimChunk>;  // (<= 64 registers)
-};
 
 // test hook: the two building blocks of block_entropy_ilp on arbitrary operands
 __global__ void k_debug_fast_terms(const double* a, const double* b, double* m_out, double* l_out, int* sp_out, uint64_t n) {
@@ -451,6 +433,623 @@ struct Selector {
     }
 };
 
+// One selection call: its arguments, the state and buffers on the device, and where the loop stands.  Each step
+// of the loop in select_core is a function of its own below.
+struct SelRun {
+    dvs_ctx* ctx;
+    dvs_comm* comm;
+    const dvs_kfreqs* f;
+    const uint32_t* order;
+    uint32_t num;
+    int mode;
+    uint32_t min_size, max_size;
+    uint32_t* sel_idx;
+    double* sel_delta;
+    double* stats5;
+    uint32_t* size_out;
+    const TrailArgs* trail;
+    cudaStream_t st = nullptr;
+    uint64_t dim = 0;
+    unsigned world = 1, rank = 0;
+    ShardArgs shard;
+    bool grow_mode = false;  // max / max_cov: the set grows to max_size before candidates replace its lowest record
+    bool use_fast = true;    // bounded-error kernels, exact evaluation only where they cannot decide
+    // trailing (dvs_count_select): the rows are still being produced on another stream; positions below
+    // `trail_limit` have been published
+    unsigned trail_limit = 0;
+    std::vector<uint8_t> valid, err;  // validity / panic flags of the records
+    std::vector<double> err_total;
+    Selector sel;
+    SelState A, B;
+    SelState* cur = &A;
+    SelState* alt = &B;
+    unsigned cap = 0, n = 0;
+    DevBuf<uint8_t> is_member;
+    DevBuf<unsigned> d_order, d_init;
+    std::optional<PhaseTimer> pt;
+    unsigned cursor = 0, accepts = 0, exact_evals = 0;
+    unsigned window = 64, window_max = 64;  // adaptive: grows while windows come back empty, shrinks after a hit
+    // persistent rounds
+    bool use_persist = false, sm_ok = false;
+    unsigned persist_grid = 0, sm_grid = 0;
+    DevBuf<SlicePart> d_slparts;  // k_sel_persist: partial sums of sliced vectors and their arrival tickets
+    DevBuf<unsigned> d_slticks;
+    DevBuf<SmPart> d_spart, d_upart, d_dpart;
+    // batched grow attempts (see k_grow_eval)
+    bool use_grow_batch = false;
+    unsigned grow_window_max = 64, grow_window = 16;
+    SelState fresh;  // clone(): the members re-summed in order (S, E), refreshed whenever the set changes
+    DevBuf<FastSum> d_gparts;
+    DevBuf<double> d_gmd, d_gmb;
+    DevBuf<SelScal> d_gscratch;
+    DevBuf<unsigned> d_ginteresting;
+    bool fresh_valid = false;
+    unsigned fresh_n = 0;
+    const SelState* fresh_of = nullptr;
+    int fresh_which = -1;
+    bool single_candidate = false;  // the grow filter has already isolated the candidate at `cursor`
+    // while the set grows at almost every candidate (e.g. cov right after the start) the filter skips
+    // nothing: after two such windows in a row it is bypassed for 1, 2, 4, 8 candidates
+    unsigned filter_streak = 0, filter_bypass = 0;
+};
+
+// trailing: wait until every record has been counted
+static int wait_counted(SelRun& r) {
+    if (r.trail_limit >= r.num) return DVS_OK;
+    DVS_CUDA_TRY(cudaStreamWaitEvent(r.st, r.trail->count_done, 0));
+    r.trail_limit = r.num;
+    return DVS_OK;
+}
+
+// reads the validity / panic flags of the records.  Every record in `order` goes through KmerSeq::new ->
+// entropy(), where a failing sum check panics: checked here for the positions below `upto`.
+static int read_flags(SelRun& r, unsigned upto) {
+    const dvs_kfreqs* f = r.f;
+    if (f->nrec) {
+        DVS_CUDA_TRY(cudaMemcpyAsync(r.valid.data(), f->valid.p, f->nrec, cudaMemcpyDeviceToHost, r.st));
+        DVS_CUDA_TRY(cudaMemcpyAsync(r.err.data(), f->err.p, f->nrec, cudaMemcpyDeviceToHost, r.st));
+        DVS_CUDA_TRY(cudaMemcpyAsync(r.err_total.data(), f->err_total.p, f->nrec * sizeof(double),
+                                     cudaMemcpyDeviceToHost, r.st));
+        DVS_CUDA_TRY(cudaStreamSynchronize(r.st));
+    }
+    for (uint32_t i = 0; i < upto; ++i)
+        if (r.valid[r.order[i]] && r.err[r.order[i]]) {
+            set_error("cannot calculate entropy as frequency vector total %.17g!=1.0", r.err_total[r.order[i]]);
+            return DVS_ERR_VALUE;
+        }
+    return DVS_OK;
+}
+
+// argument checks, the panic check over the published positions, the initial set and its state, the buffers,
+// and the round forms this call can use
+static int select_setup(SelRun& r) {
+    dvs_ctx* ctx = r.ctx;
+    const dvs_kfreqs* f = r.f;
+    const uint32_t* order = r.order;
+    const uint32_t num = r.num;
+    if (!ctx || !f || (!order && num) || !r.size_out) {
+        set_error("dvs_select: NULL argument");
+        return DVS_ERR_ARG;
+    }
+    if (r.mode < DVS_MODE_NMOST || r.mode > DVS_MODE_MAX_COV) {
+        set_error("dvs_select: bad mode %d", r.mode);
+        return DVS_ERR_ARG;
+    }
+    ctx->last_accepts = 0;
+    ctx->last_trail_accepts = 0;
+    ctx->last_trail_launches = 0;
+    ctx->last_trail_sms = 0xFFFFFFFFu;
+    if (num < r.min_size) {  // records.rs:323-325, :404-410
+        set_error("The number of sequences %u is < n %u", num, r.min_size);
+        return DVS_ERR_VALUE;
+    }
+    if (r.mode == DVS_MODE_NMOST) r.max_size = r.min_size;
+    if (!(num > r.max_size)) r.max_size = num;  // records.rs:412-416
+    for (uint32_t i = 0; i < num; ++i)
+        if (order[i] >= f->nrec) {
+            set_error("dvs_select: order[%u]=%u out of range (nrec=%u)", i, order[i], f->nrec);
+            return DVS_ERR_ARG;
+        }
+    DVS_CUDA_TRY(dvs::enter(ctx));
+    r.st = ctx->stream;
+    r.dim = f->dim;
+    dvs_comm* comm = r.comm;
+    r.world = comm ? (unsigned)comm->world : 1u;
+    r.rank = comm ? (unsigned)comm->rank : 0u;
+    memset(&r.shard, 0, sizeof r.shard);
+    r.shard.rank = (int)r.rank;
+    r.shard.world = (int)r.world;
+    for (unsigned q = 0; q < r.world && comm; ++q) r.shard.xbase[q] = comm->peer[q];
+    if (r.world > 1) DVS_TRY(comm_barrier(ctx, comm));  // every rank is here: exchange slots of earlier calls are dead
+    // trailing: start once the first chunk (>= min_size positions) is there
+    r.trail_limit = num;
+    if (r.trail) {
+        DVS_CUDA_TRY(cudaStreamWaitEvent(r.st, r.trail->first_ready, 0));
+        r.trail_limit = std::min(r.trail->limit0, num);
+        if (r.mode != DVS_MODE_NMOST || r.trail_limit < r.min_size)  // nothing to gain / not enough rows yet
+            DVS_TRY(wait_counted(r));
+    }
+    r.valid.resize(f->nrec);
+    r.err.resize(f->nrec);
+    r.err_total.resize(f->nrec);
+    DVS_TRY(read_flags(r, r.trail_limit));
+
+    std::vector<unsigned> init;  // records.rs:299-305: first min_size records, failures dropped
+    for (uint32_t i = 0; i < r.min_size; ++i)
+        if (r.valid[order[i]]) init.push_back(order[i]);
+    if (init.empty()) {
+        set_error("records cannot be empty");  // records.rs:28-30
+        return DVS_ERR_VALUE;
+    }
+    if (init.size() <= 1) {
+        set_error("must have > 1 KmerSeq");  // records.rs:227-230
+        return DVS_ERR_VALUE;
+    }
+    // (duplicates in the initial set: the reference's Vec keeps both rows; so does this one)
+
+    r.grow_mode = (r.mode != DVS_MODE_NMOST);
+    // max modes with max_size below the initial size (e.g. max_size < min_size, which only the reference's
+    // CLI rejects, cli.py:311): `size == max_size` never holds, so the set keeps growing as in
+    // records.rs:427-451 - every buffer is then sized for all `num` records
+    const bool unbounded = r.grow_mode && r.max_size < (uint32_t)init.size();
+    r.cap = (unbounded ? num : std::max<unsigned>(std::max(r.min_size, r.max_size), (unsigned)init.size())) + 1;
+    r.n = (unsigned)init.size();
+    DVS_TRY(r.A.alloc(r.dim, r.cap));
+    if (r.grow_mode) DVS_TRY(r.B.alloc(r.dim, r.cap));
+    DVS_TRY(r.is_member.alloc(f->nrec));
+    DVS_TRY(r.d_order.alloc(num));
+    DVS_TRY(r.d_init.alloc(init.size()));
+    DVS_CUDA_TRY(cudaMemsetAsync(r.is_member.p, 0, f->nrec, r.st));
+    DVS_CUDA_TRY(cudaMemcpyAsync(r.d_order.p, order, num * sizeof(unsigned), cudaMemcpyHostToDevice, r.st));
+    DVS_CUDA_TRY(cudaMemcpyAsync(r.d_init.p, init.data(), init.size() * sizeof(unsigned), cudaMemcpyHostToDevice, r.st));
+    k_set_members<<<(unsigned)((init.size() + 255) / 256), 256, 0, r.st>>>(r.is_member.p, r.d_init.p, r.n, 1);
+    DVS_LAUNCHED(ctx);
+    r.pt.emplace(ctx, DVS_PHASE_SELECT);
+    r.sel = Selector{ctx, f, r.dim, r.st, (SelScal*)ctx->pinned};
+    DVS_TRY(r.sel.build(*r.cur, r.d_init.p, r.n, -1));
+    r.window_max = std::max(64u, (unsigned)ctx->sm_count * 12u);
+    r.cursor = r.min_size;
+    // DVS_SELECT_EXACT_ONLY=1 disables the bounded-error fast path (tests compare both)
+    const char* exact_env = getenv("DVS_SELECT_EXACT_ONLY");
+    r.use_fast = !(exact_env && exact_env[0] == '1');
+
+    // DVS_SELECT_PERSIST=0: host-driven rounds, =1: the global-state persistent kernel; default: SM-replicated
+    // rounds when the state fits in shared memory.  Host-driven rounds also run where cooperative launches do not.
+    // DVS_SELECT_GRID: CTAs of the persistent kernels (tests run several ranks on ONE GPU: their kernels must be
+    // co-resident, so each takes a share of the SMs)
+    const char* grid_env = getenv("DVS_SELECT_GRID");
+    const unsigned grid_cap = grid_env && atoi(grid_env) > 0 ? (unsigned)atoi(grid_env) : 0xFFFFFFFFu;
+    const char* per_env = getenv("DVS_SELECT_PERSIST");
+    int coop = 0, per_sm = 0, per_sm2 = 0;
+    cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, ctx->device);
+    if (coop && cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sel_persist, kFastThreads, 0) != cudaSuccess)
+        per_sm = 0;
+    r.use_persist = r.use_fast && coop && per_sm > 0 && !(per_env && per_env[0] == '0');
+    r.persist_grid = std::min((unsigned)ctx->sm_count * (unsigned)std::min(per_sm, 2), std::max(1u, std::min(grid_cap, 0x7FFFFFFFu)));
+    r.sm_ok = r.use_persist && !(per_env && per_env[0] == '1') && r.dim <= kSmMaxDim;
+    if (r.sm_ok) {
+        r.sm_ok = cudaFuncSetAttribute(k_sel_persist_sm_full, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       (int)sizeof(SmShared)) == cudaSuccess &&
+                  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm2, k_sel_persist_sm_full, kFastThreads,
+                                                                sizeof(SmShared)) == cudaSuccess &&
+                  per_sm2 > 0;
+        (void)cudaGetLastError();
+    }
+    r.sm_grid = std::min(std::min<unsigned>((unsigned)ctx->sm_count, kSmMaxGrid), grid_cap);
+    if (r.sm_ok) {
+        DVS_TRY(r.d_spart.alloc(2 * kSmMaxGrid));
+        DVS_TRY(r.d_upart.alloc(kSmMaxN + 1));
+        DVS_TRY(r.d_dpart.alloc(3));  // the leader's broadcasts: scan decision (double buffered), update result
+    }
+    // batched grow attempts (see k_grow_eval): scratch for a window of candidates; DVS_SELECT_GROW_BATCH=0
+    // keeps one host-driven attempt per candidate
+    const char* gb_env = getenv("DVS_SELECT_GROW_BATCH");
+    r.use_grow_batch = r.use_fast && r.grow_mode && !(gb_env && gb_env[0] == '0');
+    r.grow_window_max = 64 * r.world;
+    if (r.use_grow_batch && r.n != r.max_size) {
+        DVS_TRY(r.fresh.alloc(r.dim, r.cap));
+        DVS_TRY(r.d_gparts.alloc((size_t)r.grow_window_max * (r.cap + 3)));
+        DVS_TRY(r.d_gmd.alloc((size_t)r.grow_window_max * r.cap));
+        DVS_TRY(r.d_gmb.alloc((size_t)r.grow_window_max * r.cap));
+        DVS_TRY(r.d_gscratch.alloc(r.grow_window_max));  // (indexed by the window offset)
+        DVS_TRY(r.d_ginteresting.alloc(1));
+    }
+    return DVS_OK;
+}
+
+// max while the set grows: evaluate a window of grow attempts on the device and move the cursor to the first
+// candidate that could be adopted (the host path then decides it), past the window when none can
+static int grow_filter(SelRun& r) {
+    if (r.filter_bypass > 0) {
+        --r.filter_bypass;
+        r.single_candidate = true;  // straight to the host path for this candidate
+        return DVS_OK;
+    }
+    dvs_ctx* ctx = r.ctx;
+    const dvs_kfreqs* f = r.f;
+    SelState* cur = r.cur;
+    const unsigned n = r.n, cursor = r.cursor, world = r.world;
+    if (!r.fresh_valid || r.fresh_n != n || r.fresh_of != cur || r.fresh_which != cur->which) {
+        k_sel_sum<<<r.sel.vec_grid(), 256, 0, r.st>>>(f->freqs.p, f->entropy.p, r.dim, cur->members(), n, -1,
+                                                      r.fresh.S(), r.fresh.members(), r.fresh.sc.p);
+        DVS_LAUNCHED(ctx);
+        r.fresh_valid = true;
+        r.fresh_n = n;
+        r.fresh_of = cur;
+        r.fresh_which = cur->which;
+    }
+    const unsigned W = std::min(r.grow_window, r.num - cursor);
+    DVS_CUDA_TRY(cudaMemsetAsync(r.d_ginteresting.p, 0xFF, sizeof(unsigned), r.st));
+    // candidate-sharded: this GPU evaluates the window candidates c with (cursor + c) % world == rank
+    const unsigned gc0 = (r.rank + world - cursor % world) % world;
+    const unsigned Wloc = W > gc0 ? (W - gc0 + world - 1) / world : 0;
+    if (Wloc) {
+        k_grow_eval<<<dim3(n + 3, Wloc), kFastThreads, 0, r.st>>>(f->freqs.p, r.dim, cur->S(), cur->members(), cur->sc.p,
+                                                                  r.fresh.S(), f->valid.p, r.is_member.p, r.d_order.p,
+                                                                  cursor, r.d_gparts.p, gc0, world);
+        DVS_LAUNCHED(ctx);
+        k_grow_decide<<<Wloc, kFastThreads, 0, r.st>>>(f->entropy.p, r.dim, cur->members(), cur->sc.p, r.fresh.sc.p,
+                                                       f->valid.p, r.is_member.p, r.d_order.p, cursor, r.d_gparts.p,
+                                                       r.d_gmd.p, r.d_gmb.p, r.cap, r.d_gscratch.p, r.d_ginteresting.p,
+                                                       r.mode == DVS_MODE_MAX_COV ? 1 : 0, gc0, world);
+        DVS_LAUNCHED(ctx);
+    }
+    if (world > 1) DVS_TRY(comm_min_u32(ctx, r.comm, r.d_ginteresting.p, r.d_ginteresting.p));
+    unsigned* h_fi = reinterpret_cast<unsigned*>(reinterpret_cast<char*>(ctx->pinned) + sizeof(SelScal));
+    DVS_CUDA_TRY(cudaMemcpyAsync(h_fi, r.d_ginteresting.p, sizeof(unsigned), cudaMemcpyDeviceToHost, r.st));
+    DVS_CUDA_TRY(cudaStreamSynchronize(r.st));
+    const unsigned fi = *h_fi;
+    if (fi == kNone) {  // the whole window was certainly rejected
+        r.cursor += W;
+        r.grow_window = std::min(r.grow_window * 2u, r.grow_window_max);
+        return DVS_OK;
+    }
+    r.grow_window = std::max(4u, std::min(r.grow_window_max, 2u * (fi - cursor + 1u)));
+    if (fi == cursor) {
+        if (++r.filter_streak >= 2) r.filter_bypass = 1u << std::min(r.filter_streak - 2u, 3u);
+    } else {
+        r.filter_streak = 0;
+    }
+    r.cursor = fi;  // everything before it is certainly rejected; the host path takes this one
+    r.single_candidate = true;
+    return DVS_OK;
+}
+
+// DVS_SELECT_TRACE: CTA 0's phase timeline of the first rounds, appended as text to the file it names;
+// DVS_SELECT_TRACE_ALL (SM-replicated kernel): every CTA's, raw u64 [256 rounds][8 slots][256 CTAs]
+static int write_trace(const unsigned long long* d_trace, size_t len, bool all, bool use_sm, const char* path) {
+    std::vector<unsigned long long> tr(len);
+    DVS_CUDA_TRY(cudaMemcpy(tr.data(), d_trace, len * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+    if (all) {
+        if (FILE* fp = fopen(path, "wb")) {
+            fwrite(tr.data(), sizeof(unsigned long long), len, fp);
+            fclose(fp);
+        }
+        return DVS_OK;
+    }
+    if (FILE* fp = fopen(path, "a")) {
+        const int slots = use_sm ? kSmTraceSlots : 4, used = use_sm ? 7 : 4;
+        fprintf(fp, use_sm ? "# round scan_ns gather_ns decide_ns update_ns gather2_ns finalize_ns next_ns (CTA 0)\n"
+                           : "# round scan_ns wait1_ns update_ns wait2_ns (CTA 0; wait = grid barrier incl. the slowest CTA)\n");
+        for (int q = 0; (q + 1) * slots < 2048 && tr[slots * (q + 1)]; ++q) {
+            fprintf(fp, "%d", q);
+            for (int p = 0; p + 1 < used; ++p) fprintf(fp, " %llu", tr[slots * q + p + 1] - tr[slots * q + p]);
+            fprintf(fp, " %llu\n", tr[slots * (q + 1)] - tr[slots * q + used - 1]);
+        }
+        fclose(fp);
+    }
+    return DVS_OK;
+}
+
+// every remaining replacing round in one launch, until the rounds finish or halt for the host (`halted`: an
+// undecided candidate or state, which the host resolves exactly).  The SM-replicated kernel runs while the state
+// fits its shared memory, k_sel_persist otherwise.  Trailing the counting, the SM-replicated kernel takes
+// DVS_TRAIL_SMS whole SMs and returns when everything has been published; anything else waits for the counting.
+static int persist_rounds(SelRun& r, bool& halted) {
+    dvs_ctx* ctx = r.ctx;
+    const dvs_kfreqs* f = r.f;
+    SelState* cur = r.cur;
+    const unsigned world = r.world;
+    const bool use_sm = r.sm_ok && r.n <= kSmMaxN;
+    const bool trailing = r.trail_limit < r.num && use_sm && world == 1;
+    if (!trailing) DVS_TRY(wait_counted(r));
+    const unsigned grid = trailing ? std::min(r.sm_grid, trail_sms(ctx->sm_count)) : (use_sm ? r.sm_grid : r.persist_grid);
+    k_sel_set_dev<<<1, 1, 0, r.st>>>(cur->sc.p, r.cursor, std::min(r.window, grid * world), grid * world, r.num,
+                                     r.accepts, (unsigned)cur->which);
+    if (r.comm) {
+        r.shard.tag_base = (unsigned)((++r.comm->sel_tag_base) << 20);
+        DVS_TRY(comm_host_rendezvous(ctx, r.comm));  // (ranks sharing one GPU only)
+    }
+    DVS_LAUNCHED(ctx);
+    const double* a_F = f->freqs.p;
+    const double* a_H = f->entropy.p;
+    uint64_t a_dim = r.dim;
+    double *a_S0 = cur->Sbuf[0].p, *a_S1 = cur->Sbuf[1].p;
+    unsigned *a_M0 = cur->membuf[0].p, *a_M1 = cur->membuf[1].p;
+    uint8_t* a_mem = r.is_member.p;
+    double *a_md = cur->mdelta.p, *a_mb = cur->mbound.p;
+    SelScal* a_sc = cur->sc.p;
+    const uint8_t* a_valid = f->valid.p;
+    const unsigned* a_order = r.d_order.p;
+    unsigned a_rounds = world > 1 ? 0xFFFF0u : 0x7fffffffu;  // (exchange tags of one launch are 20 bits)
+    unsigned long long* a_trace = nullptr;
+    DevBuf<unsigned long long> d_trace;
+    const char* tr_env = getenv("DVS_SELECT_TRACE");
+    const char* tra_env = getenv("DVS_SELECT_TRACE_ALL");
+    int a_trace_all = (use_sm && tra_env && tra_env[0]) ? 1 : 0;
+    const char* trace_path = a_trace_all ? tra_env : (tr_env && tr_env[0] ? tr_env : nullptr);
+    const size_t trace_len = a_trace_all ? (size_t)256 * kSmTraceSlots * kSmMaxGrid : 2048;
+    if (trace_path) {
+        DVS_TRY(d_trace.alloc(trace_len));
+        DVS_CUDA_TRY(cudaMemsetAsync(d_trace.p, 0, trace_len * sizeof(unsigned long long), r.st));
+        a_trace = d_trace.p;
+    }
+    if (use_sm) {
+        unsigned a_dim32 = (unsigned)r.dim;
+        double* a_S = cur->S();
+        unsigned* a_M = cur->members();
+        SmPart *a_sp = r.d_spart.p, *a_up = r.d_upart.p, *a_dp = r.d_dpart.p;
+        DVS_CUDA_TRY(cudaMemsetAsync(r.d_dpart.p, 0, 3 * sizeof(SmPart), r.st));
+        // exchange tags restart at 1 in every launch
+        DVS_CUDA_TRY(cudaMemsetAsync(r.d_spart.p, 0, 2 * kSmMaxGrid * sizeof(SmPart), r.st));
+        DVS_CUDA_TRY(cudaMemsetAsync(r.d_upart.p, 0, (kSmMaxN + 1) * sizeof(SmPart), r.st));
+        const unsigned* a_ready = trailing ? r.trail->d_ready : nullptr;
+        unsigned a_limit0 = r.trail_limit;
+        if (trailing) {
+            if (!ctx->stream_hi) {
+                int lo_p = 0, hi_p = 0;
+                DVS_CUDA_TRY(cudaDeviceGetStreamPriorityRange(&lo_p, &hi_p));
+                DVS_CUDA_TRY(cudaStreamCreateWithPriority(&ctx->stream_hi, cudaStreamNonBlocking, hi_p));
+                DVS_CUDA_TRY(cudaEventCreateWithFlags(&ctx->ev_hi_in, cudaEventDisableTiming));
+                DVS_CUDA_TRY(cudaEventCreateWithFlags(&ctx->ev_hi_out, cudaEventDisableTiming));
+            }
+            // 512 threads x 128 registers: one CTA fills an SM's register file, so these CTAs take whole SMs - the
+            // ones the counting CTAs of the launch in flight leave when it ends (the higher stream priority puts them
+            // ahead of the next counting launch's CTAs)
+            DVS_CUDA_TRY(cudaEventRecord(ctx->ev_hi_in, r.st));
+            DVS_CUDA_TRY(cudaStreamWaitEvent(ctx->stream_hi, ctx->ev_hi_in, 0));
+            k_sel_persist_sm_full<<<grid, kFastThreads, sizeof(SmShared), ctx->stream_hi>>>(
+                a_F, a_H, a_dim32, a_S, a_M, a_mem, a_md, a_mb, a_sc, a_valid, a_order, a_sp, a_up, a_dp, a_trace,
+                a_trace_all, r.shard, a_ready, a_limit0);
+            DVS_CUDA_TRY(cudaGetLastError());
+            DVS_CUDA_TRY(cudaEventRecord(ctx->ev_hi_out, ctx->stream_hi));
+            DVS_CUDA_TRY(cudaStreamWaitEvent(r.st, ctx->ev_hi_out, 0));
+        } else {
+            void* args[] = {&a_F, &a_H, &a_dim32, &a_S, &a_M, &a_mem, &a_md, &a_mb, &a_sc, &a_valid, &a_order,
+                            &a_sp, &a_up, &a_dp, &a_trace, &a_trace_all, &r.shard, &a_ready, &a_limit0};
+            DVS_CUDA_TRY(cudaLaunchCooperativeKernel((void*)k_sel_persist_sm_full, dim3(grid), dim3(kFastThreads), args,
+                                                     sizeof(SmShared), r.st));
+        }
+    } else {
+        // DVS_SELECT_SLICES (A/B measurements): 0 = one CTA per candidate / member slot, 1 = candidates of a short
+        // window are cut into slices (default), 2 = member slots of the update too (measured slower: a slice
+        // repeats the slot's set-up and pays a fence + ticket, 55 us against 33 us per update at k = 8, n = 100)
+        const char* sl_env = getenv("DVS_SELECT_SLICES");
+        unsigned a_slice_mode = sl_env ? (unsigned)atoi(sl_env) : 1u;
+        if (!r.d_slparts.p && a_slice_mode) {
+            const size_t slots = std::max<size_t>(grid, (size_t)r.cap + 1);
+            DVS_TRY(r.d_slparts.alloc(slots * kMaxSlices));
+            DVS_TRY(r.d_slticks.alloc(slots));
+            DVS_CUDA_TRY(cudaMemsetAsync(r.d_slticks.p, 0, slots * sizeof(unsigned), r.st));
+        }
+        SlicePart* a_parts = r.d_slparts.p;
+        unsigned* a_ticks = r.d_slticks.p;
+        void* args[] = {&a_F, &a_H, &a_dim, &a_S0, &a_S1, &a_M0, &a_M1, &a_mem, &a_md, &a_mb, &a_sc, &a_valid,
+                        &a_order, &a_rounds, &a_trace, &r.shard, &a_parts, &a_ticks, &a_slice_mode};
+        DVS_CUDA_TRY(cudaLaunchCooperativeKernel((void*)k_sel_persist, dim3(grid), dim3(kFastThreads), args, 0, r.st));
+    }
+    ctx->launches++;
+    DVS_TRY(r.sel.read(*cur));
+    if (a_trace) DVS_TRY(write_trace(a_trace, trace_len, a_trace_all, use_sm, trace_path));
+    const SelScal hd = *r.sel.h_sc;
+    if (hd.panic) return panic_error(hd);
+    if (trailing) {
+        ctx->last_trail_accepts += hd.accepts - r.accepts;
+        ++ctx->last_trail_launches;
+        std::vector<unsigned> smid(grid);
+        DVS_CUDA_TRY(cudaMemcpyAsync(smid.data(), r.trail->d_ready + kTrailSmidOff, grid * sizeof(unsigned),
+                                     cudaMemcpyDeviceToHost, r.st));
+        DVS_CUDA_TRY(cudaStreamSynchronize(r.st));
+        std::sort(smid.begin(), smid.end());
+        const unsigned distinct = (unsigned)(std::unique(smid.begin(), smid.end()) - smid.begin());
+        ctx->last_trail_sms = std::min(ctx->last_trail_sms, distinct);
+        r.trail_limit = std::max(r.trail_limit, std::min(hd.limit, r.num));
+    }
+    r.cursor = hd.cursor;
+    r.window = hd.window;
+    r.accepts = hd.accepts;
+    cur->which = (int)hd.which;
+    halted = hd.halt != 0;
+    if (halted) DVS_TRY(r.sel.reset_scan(*cur));
+    return DVS_OK;
+}
+
+// one host-driven round: score a window of candidates, decide undecided candidates and states exactly, and let
+// the first acceptance replace the lowest record (records.rs:111-118).  While the set grows (max), the accepted
+// candidate is left in `grow_row` for grow_attempt instead, with the scan's scalars in `h`.
+static int host_window(SelRun& r, int& grow_row, SelScal& h) {
+    const dvs_kfreqs* f = r.f;
+    SelState* cur = r.cur;
+    grow_row = -1;
+    if (!r.use_persist || r.cursor >= r.trail_limit) DVS_TRY(wait_counted(r));  // (host rounds do not trail)
+    const unsigned count = r.single_candidate ? 1u : std::min(r.window, r.trail_limit - r.cursor);
+    r.single_candidate = false;
+    unsigned pos = kNone;
+    if (r.use_fast) {
+        DVS_TRY(r.sel.scan_fast(*cur, r.is_member.p, r.d_order.p, r.cursor, count));
+        DVS_TRY(r.sel.read(*cur));
+        h = *r.sel.h_sc;
+        if (h.panic) return panic_error(h);
+        if (h.state_unsure) {
+            // the last fast update could not certify lowest_index / a sum check: redo it exactly and
+            // re-score the window against the now certain state
+            DVS_TRY(r.sel.update(*cur, r.n));
+            ++r.exact_evals;
+            return DVS_OK;
+        }
+        if (h.first_unsure < h.first_true) {
+            // an undecided candidate comes before the first certain acceptance: decide it exactly
+            const unsigned pu = h.first_unsure;
+            if (!h.exact) DVS_TRY(r.sel.update(*cur, r.n));
+            DVS_TRY(r.sel.scan(*cur, f, r.is_member.p, r.d_order.p, pu, 1, nullptr));
+            DVS_TRY(r.sel.read(*cur));
+            h = *r.sel.h_sc;
+            ++r.exact_evals;
+            if (h.panic) return panic_error(h);
+            if (h.first_panic == pu) {
+                set_error("cannot calculate entropy as frequency vector total !=1.0 (candidate at position %u)", pu);
+                return DVS_ERR_VALUE;
+            }
+            if (h.first_true != pu) {  // rejected by the exact evaluation: carry on after it
+                DVS_TRY(r.sel.reset_scan(*cur));
+                r.cursor = pu + 1;
+                return DVS_OK;
+            }
+            pos = pu;
+        } else if (h.first_true != kNone) {
+            pos = h.first_true;
+        }
+    } else {
+        DVS_TRY(r.sel.scan(*cur, f, r.is_member.p, r.d_order.p, r.cursor, count, nullptr));
+        DVS_TRY(r.sel.read(*cur));
+        h = *r.sel.h_sc;
+        if (h.panic) return panic_error(h);
+        if (h.first_panic != kNone && h.first_panic <= h.first_true) {
+            set_error("cannot calculate entropy as frequency vector total !=1.0 (candidate at position %u)",
+                      h.first_panic);
+            return DVS_ERR_VALUE;
+        }
+        pos = h.first_true;
+    }
+    if (pos == kNone) {
+        r.cursor += count;
+        r.window = std::min(r.window * 2, r.window_max);
+        return DVS_OK;
+    }
+    const unsigned row = r.order[pos];
+    r.window = std::max(64u, std::min(r.window_max, 2 * (pos - r.cursor + 1)));
+    r.cursor = pos + 1;
+    if (r.grow_mode && r.n != r.max_size) {
+        grow_row = (int)row;
+        return DVS_OK;
+    }
+    DVS_TRY(r.use_fast ? r.sel.replace_fast(*cur, r.n, row, r.is_member.p) : r.sel.replace(*cur, r.n, row, r.is_member.p));
+    ++r.accepts;
+    return DVS_OK;
+}
+
+// records.rs:434-451: nw = clone(); nw.push(rec); keep whichever has the larger statistic.  First tried with the
+// bounded-error kernels: the comparison is decided from them only when it holds for every admissible error;
+// otherwise both states are evaluated by the exact kernel.  `h`: the scalars of the current state.
+static int grow_attempt(SelRun& r, unsigned row, SelScal h) {
+    const bool use_cov = (r.mode == DVS_MODE_MAX_COV);
+    auto adopt = [&]() -> int {
+        std::swap(r.cur, r.alt);
+        ++r.n;
+        ++r.accepts;
+        uint8_t one = 1;
+        DVS_CUDA_TRY(cudaMemcpyAsync(r.is_member.p + row, &one, 1, cudaMemcpyHostToDevice, r.st));
+        DVS_CUDA_TRY(cudaStreamSynchronize(r.st));
+        return DVS_OK;
+    };
+    if (r.use_fast && !h.state_unsure) {
+        DVS_TRY(r.sel.build_fast(*r.alt, r.cur->members(), r.n, (int)row));
+        DVS_TRY(r.sel.read(*r.alt));
+        const SelScal hf = *r.sel.h_sc;
+        if (hf.panic) return panic_error(hf);
+        if (!hf.state_unsure) {
+            const double sa_f = use_cov ? h.cov : h.stdv, ba = h.exact ? 0.0 : (use_cov ? h.cov_bound : h.std_bound);
+            const double sb_f = use_cov ? hf.cov : hf.stdv, bb = use_cov ? hf.cov_bound : hf.std_bound;
+            if (sb_f - bb > sa_f + ba) return adopt();
+            if (sb_f + bb < sa_f - ba) return r.sel.reset_scan(*r.cur);  // candidate discarded
+        }
+    }
+    if (r.use_fast) ++r.exact_evals;
+    if (!h.exact) {
+        DVS_TRY(r.sel.update(*r.cur, r.n));
+        DVS_TRY(r.sel.read(*r.cur));
+        h = *r.sel.h_sc;
+        if (h.panic) return panic_error(h);
+    }
+    DVS_TRY(r.sel.build(*r.alt, r.cur->members(), r.n, (int)row));
+    DVS_TRY(r.sel.read(*r.alt));
+    const SelScal hb = *r.sel.h_sc;
+    if (hb.panic) return panic_error(hb);
+    const double sa = use_cov ? h.cov : h.stdv;
+    const double sb = use_cov ? hb.cov : hb.stdv;
+    if (sb > sa) return adopt();
+    return r.sel.reset_scan(*r.cur);  // candidate discarded: re-arm the min-index reduction of `cur`
+}
+
+// the panic check of the records that were not published when a trailing selection started, the exact
+// re-evaluation of the final state (reported numbers are exact), and the copies out
+static int select_finish(SelRun& r) {
+    dvs_ctx* ctx = r.ctx;
+    if (r.trail) {
+        DVS_CUDA_TRY(cudaStreamWaitEvent(r.st, r.trail->count_done, 0));
+        DVS_TRY(read_flags(r, r.num));
+    }
+    DVS_TRY(r.sel.read(*r.cur));
+    if (!r.sel.h_sc->exact || r.sel.h_sc->state_unsure) DVS_TRY(r.sel.update(*r.cur, r.n));
+    ctx->last_exact_evals = r.exact_evals;
+    DVS_TRY(r.sel.read(*r.cur));
+    const SelScal h = *r.sel.h_sc;
+    if (h.panic) return panic_error(h);
+    if (r.sel_idx)
+        DVS_CUDA_TRY(cudaMemcpyAsync(r.sel_idx, r.cur->members(), r.n * sizeof(unsigned), cudaMemcpyDeviceToHost, r.st));
+    if (r.sel_delta)
+        DVS_CUDA_TRY(cudaMemcpyAsync(r.sel_delta, r.cur->mdelta.p, r.n * sizeof(double), cudaMemcpyDeviceToHost, r.st));
+    DVS_CUDA_TRY(cudaStreamSynchronize(r.st));
+    if (r.stats5) {
+        r.stats5[0] = h.total_jsd;
+        r.stats5[1] = h.mean;
+        r.stats5[2] = h.stdv;
+        r.stats5[3] = h.cov;
+        r.stats5[4] = h.E;
+    }
+    *r.size_out = r.n;
+    ctx->last_accepts = r.accepts;
+    if (r.world > 1) DVS_TRY(comm_check_error(ctx, r.comm, "dvs_select_sharded"));
+    return DVS_OK;
+}
+
+// comm == nullptr: one GPU.  Otherwise every rank calls this with the same rows (a kfreqs made by
+// dvs_count_kmers_sharded / dvs_kfreqs_allgather), the same order and the same arguments: the state and
+// every host-side decision are replicated (identical inputs, identical kernels), while the windows of
+// candidates are scored candidate-sharded with an all-reduce(min) of the first interesting position.
+static int select_core(dvs_ctx* ctx, dvs_comm* comm, const dvs_kfreqs* f, const uint32_t* order, uint32_t num, int mode,
+                       uint32_t min_size, uint32_t max_size, uint32_t* sel_idx, double* sel_delta, double* stats5,
+                       uint32_t* size_out, const TrailArgs* trail = nullptr) {
+    SelRun r{ctx, comm, f, order, num, mode, min_size, max_size, sel_idx, sel_delta, stats5, size_out, trail};
+    DVS_TRY(select_setup(r));
+    while (r.cursor < num) {
+        const bool growing = r.grow_mode && r.n != r.max_size;  // max below its size: candidates join the set
+        if (growing && r.use_grow_batch && !r.single_candidate) {
+            DVS_TRY(grow_filter(r));  // batched grow attempts isolate the next candidate worth one
+            continue;
+        }
+        if (!growing && r.use_persist) {  // replacing rounds on the device, until they finish or halt
+            bool halted = false;
+            DVS_TRY(persist_rounds(r, halted));
+            if (!halted) continue;
+            if (r.cursor >= num) break;
+        }
+        // host-driven: the rounds themselves without persistent kernels (DVS_SELECT_PERSIST=0, exact-only,
+        // no cooperative launch), a halted round's exact decision, and every candidate of a growing set
+        int grow_row = -1;
+        SelScal h;
+        DVS_TRY(host_window(r, grow_row, h));
+        if (grow_row >= 0) DVS_TRY(grow_attempt(r, (unsigned)grow_row, h));
+    }
+    return select_finish(r);
+}
+
+int select_with_trail(dvs_ctx* ctx, const dvs_kfreqs* f, const uint32_t* order, uint32_t num, int mode, uint32_t min_size,
+                      uint32_t max_size, uint32_t* sel_idx, double* sel_delta, double* stats5, uint32_t* size_out,
+                      const TrailArgs* trail) {
+    return select_core(ctx, nullptr, f, order, num, mode, min_size, max_size, sel_idx, sel_delta, stats5, size_out, trail);
+}
+
 }  // namespace dvs
 
 using namespace dvs;
@@ -462,601 +1061,6 @@ struct dvs_summed {
     unsigned n = 0;
 };
 
-extern "C" {
-
-// comm == nullptr: one GPU.  Otherwise every rank calls this with the same rows (a kfreqs made by
-// dvs_count_kmers_sharded / dvs_kfreqs_allgather), the same order and the same arguments: the state and
-// every host-side decision are replicated (identical inputs, identical kernels), while the windows of
-// candidates are scored candidate-sharded with an all-reduce(min) of the first interesting position.
-static int select_core(dvs_ctx* ctx, dvs_comm* comm, const dvs_kfreqs* f, const uint32_t* order, uint32_t num, int mode,
-                       uint32_t min_size, uint32_t max_size, uint32_t* sel_idx, double* sel_delta, double* stats5,
-                       uint32_t* size_out, const TrailArgs* trail = nullptr) {
-    if (!ctx || !f || (!order && num) || !size_out) {
-        set_error("dvs_select: NULL argument");
-        return DVS_ERR_ARG;
-    }
-    if (mode < DVS_MODE_NMOST || mode > DVS_MODE_MAX_COV) {
-        set_error("dvs_select: bad mode %d", mode);
-        return DVS_ERR_ARG;
-    }
-    ctx->last_accepts = 0;
-    ctx->last_trail_accepts = 0;
-    ctx->last_trail_launches = 0;
-    ctx->last_trail_sms = 0xFFFFFFFFu;
-    if (num < min_size) {  // records.rs:323-325, :404-410
-        set_error("The number of sequences %u is < n %u", num, min_size);
-        return DVS_ERR_VALUE;
-    }
-    if (mode == DVS_MODE_NMOST) max_size = min_size;
-    if (!(num > max_size)) max_size = num;  // records.rs:412-416
-    for (uint32_t i = 0; i < num; ++i)
-        if (order[i] >= f->nrec) {
-            set_error("dvs_select: order[%u]=%u out of range (nrec=%u)", i, order[i], f->nrec);
-            return DVS_ERR_ARG;
-        }
-    DVS_CUDA_TRY(dvs::enter(ctx));
-    cudaStream_t st = ctx->stream;
-    const uint64_t dim = f->dim;
-    const unsigned world = comm ? (unsigned)comm->world : 1u, rank = comm ? (unsigned)comm->rank : 0u;
-    ShardArgs shard;
-    memset(&shard, 0, sizeof shard);
-    shard.rank = (int)rank;
-    shard.world = (int)world;
-    for (unsigned r = 0; r < world && comm; ++r) shard.xbase[r] = comm->peer[r];
-    if (world > 1) DVS_TRY(comm_barrier(ctx, comm));  // every rank is here: exchange slots of earlier calls are dead
-    // trailing mode (dvs_count_select): the rows are still being produced on another stream; positions below
-    // `trail_limit` have been published.  Start once the first chunk (>= min_size positions) is there.
-    unsigned trail_limit = num;
-    if (trail) {
-        DVS_CUDA_TRY(cudaStreamWaitEvent(st, trail->first_ready, 0));
-        trail_limit = std::min(trail->limit0, num);
-        if (mode != DVS_MODE_NMOST || trail_limit < min_size) {  // nothing to gain / not enough rows yet: wait for all
-            DVS_CUDA_TRY(cudaStreamWaitEvent(st, trail->count_done, 0));
-            trail_limit = num;
-        }
-    }
-
-    // validity / panic flags of the records, needed on the host to form the initial set
-    std::vector<uint8_t> valid(f->nrec), err(f->nrec);
-    std::vector<double> err_total(f->nrec);
-    if (f->nrec) {
-        DVS_CUDA_TRY(cudaMemcpyAsync(valid.data(), f->valid.p, f->nrec, cudaMemcpyDeviceToHost, st));
-        DVS_CUDA_TRY(cudaMemcpyAsync(err.data(), f->err.p, f->nrec, cudaMemcpyDeviceToHost, st));
-        DVS_CUDA_TRY(cudaMemcpyAsync(err_total.data(), f->err_total.p, f->nrec * sizeof(double),
-                                     cudaMemcpyDeviceToHost, st));
-        DVS_CUDA_TRY(cudaStreamSynchronize(st));
-    }
-    // every record in `order` goes through KmerSeq::new -> entropy(); a failing sum check panics
-    // (trailing mode: the records published so far; all of them once the counting has finished, below)
-    for (uint32_t i = 0; i < trail_limit; ++i)
-        if (valid[order[i]] && err[order[i]]) {
-            set_error("cannot calculate entropy as frequency vector total %.17g!=1.0", err_total[order[i]]);
-            return DVS_ERR_VALUE;
-        }
-
-    std::vector<unsigned> init;  // records.rs:299-305: first min_size records, failures dropped
-    for (uint32_t i = 0; i < min_size; ++i)
-        if (valid[order[i]]) init.push_back(order[i]);
-    if (init.empty()) {
-        set_error("records cannot be empty");  // records.rs:28-30
-        return DVS_ERR_VALUE;
-    }
-    if (init.size() <= 1) {
-        set_error("must have > 1 KmerSeq");  // records.rs:227-230
-        return DVS_ERR_VALUE;
-    }
-    {   // duplicates in the initial set: the reference's Vec keeps both rows; keep that behaviour
-    }
-
-    const bool grow_mode = (mode != DVS_MODE_NMOST);
-    // max modes with max_size below the initial size (e.g. max_size < min_size, which only the reference's
-    // CLI rejects, cli.py:311): `size == max_size` never holds, so the set keeps growing as in
-    // records.rs:427-451 - every buffer is then sized for all `num` records
-    const bool unbounded = grow_mode && max_size < (uint32_t)init.size();
-    const unsigned cap = (unbounded ? num : std::max<unsigned>(std::max(min_size, max_size), (unsigned)init.size())) + 1;
-    SelState A, B;
-    DVS_TRY(A.alloc(dim, cap));
-    if (grow_mode) DVS_TRY(B.alloc(dim, cap));
-    DevBuf<uint8_t> is_member;
-    DevBuf<unsigned> d_order, d_init;
-    DVS_TRY(is_member.alloc(f->nrec));
-    DVS_TRY(d_order.alloc(num));
-    DVS_TRY(d_init.alloc(init.size()));
-    DVS_CUDA_TRY(cudaMemsetAsync(is_member.p, 0, f->nrec, st));
-    DVS_CUDA_TRY(cudaMemcpyAsync(d_order.p, order, num * sizeof(unsigned), cudaMemcpyHostToDevice, st));
-    DVS_CUDA_TRY(cudaMemcpyAsync(d_init.p, init.data(), init.size() * sizeof(unsigned), cudaMemcpyHostToDevice, st));
-    k_set_members<<<(unsigned)((init.size() + 255) / 256), 256, 0, st>>>(is_member.p, d_init.p, (unsigned)init.size(), 1);
-    DVS_LAUNCHED(ctx);
-
-    PhaseTimer pt(ctx, DVS_PHASE_SELECT);
-    Selector sel{ctx, f, dim, st, (SelScal*)ctx->pinned};
-    SelState* cur = &A;
-    SelState* alt = &B;
-    unsigned n = (unsigned)init.size();
-    DVS_TRY(sel.build(*cur, d_init.p, n, -1));
-
-    const unsigned window_max = std::max(64u, (unsigned)ctx->sm_count * 12u);
-    unsigned cursor = min_size;
-    unsigned accepts = 0;
-    unsigned window = 64;  // adaptive: grows while windows come back empty, shrinks after a hit
-    // DVS_SELECT_EXACT_ONLY=1 disables the bounded-error fast path (tests compare both)
-    const char* exact_env = getenv("DVS_SELECT_EXACT_ONLY");
-    const bool use_fast = !(exact_env && exact_env[0] == '1');
-    unsigned exact_evals = 0;
-    const unsigned window_max_dev = std::max(64u, (unsigned)ctx->sm_count * 4u);  // grid of a device-driven scan
-    const char* dev_env = getenv("DVS_SELECT_HOST_LOOP");
-    const bool use_dev = use_fast && !(dev_env && dev_env[0] == '1');
-    constexpr int kRoundsPerBatch = 32;
-    // DVS_SELECT_PERSIST=0 keeps the two-launches-per-round form, =1 the global-state persistent kernel
-    // (A/B measurements, fallbacks); default: SM-replicated rounds when the state fits in shared memory
-    // DVS_SELECT_GRID: CTAs of the persistent kernels (tests run several ranks on ONE GPU: their kernels must be
-    // co-resident, so each takes a share of the SMs)
-    const char* grid_env = getenv("DVS_SELECT_GRID");
-    const unsigned grid_cap = grid_env && atoi(grid_env) > 0 ? (unsigned)atoi(grid_env) : 0xFFFFFFFFu;
-    const char* per_env = getenv("DVS_SELECT_PERSIST");
-    int coop = 0, per_sm = 0, per_sm2 = 0;
-    cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, ctx->device);
-    if (coop && cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sel_persist, kFastThreads, 0) != cudaSuccess)
-        per_sm = 0;
-    const bool use_persist = use_dev && coop && per_sm > 0 && !(per_env && per_env[0] == '0');
-    const unsigned persist_grid = std::min((unsigned)ctx->sm_count * (unsigned)std::min(per_sm, 2), std::max(1u, std::min(grid_cap, 0x7FFFFFFFu)));
-    bool sm_ok = use_persist && !(per_env && per_env[0] == '1') && dim <= kSmMaxDim;
-    if (sm_ok) {
-        sm_ok = cudaFuncSetAttribute(k_sel_persist_sm_full, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     (int)sizeof(SmShared)) == cudaSuccess &&
-                cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm2, k_sel_persist_sm_full, kFastThreads,
-                                                              sizeof(SmShared)) == cudaSuccess &&
-                per_sm2 > 0;
-        (void)cudaGetLastError();
-    }
-    const unsigned sm_grid = std::min(std::min<unsigned>((unsigned)ctx->sm_count, kSmMaxGrid), grid_cap);
-    const int slim_threads = 128 * (trail_shape() + 1);
-    const auto k_slim = slim_threads == 384 ? SlimKernel<384>::fn : (slim_threads == 256 ? SlimKernel<256>::fn : SlimKernel<128>::fn);
-    bool slim_ok = false;
-    if (trail && sm_ok) {
-        slim_ok = cudaFuncSetAttribute(k_slim, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       (int)sizeof(SmSharedSlim)) == cudaSuccess &&
-                  cudaFuncSetAttribute(k_slim, cudaFuncAttributePreferredSharedMemoryCarveout,
-                                       (int)cudaSharedmemCarveoutMaxShared) == cudaSuccess;
-        (void)cudaGetLastError();
-    }
-    DevBuf<SlicePart> d_slparts;  // k_sel_persist: partial sums of sliced vectors and their arrival tickets
-    DevBuf<unsigned> d_slticks;
-    DevBuf<SmPart> d_spart, d_upart, d_dpart;
-    if (sm_ok) {
-        DVS_TRY(d_spart.alloc(2 * kSmMaxGrid));
-        DVS_TRY(d_upart.alloc(kSmMaxN + 1));
-        DVS_TRY(d_dpart.alloc(3));  // the leader's broadcasts: scan decision (double buffered), update result
-    }
-    // batched grow attempts (see k_grow_eval): scratch for a window of candidates; DVS_SELECT_GROW_BATCH=0
-    // keeps one host-driven attempt per candidate
-    const char* gb_env = getenv("DVS_SELECT_GROW_BATCH");
-    const bool use_grow_batch = use_fast && grow_mode && !(gb_env && gb_env[0] == '0');
-    const unsigned kGrowWindowMax = 64 * world;
-    SelState fresh;  // clone(): the members re-summed in order (S, E), refreshed whenever the set changes
-    DevBuf<FastSum> d_gparts;
-    DevBuf<double> d_gmd, d_gmb;
-    DevBuf<SelScal> d_gscratch;
-    DevBuf<unsigned> d_ginteresting;
-    bool fresh_valid = false;
-    unsigned grow_window = 16;
-    if (use_grow_batch && n != max_size) {
-        DVS_TRY(fresh.alloc(dim, cap));
-        DVS_TRY(d_gparts.alloc((size_t)kGrowWindowMax * (cap + 3)));
-        DVS_TRY(d_gmd.alloc((size_t)kGrowWindowMax * cap));
-        DVS_TRY(d_gmb.alloc((size_t)kGrowWindowMax * cap));
-        DVS_TRY(d_gscratch.alloc(kGrowWindowMax));  // (indexed by the window offset)
-        DVS_TRY(d_ginteresting.alloc(1));
-    }
-    unsigned fresh_n = 0;
-    const SelState* fresh_of = nullptr;
-    int fresh_which = -1;
-    bool single_candidate = false;  // the grow filter has already isolated the candidate at `cursor`
-    // while the set grows at almost every candidate (e.g. cov right after the start) the filter skips
-    // nothing: after two such windows in a row it is bypassed for 1, 2, 4, 8 candidates
-    unsigned filter_streak = 0, filter_bypass = 0;
-    while (cursor < num) {
-        if (use_grow_batch && n != max_size && !single_candidate && filter_bypass > 0) {
-            --filter_bypass;
-            single_candidate = true;  // straight to the host path for this candidate
-            continue;
-        }
-        if (use_grow_batch && n != max_size && !single_candidate) {
-            if (!fresh_valid || fresh_n != n || fresh_of != cur || fresh_which != cur->which) {
-                k_sel_sum<<<sel.vec_grid(), 256, 0, st>>>(f->freqs.p, f->entropy.p, dim, cur->members(), n, -1, fresh.S(),
-                                                          fresh.members(), fresh.sc.p);
-                DVS_LAUNCHED(ctx);
-                fresh_valid = true;
-                fresh_n = n;
-                fresh_of = cur;
-                fresh_which = cur->which;
-            }
-            const unsigned W = std::min(grow_window, num - cursor);
-            DVS_CUDA_TRY(cudaMemsetAsync(d_ginteresting.p, 0xFF, sizeof(unsigned), st));
-            // candidate-sharded: this GPU evaluates the window candidates c with (cursor + c) % world == rank
-            const unsigned gc0 = (rank + world - cursor % world) % world;
-            const unsigned Wloc = W > gc0 ? (W - gc0 + world - 1) / world : 0;
-            if (Wloc) {
-                k_grow_eval<<<dim3(n + 3, Wloc), kFastThreads, 0, st>>>(f->freqs.p, dim, cur->S(), cur->members(), cur->sc.p,
-                                                                        fresh.S(), f->valid.p, is_member.p, d_order.p,
-                                                                        cursor, d_gparts.p, gc0, world);
-                DVS_LAUNCHED(ctx);
-                k_grow_decide<<<Wloc, kFastThreads, 0, st>>>(f->entropy.p, dim, cur->members(), cur->sc.p, fresh.sc.p,
-                                                             f->valid.p, is_member.p, d_order.p, cursor, d_gparts.p, d_gmd.p,
-                                                             d_gmb.p, cap, d_gscratch.p, d_ginteresting.p,
-                                                             mode == DVS_MODE_MAX_COV ? 1 : 0, gc0, world);
-                DVS_LAUNCHED(ctx);
-            }
-            if (world > 1) DVS_TRY(comm_min_u32(ctx, comm, d_ginteresting.p, d_ginteresting.p));
-            unsigned* h_fi = reinterpret_cast<unsigned*>(reinterpret_cast<char*>(ctx->pinned) + sizeof(SelScal));
-            DVS_CUDA_TRY(cudaMemcpyAsync(h_fi, d_ginteresting.p, sizeof(unsigned), cudaMemcpyDeviceToHost, st));
-            DVS_CUDA_TRY(cudaStreamSynchronize(st));
-            const unsigned fi = *h_fi;
-            if (fi == kNone) {  // the whole window was certainly rejected
-                cursor += W;
-                grow_window = std::min(grow_window * 2u, kGrowWindowMax);
-                continue;
-            }
-            grow_window = std::max(4u, std::min(kGrowWindowMax, 2u * (fi - cursor + 1u)));
-            if (fi == cursor) {
-                if (++filter_streak >= 2) filter_bypass = 1u << std::min(filter_streak - 2u, 3u);
-            } else {
-                filter_streak = 0;
-            }
-            cursor = fi;  // everything before it is certainly rejected; the host path below takes this one
-            single_candidate = true;
-            continue;
-        }
-        if (trail && trail_limit < num && !use_persist) {  // only the persistent kernel knows how to trail
-            DVS_CUDA_TRY(cudaStreamWaitEvent(st, trail->count_done, 0));
-            trail_limit = num;
-        }
-        if (use_persist && (!grow_mode || n == max_size)) {
-            // every remaining round in one cooperative launch (until done, or halted for the host)
-            const bool use_sm = sm_ok && n <= kSmMaxN;
-            // trailing rounds need the slim SM-replicated kernel; anything else waits for the counting to finish
-            const bool dedicated = trail_shape() == 3;  // the selection owns whole SMs (fused.cuh)
-            const bool trailing = trail && trail_limit < num && use_sm && world == 1 &&
-                                  (dedicated || (slim_ok && n <= kSmSlimMaxN));
-            if (trail && trail_limit < num && !trailing) {
-                DVS_CUDA_TRY(cudaStreamWaitEvent(st, trail->count_done, 0));
-                trail_limit = num;
-            }
-            const unsigned grid = (trailing && dedicated) ? std::min(sm_grid, trail_sms(ctx->sm_count))
-                                                           : (use_sm ? sm_grid : persist_grid);
-            k_sel_set_dev<<<1, 1, 0, st>>>(cur->sc.p, cursor, std::min(window, grid * world), grid * world, num, accepts,
-                                           (unsigned)cur->which);
-            if (comm) {
-                shard.tag_base = (unsigned)((++comm->sel_tag_base) << 20);
-                DVS_TRY(comm_host_rendezvous(ctx, comm));  // (ranks sharing one GPU only)
-            }
-            DVS_LAUNCHED(ctx);
-            const double* a_F = f->freqs.p;
-            const double* a_H = f->entropy.p;
-            uint64_t a_dim = dim;
-            double *a_S0 = cur->Sbuf[0].p, *a_S1 = cur->Sbuf[1].p;
-            unsigned *a_M0 = cur->membuf[0].p, *a_M1 = cur->membuf[1].p;
-            uint8_t* a_mem = is_member.p;
-            double *a_md = cur->mdelta.p, *a_mb = cur->mbound.p;
-            SelScal* a_sc = cur->sc.p;
-            const uint8_t* a_valid = f->valid.p;
-            const unsigned* a_order = d_order.p;
-            unsigned a_rounds = world > 1 ? 0xFFFF0u : 0x7fffffffu;  // (exchange tags of one launch are 20 bits)
-            unsigned long long* a_trace = nullptr;
-            DevBuf<unsigned long long> d_trace;
-            const char* tr_env = getenv("DVS_SELECT_TRACE");
-            const char* tra_env = getenv("DVS_SELECT_TRACE_ALL");  // raw u64 [256 rounds][8 slots][256 CTAs]
-            int a_trace_all = (use_sm && tra_env && tra_env[0]) ? 1 : 0;
-            const size_t trace_len = a_trace_all ? (size_t)256 * kSmTraceSlots * kSmMaxGrid : 2048;
-            if (a_trace_all) tr_env = nullptr;
-            if ((tr_env && tr_env[0]) || a_trace_all) {
-                DVS_TRY(d_trace.alloc(trace_len));
-                DVS_CUDA_TRY(cudaMemsetAsync(d_trace.p, 0, trace_len * sizeof(unsigned long long), st));
-                a_trace = d_trace.p;
-            }
-            if (use_sm) {
-                unsigned a_dim32 = (unsigned)dim;
-                double* a_S = cur->S();
-                unsigned* a_M = cur->members();
-                SmPart *a_sp = d_spart.p, *a_up = d_upart.p, *a_dp = d_dpart.p;
-                DVS_CUDA_TRY(cudaMemsetAsync(d_dpart.p, 0, 3 * sizeof(SmPart), st));
-                // exchange tags restart at 1 in every launch
-                DVS_CUDA_TRY(cudaMemsetAsync(d_spart.p, 0, 2 * kSmMaxGrid * sizeof(SmPart), st));
-                DVS_CUDA_TRY(cudaMemsetAsync(d_upart.p, 0, (kSmMaxN + 1) * sizeof(SmPart), st));
-                const unsigned* a_ready = trailing ? trail->d_ready : nullptr;
-                unsigned a_limit0 = trail_limit;
-                void* args[] = {&a_F, &a_H, &a_dim32, &a_S, &a_M, &a_mem, &a_md, &a_mb, &a_sc, &a_valid, &a_order,
-                                &a_sp, &a_up, &a_dp, &a_trace, &a_trace_all, &shard, &a_ready, &a_limit0};
-                if (trailing && dedicated) {
-                    if (!ctx->stream_hi) {
-                        int lo_p = 0, hi_p = 0;
-                        DVS_CUDA_TRY(cudaDeviceGetStreamPriorityRange(&lo_p, &hi_p));
-                        DVS_CUDA_TRY(cudaStreamCreateWithPriority(&ctx->stream_hi, cudaStreamNonBlocking, hi_p));
-                        DVS_CUDA_TRY(cudaEventCreateWithFlags(&ctx->ev_hi_in, cudaEventDisableTiming));
-                        DVS_CUDA_TRY(cudaEventCreateWithFlags(&ctx->ev_hi_out, cudaEventDisableTiming));
-                    }
-                    // 512 threads x 128 registers: one CTA fills an SM's register file, so these CTAs take whole SMs -
-                    // the ones the counting CTAs of the launch in flight leave when it ends (the higher stream priority
-                    // puts them ahead of the next counting launch's CTAs)
-                    DVS_CUDA_TRY(cudaEventRecord(ctx->ev_hi_in, st));
-                    DVS_CUDA_TRY(cudaStreamWaitEvent(ctx->stream_hi, ctx->ev_hi_in, 0));
-                    k_sel_persist_sm_full<<<grid, kFastThreads, sizeof(SmShared), ctx->stream_hi>>>(
-                        a_F, a_H, a_dim32, a_S, a_M, a_mem, a_md, a_mb, a_sc, a_valid, a_order, a_sp, a_up, a_dp, a_trace,
-                        a_trace_all, shard, a_ready, a_limit0);
-                    DVS_CUDA_TRY(cudaGetLastError());
-                    DVS_CUDA_TRY(cudaEventRecord(ctx->ev_hi_out, ctx->stream_hi));
-                    DVS_CUDA_TRY(cudaStreamWaitEvent(st, ctx->ev_hi_out, 0));
-                } else if (trailing) {
-                    // a plain launch, made when every SM holds a counting CTA: beside it exactly one of these CTAs
-                    // fits (registers), so they land one per SM.  Launched between two counting launches they
-                    // would pack three to an SM and keep the counting off a third of the GPU.
-                    k_wait_resident<<<1, 1, 0, st>>>(trail->d_resident, std::min<unsigned>(grid, (unsigned)ctx->sm_count),
-                                                     trail->d_ready, num);
-                    DVS_LAUNCHED(ctx);
-                }
-                if (trailing && dedicated) {
-                } else if (trailing)
-                    k_slim<<<grid, slim_threads, sizeof(SmSharedSlim), st>>>(
-                        a_F, a_H, a_dim32, a_S, a_M, a_mem, a_md, a_mb, a_sc, a_valid, a_order, a_sp, a_up, a_dp, a_trace,
-                        a_trace_all, shard, a_ready, a_limit0);
-                else
-                    DVS_CUDA_TRY(cudaLaunchCooperativeKernel((void*)k_sel_persist_sm_full, dim3(grid), dim3(kFastThreads),
-                                                             args, sizeof(SmShared), st));
-            } else {
-                // DVS_SELECT_SLICES (A/B measurements): 0 = one CTA per candidate / member slot, 1 = candidates of a short
-                // window are cut into slices (default), 2 = member slots of the update too (measured slower: a slice
-                // repeats the slot's set-up and pays a fence + ticket, 55 us against 33 us per update at k = 8, n = 100)
-                const char* sl_env = getenv("DVS_SELECT_SLICES");
-                unsigned a_slice_mode = sl_env ? (unsigned)atoi(sl_env) : 1u;
-                if (!d_slparts.p && a_slice_mode) {
-                    const size_t slots = std::max<size_t>(grid, (size_t)cap + 1);
-                    DVS_TRY(d_slparts.alloc(slots * kMaxSlices));
-                    DVS_TRY(d_slticks.alloc(slots));
-                    DVS_CUDA_TRY(cudaMemsetAsync(d_slticks.p, 0, slots * sizeof(unsigned), st));
-                }
-                SlicePart* a_parts = d_slparts.p;
-                unsigned* a_ticks = d_slticks.p;
-                void* args[] = {&a_F, &a_H, &a_dim, &a_S0, &a_S1, &a_M0, &a_M1, &a_mem, &a_md, &a_mb, &a_sc, &a_valid,
-                                &a_order, &a_rounds, &a_trace, &shard, &a_parts, &a_ticks, &a_slice_mode};
-                DVS_CUDA_TRY(cudaLaunchCooperativeKernel((void*)k_sel_persist, dim3(grid), dim3(kFastThreads), args, 0, st));
-            }
-            ctx->launches++;
-            DVS_TRY(sel.read(*cur));
-            if (a_trace && a_trace_all) {
-                std::vector<unsigned long long> tr(trace_len);
-                DVS_CUDA_TRY(cudaMemcpy(tr.data(), a_trace, trace_len * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-                if (FILE* fp = fopen(tra_env, "wb")) {
-                    fwrite(tr.data(), sizeof(unsigned long long), trace_len, fp);
-                    fclose(fp);
-                }
-            } else if (a_trace) {  // phase timeline of CTA 0 to the file named by DVS_SELECT_TRACE
-                std::vector<unsigned long long> tr(2048);
-                DVS_CUDA_TRY(cudaMemcpy(tr.data(), a_trace, 2048 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-                if (FILE* fp = fopen(tr_env, "a")) {
-                    const int slots = use_sm ? kSmTraceSlots : 4, used = use_sm ? 7 : 4;
-                    fprintf(fp, use_sm ? "# round scan_ns gather_ns decide_ns update_ns gather2_ns finalize_ns next_ns (CTA 0)\n"
-                                       : "# round scan_ns wait1_ns update_ns wait2_ns (CTA 0; wait = grid barrier incl. the slowest CTA)\n");
-                    for (int r = 0; (r + 1) * slots < 2048 && tr[slots * (r + 1)]; ++r) {
-                        fprintf(fp, "%d", r);
-                        for (int q = 0; q + 1 < used; ++q) fprintf(fp, " %llu", tr[slots * r + q + 1] - tr[slots * r + q]);
-                        fprintf(fp, " %llu\n", tr[slots * (r + 1)] - tr[slots * r + used - 1]);
-                    }
-                    fclose(fp);
-                }
-            }
-            const SelScal hd = *sel.h_sc;
-            if (hd.panic) return panic_error(hd);
-            if (trailing) {
-                ctx->last_trail_accepts += hd.accepts - accepts;
-                ++ctx->last_trail_launches;
-                std::vector<unsigned> smid(grid);
-                DVS_CUDA_TRY(cudaMemcpyAsync(smid.data(), trail->d_ready + kTrailSmidOff, grid * sizeof(unsigned),
-                                             cudaMemcpyDeviceToHost, st));
-                DVS_CUDA_TRY(cudaStreamSynchronize(st));
-                std::sort(smid.begin(), smid.end());
-                const unsigned distinct = (unsigned)(std::unique(smid.begin(), smid.end()) - smid.begin());
-                ctx->last_trail_sms = std::min(ctx->last_trail_sms, distinct);
-            }
-            cursor = hd.cursor;
-            window = hd.window;
-            accepts = hd.accepts;
-            cur->which = (int)hd.which;
-            if (trailing) trail_limit = std::max(trail_limit, std::min(hd.limit, num));
-            if (!hd.halt) continue;  // finished (or, trailing, everything is published: the stand-alone kernel goes on)
-            DVS_TRY(sel.reset_scan(*cur));
-            if (cursor >= num) break;
-        } else if (use_dev && world == 1 && (!grow_mode || n == max_size)) {
-            // Device-driven rounds: scan + decide + replace/update are enqueued kRoundsPerBatch times
-            // without any read-back; the kernels carry cursor / window / accepts in the scalar block
-            // and stop doing work once they halt (undecided within the error bound) or finish.
-            k_sel_set_dev<<<1, 1, 0, st>>>(cur->sc.p, cursor, std::min(window, window_max_dev), window_max_dev, num,
-                                           accepts, (unsigned)cur->which);
-            DVS_LAUNCHED(ctx);
-            for (int r = 0; r < kRoundsPerBatch; ++r) {
-                k_sel_scan_dev<<<window_max_dev, kFastThreads, 0, st>>>(
-                    f->freqs.p, f->entropy.p, dim, cur->Sbuf[0].p, cur->Sbuf[1].p, cur->membuf[0].p, cur->membuf[1].p,
-                    cur->sc.p, f->valid.p, is_member.p, d_order.p);
-                DVS_LAUNCHED(ctx);
-                k_sel_round_dev<<<n + 1, kFastThreads, 0, st>>>(
-                    f->freqs.p, f->entropy.p, dim, cur->Sbuf[0].p, cur->Sbuf[1].p, cur->membuf[0].p, cur->membuf[1].p,
-                    is_member.p, cur->mdelta.p, cur->mbound.p, cur->sc.p, d_order.p);
-                DVS_LAUNCHED(ctx);
-            }
-            DVS_TRY(sel.read(*cur));
-            const SelScal hd = *sel.h_sc;
-            if (hd.panic) return panic_error(hd);
-            cursor = hd.cursor;
-            window = hd.window;
-            accepts = hd.accepts;
-            cur->which = (int)hd.which;
-            if (!hd.halt) continue;  // finished, or simply out of enqueued rounds
-            // halted: one host-driven iteration below resolves the undecided state / candidate exactly
-            DVS_TRY(sel.reset_scan(*cur));
-            if (cursor >= num) break;
-        }
-        if (cursor >= trail_limit) {  // (trailing) nothing published beyond the cursor: wait for all of it
-            DVS_CUDA_TRY(cudaStreamWaitEvent(st, trail->count_done, 0));
-            trail_limit = num;
-        }
-        const unsigned count = single_candidate ? 1u : std::min(window, trail_limit - cursor);
-        single_candidate = false;
-        SelScal h;
-        unsigned pos = kNone;
-        if (use_fast) {
-            DVS_TRY(sel.scan_fast(*cur, is_member.p, d_order.p, cursor, count));
-            DVS_TRY(sel.read(*cur));
-            h = *sel.h_sc;
-            if (h.panic) return panic_error(h);
-            if (h.state_unsure) {
-                // the last fast update could not certify lowest_index / a sum check: redo it exactly and
-                // re-score the window against the now certain state
-                DVS_TRY(sel.update(*cur, n));
-                ++exact_evals;
-                continue;
-            }
-            if (h.first_unsure < h.first_true) {
-                // an undecided candidate comes before the first certain acceptance: decide it exactly
-                const unsigned pu = h.first_unsure;
-                if (!h.exact) DVS_TRY(sel.update(*cur, n));
-                DVS_TRY(sel.scan(*cur, f, is_member.p, d_order.p, pu, 1, nullptr));
-                DVS_TRY(sel.read(*cur));
-                h = *sel.h_sc;
-                ++exact_evals;
-                if (h.panic) return panic_error(h);
-                if (h.first_panic == pu) {
-                    set_error("cannot calculate entropy as frequency vector total !=1.0 (candidate at position %u)", pu);
-                    return DVS_ERR_VALUE;
-                }
-                if (h.first_true != pu) {  // rejected by the exact evaluation: carry on after it
-                    DVS_TRY(sel.reset_scan(*cur));
-                    cursor = pu + 1;
-                    continue;
-                }
-                pos = pu;
-            } else if (h.first_true != kNone) {
-                pos = h.first_true;
-            }
-        } else {
-            DVS_TRY(sel.scan(*cur, f, is_member.p, d_order.p, cursor, count, nullptr));
-            DVS_TRY(sel.read(*cur));
-            h = *sel.h_sc;
-            if (h.panic) return panic_error(h);
-            if (h.first_panic != kNone && h.first_panic <= h.first_true) {
-                set_error("cannot calculate entropy as frequency vector total !=1.0 (candidate at position %u)",
-                          h.first_panic);
-                return DVS_ERR_VALUE;
-            }
-            pos = h.first_true;
-        }
-        if (pos == kNone) {
-            cursor += count;
-            window = std::min(window * 2, window_max);
-            continue;
-        }
-        const unsigned row = order[pos];
-        window = std::max(64u, std::min(window_max, 2 * (pos - cursor + 1)));
-        cursor = pos + 1;
-        if (!grow_mode || n == max_size) {  // replace_lowest, records.rs:111-118
-            DVS_TRY(use_fast ? sel.replace_fast(*cur, n, row, is_member.p) : sel.replace(*cur, n, row, is_member.p));
-            ++accepts;
-            continue;
-        }
-        // records.rs:434-451: nw = clone(); nw.push(rec); keep whichever has the larger statistic.
-        // First try with the bounded-error kernels: the comparison is decided from them only when it
-        // holds for every admissible error; otherwise both states are evaluated by the exact kernel.
-        const bool use_cov = (mode == DVS_MODE_MAX_COV);
-        int decided = -1;  // -1 undecided, 0 discard candidate, 1 adopt the grown set
-        if (use_fast && !h.state_unsure) {
-            DVS_TRY(sel.build_fast(*alt, cur->members(), n, (int)row));
-            DVS_TRY(sel.read(*alt));
-            const SelScal hf = *sel.h_sc;
-            if (hf.panic) return panic_error(hf);
-            if (!hf.state_unsure) {
-                const double sa_f = use_cov ? h.cov : h.stdv, ba = h.exact ? 0.0 : (use_cov ? h.cov_bound : h.std_bound);
-                const double sb_f = use_cov ? hf.cov : hf.stdv, bb = use_cov ? hf.cov_bound : hf.std_bound;
-                if (sb_f - bb > sa_f + ba) decided = 1;
-                else if (sb_f + bb < sa_f - ba) decided = 0;
-            }
-        }
-        if (decided == 1) {
-            std::swap(cur, alt);
-            ++n;
-            ++accepts;
-            uint8_t one = 1;
-            DVS_CUDA_TRY(cudaMemcpyAsync(is_member.p + row, &one, 1, cudaMemcpyHostToDevice, st));
-            DVS_CUDA_TRY(cudaStreamSynchronize(st));
-            continue;
-        }
-        if (decided == 0) {
-            DVS_TRY(sel.reset_scan(*cur));
-            continue;
-        }
-        if (use_fast) ++exact_evals;
-        if (!h.exact) {
-            DVS_TRY(sel.update(*cur, n));
-            DVS_TRY(sel.read(*cur));
-            h = *sel.h_sc;
-            if (h.panic) return panic_error(h);
-        }
-        DVS_TRY(sel.build(*alt, cur->members(), n, (int)row));
-        DVS_TRY(sel.read(*alt));
-        const SelScal hb = *sel.h_sc;
-        if (hb.panic) return panic_error(hb);
-        const double sa = use_cov ? h.cov : h.stdv;
-        const double sb = use_cov ? hb.cov : hb.stdv;
-        if (sb > sa) {
-            std::swap(cur, alt);
-            ++n;
-            ++accepts;
-            uint8_t one = 1;
-            DVS_CUDA_TRY(cudaMemcpyAsync(is_member.p + row, &one, 1, cudaMemcpyHostToDevice, st));
-            DVS_CUDA_TRY(cudaStreamSynchronize(st));
-        } else {
-            DVS_TRY(sel.reset_scan(*cur));  // candidate discarded: re-arm the min-index reduction of `cur`
-        }
-    }
-    if (trail) {  // the records that were not published when the selection started: the reference's panic check
-        DVS_CUDA_TRY(cudaStreamWaitEvent(st, trail->count_done, 0));
-        DVS_CUDA_TRY(cudaMemcpyAsync(valid.data(), f->valid.p, f->nrec, cudaMemcpyDeviceToHost, st));
-        DVS_CUDA_TRY(cudaMemcpyAsync(err.data(), f->err.p, f->nrec, cudaMemcpyDeviceToHost, st));
-        DVS_CUDA_TRY(cudaMemcpyAsync(err_total.data(), f->err_total.p, f->nrec * sizeof(double), cudaMemcpyDeviceToHost, st));
-        DVS_CUDA_TRY(cudaStreamSynchronize(st));
-        for (uint32_t i = 0; i < num; ++i)
-            if (valid[order[i]] && err[order[i]]) {
-                set_error("cannot calculate entropy as frequency vector total %.17g!=1.0", err_total[order[i]]);
-                return DVS_ERR_VALUE;
-            }
-    }
-    DVS_TRY(sel.read(*cur));
-    if (!sel.h_sc->exact || sel.h_sc->state_unsure) DVS_TRY(sel.update(*cur, n));  // reported numbers are exact
-    ctx->last_exact_evals = exact_evals;
-    DVS_TRY(sel.read(*cur));
-    const SelScal h = *sel.h_sc;
-    if (h.panic) return panic_error(h);
-    if (sel_idx) DVS_CUDA_TRY(cudaMemcpyAsync(sel_idx, cur->members(), n * sizeof(unsigned), cudaMemcpyDeviceToHost, st));
-    if (sel_delta) DVS_CUDA_TRY(cudaMemcpyAsync(sel_delta, cur->mdelta.p, n * sizeof(double), cudaMemcpyDeviceToHost, st));
-    DVS_CUDA_TRY(cudaStreamSynchronize(st));
-    if (stats5) {
-        stats5[0] = h.total_jsd;
-        stats5[1] = h.mean;
-        stats5[2] = h.stdv;
-        stats5[3] = h.cov;
-        stats5[4] = h.E;
-    }
-    *size_out = n;
-    ctx->last_accepts = accepts;
-    if (world > 1) DVS_TRY(comm_check_error(ctx, comm, "dvs_select_sharded"));
-    return DVS_OK;
-}
-
-}  // extern "C"
-namespace dvs {
-int select_with_trail(dvs_ctx* ctx, const dvs_kfreqs* f, const uint32_t* order, uint32_t num, int mode, uint32_t min_size,
-                      uint32_t max_size, uint32_t* sel_idx, double* sel_delta, double* stats5, uint32_t* size_out,
-                      const TrailArgs* trail) {
-    return select_core(ctx, nullptr, f, order, num, mode, min_size, max_size, sel_idx, sel_delta, stats5, size_out, trail);
-}
-}  // namespace dvs
 extern "C" {
 
 int dvs_select(dvs_ctx* ctx, const dvs_kfreqs* f, const uint32_t* order, uint32_t num, int mode, uint32_t min_size,

@@ -1,4 +1,4 @@
-// select_fast.cuh — bounded-error selection kernels: term evaluation, scan / update / replace, device-driven and cooperative rounds
+// select_fast.cuh — bounded-error selection kernels: term evaluation, scan / update / replace, cooperative rounds
 // Part of select.cu (included inside namespace dvs, after the exact kernels); split out for readability only.
 #pragma once
 
@@ -155,8 +155,8 @@ __device__ FastSum block_entropy_ilp(unsigned lo, unsigned hi, Num num, const Fa
     return r;
 }
 
-// The same evaluation for the kernels that keep their state in global memory (host-driven and
-// device-driven rounds, the cooperative kernel, the batched grow attempts — the k >= 7 paths): m_i =
+// The same evaluation for the kernels that keep their state in global memory (host-driven rounds, the
+// cooperative kernel, the batched grow attempts — the k >= 7 paths): m_i =
 // num(i) / divisor, optionally clamped (<= EPS -> 0).  Stages the log2 table itself; divisors beyond the
 // range the exact division was verified for, and vectors longer than 2^30, take the one-element-at-a-time
 // form with __ddiv_rn (same values either way).
@@ -373,23 +373,6 @@ k_sel_scan_fast(const double* __restrict__ F, const double* __restrict__ H, uint
     scan_fast_body(F, H, dim, S, sc, load_scan_scal(sc, members), valid, is_member, order, pos0 + blockIdx.x);
 }
 
-// device-driven window: cursor / window / current buffer come from the scalar block, so the host can
-// enqueue many rounds back to back without reading anything back
-__global__ void __launch_bounds__(kFastThreads)
-k_sel_scan_dev(const double* __restrict__ F, const double* __restrict__ H, uint64_t dim, const double* __restrict__ S0,
-               const double* __restrict__ S1, const unsigned* __restrict__ M0, const unsigned* __restrict__ M1,
-               SelScal* sc, const uint8_t* __restrict__ valid, const uint8_t* __restrict__ is_member,
-               const unsigned* __restrict__ order) {
-    if (sc->halt) return;
-    const unsigned cursor = sc->cursor, num = sc->num;
-    if (cursor >= num) return;
-    const unsigned count = min(sc->window, num - cursor);
-    if (blockIdx.x >= count) return;
-    const unsigned w = sc->which;
-    scan_fast_body(F, H, dim, w ? S1 : S0, sc, load_scan_scal(sc, w ? M1 : M0), valid, is_member, order,
-                   cursor + blockIdx.x);
-}
-
 // fast total_jsd + get_lowest_record_index: same shape as k_sel_update.  Leaves approximate
 // total_jsd (with total_bound) and mdelta, and lowest_index only if it is certain.
 __global__ void __launch_bounds__(kFastThreads)
@@ -530,43 +513,6 @@ k_sel_replace_update_fast(const double* __restrict__ F, const double* __restrict
                           SelScal* sc, unsigned cand_row) {
     replace_update_fast_body(F, H, dim, S_in, S_out, m_in, m_out, is_member, mdelta, mbound, sc, cand_row, kNone, 0u,
                              blockIdx.x, sc->n, sc->lowest, sc->E);
-}
-
-// One device-driven round after k_sel_scan_dev: every CTA takes the same decision from the scalar
-// block (only the last CTA to finish modifies it): accept the first certain candidate (fused
-// replace + update), advance past an empty window, or halt for the host when the first
-// interesting candidate / the state could not be decided within the error bound.
-__global__ void __launch_bounds__(kFastThreads)
-k_sel_round_dev(const double* __restrict__ F, const double* __restrict__ H, uint64_t dim, double* __restrict__ S0,
-                double* __restrict__ S1, unsigned* __restrict__ M0, unsigned* __restrict__ M1,
-                uint8_t* __restrict__ is_member, double* __restrict__ mdelta, double* __restrict__ mbound, SelScal* sc,
-                const unsigned* __restrict__ order) {
-    __shared__ unsigned s_last2;
-    if (sc->halt) return;
-    const unsigned cursor = sc->cursor, num = sc->num;
-    if (cursor >= num) return;
-    const unsigned window = sc->window, count = min(window, num - cursor);
-    const unsigned ft = sc->first_true, fu = sc->first_unsure, su = sc->state_unsure, n = sc->n;
-    if (!su && !(fu < ft) && ft != kNone) {
-        const unsigned w = sc->which;
-        replace_update_fast_body(F, H, dim, w ? S1 : S0, w ? S0 : S1, w ? M1 : M0, w ? M0 : M1, is_member, mdelta,
-                                 mbound, sc, order[ft], ft, cursor, blockIdx.x, n, sc->lowest, sc->E);
-        return;
-    }
-    if (threadIdx.x == 0) {
-        __threadfence();
-        s_last2 = (atomicAdd(&sc->ticket, 1u) == n) ? 1u : 0u;
-    }
-    __syncthreads();
-    if (s_last2 && threadIdx.x == 0) {
-        sc->ticket = 0;
-        if (su || fu < ft) {
-            sc->halt = 1u;
-        } else {  // empty window
-            sc->cursor = cursor + count;
-            sc->window = min(window * 2u, sc->window_max);
-        }
-    }
 }
 
 // ---- sliced evaluation for the cooperative kernel (vectors that do not fit shared memory: k >= 7) ----
@@ -725,8 +671,9 @@ __device__ __forceinline__ void replace_update_sliced_body(
 // All device-driven rounds in ONE cooperative launch: the CTAs stay resident, a round is
 //   scan (one candidate per CTA and pass) | grid barrier | accept: fused replace + update over n+1 member
 //   slots, or advance / halt | grid barrier
-// with the same scalar-block protocol as k_sel_scan_dev / k_sel_round_dev, so the host loop and the exact
-// fallbacks are unchanged.  Against the two-launches-per-round form this removes the launch and block
+// The kernel carries cursor / window / accepts / which in the scalar block and halts for the host when the
+// first interesting candidate or the state cannot be decided within the error bound; the host then resolves
+// it exactly and launches again.  Against two launches per round this removes the launch and block
 // scheduling latency of ~2 x 350 dependent kernels per nmost run and loads the round's scalars once per
 // CTA instead of through chains of dependent global loads.
 struct RoundScal {

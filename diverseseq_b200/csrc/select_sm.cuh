@@ -54,9 +54,7 @@ struct SmSharedT {
     unsigned ft, fu, unsure, xft, xfu, dead, limit;
     double2 ltab[64];  // glibc log2 table {1/c, log2 c}
 };
-using SmShared = SmSharedT<kSmMaxN, kSmChunk>;           // stand-alone kernel: ~105 KB
-constexpr unsigned kSmSlimMaxN = 256, kSmSlimChunk = 1280;
-using SmSharedSlim = SmSharedT<kSmSlimMaxN, kSmSlimChunk>;  // trailing kernel beside the counting CTA: ~62 KB
+using SmShared = SmSharedT<kSmMaxN, kSmChunk>;  // ~105 KB
 
 __device__ __forceinline__ void sm_st128(void* p, unsigned long long lo, unsigned long long hi) {
     asm volatile("{ .reg .b128 v; mov.b128 v, {%1, %2}; st.relaxed.gpu.global.b128 [%0], v; }" ::"l"(p), "l"(lo), "l"(hi)
@@ -130,9 +128,8 @@ __device__ __forceinline__ unsigned sm_finalize(double* md, const double* mb_, u
 constexpr int kSmTraceSlots = 8;
 constexpr unsigned kTrailSmidOff = 64;  // words behind the ready word: %smid of every CTA of the last trailing launch
 
-// NT = threads per CTA: 512 for the stand-alone selection (one CTA owns its SM); 128 for the TRAILING form that runs
-// beside the counting kernel in the registers and shared memory it leaves free (dvs_count_select): it examines a
-// position only once the record's row has been published (`ready_pos`), so the rounds trail the counting.
+// One CTA of NT = 512 threads owns its SM.  In the TRAILING form (dvs_count_select) the kernel examines a position
+// only once the record's row has been published (`ready_pos`), so the rounds trail the counting.
 template <int NT, int MINB, unsigned MAXN, unsigned CHUNK>
 __global__ void __launch_bounds__(NT, MINB)
 k_sel_persist_sm_t(const double* __restrict__ F, const double* __restrict__ H, unsigned dim, double* S_glob,

@@ -60,7 +60,7 @@ def test_fullsize_counts_and_entropies_equal_the_oracle(full):
 def test_fullsize_nmost_equals_the_oracle_in_every_round_form(full, monkeypatch):
     lib, ctx, ss, kf, g = full
     order = np.random.default_rng(SEED).permutation(NREC).astype(np.uint32)
-    for persist in ("2", "1", "0"):  # SM-replicated rounds, cooperative grid.sync rounds, two launches per round
+    for persist in ("2", "1", "0"):  # SM-replicated rounds, cooperative grid.sync rounds, host-driven rounds
         monkeypatch.setenv("DVS_SELECT_PERSIST", persist)
         idx, delta, stats = kf.select(order, lib.MODE_NMOST, N)
         assert idx.tolist() == g["ids"].tolist()                                  # same set, same Vec order

@@ -298,10 +298,9 @@ def test_select_fast_path_equals_exact_only(lib, ctx, orc, monkeypatch):
         i0, d0, s0 = kf.select(order, mode, lo, hi)
         assert ctx._lib.dvs_select_last_exact_evals(ctx.handle) == 0
         monkeypatch.setenv("DVS_SELECT_EXACT_ONLY", "0")
-        # host-driven fast rounds, two launches per device-driven round, the global-state persistent
-        # kernel, the SM-replicated persistent kernel (default)
-        for host_loop, persist in (("1", "0"), ("0", "0"), ("0", "1"), ("0", "2")):
-            monkeypatch.setenv("DVS_SELECT_HOST_LOOP", host_loop)
+        # host-driven fast rounds, the global-state persistent kernel, the SM-replicated persistent
+        # kernel (default)
+        for persist in ("0", "1", "2"):
             monkeypatch.setenv("DVS_SELECT_PERSIST", persist)
             i1, d1, s1 = kf.select(order, mode, lo, hi)
             assert i0.tolist() == i1.tolist() and np.array_equal(d0, d1) and np.array_equal(s0, s1)

@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Counting-kernel A/B timings on the bench workload (10,500 synthetic genomes, k=6 by default):
 
-    python tools/bench_count.py [--k 6] [--nrec 10500] [--variants default,s3,...]
+    python tools/bench_count.py [--k 6] [--nrec 10500] [--variants default,super]
 
 A variant is a comma-free name from VARIANTS below (a set of environment switches read by dvs_count_kmers on every
 call).  Every variant's count rows are compared with the default kernel's on a sample of records."""
@@ -18,18 +18,7 @@ from diverseseq_b200 import _lib  # noqa: E402
 
 VARIANTS = {
     "default": {},                                   # (k+2)-mers / 16-bit halves, 1024 threads x 3 KB-steps in flight
-    "s3_1024x2": {"DVS_COUNT_S3_SHAPE": "1"},
-    "s3_512x4": {"DVS_COUNT_S3_SHAPE": "2"},
-    "s3scr": {"DVS_COUNT_SCRAMBLE": "1"},
-    # a smaller L1 (what a co-resident kernel's shared memory costs): 144 KB table + pad -> carve-out 196 / 228 KB
-    "x2_pad18": {"DVS_COUNT_S3_SHAPE": "1", "DVS_COUNT_SMEM_PAD": "18000"},
-    "x2_pad48": {"DVS_COUNT_S3_SHAPE": "1", "DVS_COUNT_SMEM_PAD": "48000"},
-    "x2_pad66": {"DVS_COUNT_S3_SHAPE": "1", "DVS_COUNT_SMEM_PAD": "66000"},
-    "x2_pad80": {"DVS_COUNT_S3_SHAPE": "1", "DVS_COUNT_SMEM_PAD": "80000"},
-    "x3_pad48": {"DVS_COUNT_SMEM_PAD": "48000"},
-    "x3_pad80": {"DVS_COUNT_SMEM_PAD": "80000"},
     "super": {"DVS_COUNT_S3": "0"},                   # (k+1)-mer kernel of round 1
-    "super_noscr": {"DVS_COUNT_S3": "0", "DVS_COUNT_SCRAMBLE": "0"},
 }
 KEYS = sorted({k for v in VARIANTS.values() for k in v})
 
@@ -39,7 +28,7 @@ def main():
     ap.add_argument("--k", type=int, default=6)
     ap.add_argument("--nrec", type=int, default=10500)
     ap.add_argument("--mean-len", type=int, default=4_000_000)
-    ap.add_argument("--variants", default="default,s3_1024x2,s3_512x4,super")
+    ap.add_argument("--variants", default="default,super")
     ap.add_argument("--reps", type=int, default=5)
     a = ap.parse_args()
     ctx = _lib.Context(0)

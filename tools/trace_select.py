@@ -4,7 +4,7 @@ wall time of each form on the benchmark set (nmost n=100, k=6, 10.5k genomes):
 
     python tools/trace_select.py [--mean-len 4000000] [--out gpurun_out/sel_trace.txt]
 
-DVS_SELECT_PERSIST: 0 = two launches per round, 1 = global-state persistent kernel, 2 = SM-replicated."""
+DVS_SELECT_PERSIST: 0 = host-driven rounds, 1 = global-state persistent kernel, 2 = SM-replicated."""
 from __future__ import annotations
 
 import argparse
