@@ -21,6 +21,7 @@ import hashlib
 import numpy as np
 
 from . import _lib
+from .distance import counts_sparse_for_selection
 
 __all__ = [
     "ZarrStoreWrapper", "SummedRecordsResult", "LazySeq", "make_zarr_store", "get_seqids_from_store",
@@ -169,9 +170,12 @@ class SummedRecordsResult:
         return f"SummedRecordsResult(size={self.size}, total_jsd={self.total_jsd!r}, k={self.k})"
 
 
-def _make_result(names, kfreq_rows, deltas, stats, k, num_states) -> SummedRecordsResult:
+def _make_result(names, kfreq_rows, deltas, stats, k, num_states, as_lists: bool = True) -> SummedRecordsResult:
+    """as_lists=False keeps each record's frequency row a float64 ndarray (the sparse route at k >= 10, where a
+    Python list of 4^k floats would take ~0.4 GB per record)"""
     r = SummedRecordsResult()
-    r.records = [(names[i], kfreq_rows[i].tolist(), float(deltas[i])) for i in range(len(names))]
+    r.records = [(names[i], kfreq_rows[i].tolist() if as_lists else kfreq_rows[i], float(deltas[i]))
+                 for i in range(len(names))]
     r.total_jsd = float(stats[0])
     r.mean_delta_jsd = float(stats[1])
     r.std_delta_jsd = float(stats[2])
@@ -215,6 +219,10 @@ def _select_from_store(store, seqids, k, num_states, mode, min_size, max_size) -
         raise ValueError("k cannot be 0")
     if len(seqids) < min_size:  # before any counting, like records.rs:323-325
         raise ValueError(f"The number of sequences {len(seqids)} is < n {min_size}")
+    if counts_sparse_for_selection(k, num_states):  # no dense row in memory; the same selection bit for bit
+        sp = _lib.KSparse.count(ctx, seqset, k, num_states, want_entropy=True)
+        idx, delta, stats = sp.select(order, mode, min_size, max_size)
+        return _make_result([names[r] for r in idx], sp.dense_rows(idx), delta, stats, k, num_states, as_lists=False)
     # one call: for nmost at k = 4..6 the selection rounds trail the counting (dvs_count_select); every other case runs
     # the two steps back to back inside it, with the same results and errors
     kf, idx, delta, stats = _lib.KFreqs.count_select(ctx, seqset, k, order, mode, min_size, max_size, num_states)

@@ -73,6 +73,7 @@ SIGNATURES = {
     "dvs_ksparse_free": (None, [_vp]),
     "dvs_euclid_distances_sparse": (_i32, [_vp, _vp, _u32, _u32, _vp]),
     "dvs_select": (_i32, [_vp, _vp, _vp, _u32, _i32, _u32, _u32, _vp, _vp, _vp, C.POINTER(_u32)]),
+    "dvs_select_sparse": (_i32, [_vp, _vp, _vp, _u32, _i32, _u32, _u32, _vp, _vp, _vp, C.POINTER(_u32)]),
     "dvs_count_select": (_i32, [_vp, _vp, _i32, _i32, _vp, _u32, _i32, _u32, _u32, _u32, C.POINTER(_vp), _vp, _vp, _vp,
                                 C.POINTER(_u32)]),
     "dvs_select_last_accepts": (_u32, [_vp]),
@@ -586,6 +587,7 @@ class KSparse(_Handle):
                                               C.byref(h)))
         out = cls(ctx, h)
         out.has_entropy = bool(want_entropy)
+        out.k, out.num_states = int(k), int(num_states)
         return out
 
     @property
@@ -610,6 +612,38 @@ class KSparse(_Handle):
             check(self.ctx._lib.dvs_ksparse_download(self.ctx.handle, self.handle, int(rec), ptr(idx), ptr(cnt), n.value,
                                                      C.byref(n)))
         return idx, cnt
+
+    def select(self, order, mode: int, min_size: int, max_size: int = 0):
+        """nmost / max selection over the sparse rows (dvs_select_sparse; needs want_entropy=True at count time);
+        the same (row indices, delta_jsd, stats5) as KFreqs.select over the dense rows of the same records"""
+        order = np.ascontiguousarray(order, dtype=np.uint32)
+        cap = max(int(min_size), int(max_size), 1) + 1
+        if int(mode) != MODE_NMOST and int(max_size) < int(min_size):
+            cap = order.size + 1  # the set can grow without bound (dvs_b200.h, dvs_select)
+        idx = np.zeros(cap, dtype=np.uint32)
+        delta = np.zeros(cap, dtype=np.float64)
+        stats = np.zeros(5, dtype=np.float64)
+        size = _u32(0)
+        check(self.ctx._lib.dvs_select_sparse(self.ctx.handle, self.handle, ptr(order) if order.size else None,
+                                              order.size, int(mode), int(min_size), int(max_size), ptr(idx), ptr(delta),
+                                              ptr(stats), C.byref(size)))
+        n = size.value
+        return idx[:n].copy(), delta[:n].copy(), stats
+
+    def dense_rows(self, rows) -> np.ndarray:
+        """frequency rows `rows` as one [len(rows), num_states^k] f64 array, formed on the host from the downloaded
+        (index, count) lists with the same IEEE division as the dense rows (count / total; a record without valid
+        k-mers gives 0 / 0 = NaN everywhere, as its dense row does)"""
+        rows = np.ascontiguousarray(rows, dtype=np.uint32)
+        out = np.zeros((rows.size, self.num_states ** self.k), dtype=np.float64)
+        for i, r in enumerate(rows):
+            idx, cnt = self.record(int(r))
+            total = float(cnt.sum(dtype=np.uint64))
+            if total == 0.0:
+                out[i] = np.nan
+            else:
+                out[i, idx] = cnt.astype(np.float64) / total
+        return out
 
     def euclidean(self, row_begin: int = 0, row_end: int | None = None) -> np.ndarray:
         """rows [row_begin, row_end) of the Euclidean distance matrix of the frequency rows (dvs_euclid_distances_sparse)"""

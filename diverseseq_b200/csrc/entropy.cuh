@@ -58,8 +58,15 @@ __device__ __forceinline__ double div_exact(double a, const FastDiv& d) {
     return __fma_rn(r, d.y, q);
 }
 
-template <class Elem>
-__device__ EntropyResult block_entropy_exact(uint64_t dim, Elem elem, double* smem) {
+// Staging hook of a row source (select.cu): called by every thread of the block with the first element of each
+// group of kEntStageTiles tiles before the producers read it.  Rows held in memory need none.
+constexpr int kEntStageTiles = 8;
+struct NoStage {
+    __device__ __forceinline__ void operator()(uint64_t) const {}
+};
+
+template <class Elem, class Stage = NoStage>
+__device__ EntropyResult block_entropy_exact(uint64_t dim, Elem elem, double* smem, Stage stage = Stage()) {
     double* term[2] = {smem, smem + 2 * kEntTile};
     double* val[2] = {smem + kEntTile, smem + 3 * kEntTile};
     __shared__ double s_res[2];
@@ -94,9 +101,13 @@ __device__ EntropyResult block_entropy_exact(uint64_t dim, Elem elem, double* sm
     };
 
     double acc = 0.0;  // lane 0: e-chain, lane 1: t-chain
-    if (ntiles > 0) produce(0, tid, kEntThreads);  // everybody helps with the first tile
+    if (ntiles > 0) {
+        stage(0);
+        produce(0, tid, kEntThreads);  // everybody helps with the first tile
+    }
     __syncthreads();
     for (uint64_t tile = 0; tile < ntiles; ++tile) {
+        if ((tile + 1) % kEntStageTiles == 0 && tile + 1 < ntiles) stage((tile + 1) * kEntTile);
         if (warp == 0) {
             if (lane < 2) {
                 const uint64_t base = tile * kEntTile;

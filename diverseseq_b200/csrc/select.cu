@@ -27,6 +27,7 @@
 #include "common.cuh"
 #include "entropy.cuh"
 #include "fused.cuh"
+#include "sparse.cuh"
 
 namespace cg = cooperative_groups;
 
@@ -92,53 +93,198 @@ struct SelState {
     }
 };
 
+// ------------------------------------------------------------------------------ row sources ----
+// Where a kernel gets element i of a record's frequency row.  A kernel binds the rows it reads to the slots of a
+// view (v.row(slot, record, dim)) and hands the view to the entropy helper as its staging hook.
+//   DenseRows   the [nrec][dim] rows of a dvs_kfreqs: a bound row is F + record * dim; nothing is staged.
+//   SparseRows  the bucket-major (index, count) rows of a dvs_ksparse (sparse.cuh).  A bucket holds the entries of
+//               4,096 consecutive bins: one pass of the bounded-error kernels (8 x kFastThreads elements) and
+//               kEntStageTiles tiles of the exact ones.  Before a pass, the CTA stages the bucket's counts of every
+//               bound row in shared memory (16 KB per row, 0 where the row has no entry), and element i is then
+//               div_exact(count, total): the division k_freq_entropy forms the dense row with.  Every element, and
+//               with it every sum, error bound and decision, is therefore the dense path's bit for bit.
+// The selection state S stays dense either way (4^k f64): the clamps and the reference's sums run over all elements.
+struct DenseRows {
+    static constexpr bool kSparse = false;
+    const double* __restrict__ F;
+    struct View {
+        const double* __restrict__ F;
+        __device__ __forceinline__ const double* row(int, unsigned r, uint64_t dim) const { return F + (size_t)r * dim; }
+        // a candidate row of another dvs_kfreqs (dvs_summed_delta_jsd)
+        __device__ __forceinline__ const double* cand_row(const double* C, int, unsigned r, uint64_t dim) const {
+            return C + (size_t)r * dim;
+        }
+        __device__ __forceinline__ void operator()(uint64_t) const {}
+    };
+    __device__ __forceinline__ View view(uint32_t*) const { return View{F}; }
+};
+
+static_assert(kEntTile * kEntStageTiles == (int)kSpLowBins, "a tile group of the exact kernels must be one bucket");
+constexpr int kStageSlots = 3;  // rows one kernel reads at most (the fused replace + update: lowest, candidate, member)
+constexpr size_t kStageBytes = (size_t)kSpLowBins * sizeof(uint32_t);
+
+struct SpRow {
+    const uint32_t* s;  // staged counts of the current bucket
+    FastDiv dv;         // the record's number of valid k-mers
+    __device__ __forceinline__ double operator[](uint64_t i) const {
+        return div_exact((double)s[i & (kSpLowBins - 1u)], dv);
+    }
+};
+
+struct SparseRowsData {
+    const uint32_t *idx, *cnt, *bucket_ptr, *bucket_nnz;
+    const uint64_t *offsets, *totals;
+    uint32_t nb;
+    // first slot and entries of bucket b of record r
+    __device__ __forceinline__ uint64_t bucket_at(unsigned r, uint32_t b) const {
+        return offsets[r] + bucket_ptr[(size_t)r * (nb + 1) + b];
+    }
+    __device__ __forceinline__ uint32_t bucket_len(unsigned r, uint32_t b) const { return bucket_nnz[(size_t)r * nb + b]; }
+};
+struct SparseRows : SparseRowsData {
+    static constexpr bool kSparse = true;
+    struct View {
+        SparseRowsData src;
+        uint32_t* smem;  // kStageSlots x 4,096 counts
+        unsigned rows[kStageSlots];
+        int nbound;
+        __device__ __forceinline__ SpRow row(int slot, unsigned r, uint64_t) {
+            rows[slot] = r;
+            nbound = max(nbound, slot + 1);
+            return SpRow{smem + (size_t)slot * kSpLowBins, make_fast_div((double)src.totals[r])};
+        }
+        __device__ __forceinline__ SpRow cand_row(const double*, int slot, unsigned r, uint64_t dim) { return row(slot, r, dim); }
+        // every thread of the CTA: stage the bucket that starts at element `base` of every bound row
+        __device__ void operator()(uint64_t base) const {
+            const uint32_t b = (uint32_t)(base >> kSpLowBits);
+            __syncthreads();  // the previous bucket has been read
+            uint4* z = reinterpret_cast<uint4*>(smem);
+            for (unsigned i = threadIdx.x; i < (unsigned)nbound * (kSpLowBins / 4); i += blockDim.x) z[i] = make_uint4(0, 0, 0, 0);
+            __syncthreads();
+#pragma unroll
+            for (int q = 0; q < kStageSlots; ++q) {
+                if (q < nbound) {
+                    const uint64_t at = src.bucket_at(rows[q], b);
+                    const uint32_t n = src.bucket_len(rows[q], b);
+                    uint32_t* d = smem + (size_t)q * kSpLowBins;
+                    for (uint32_t e = threadIdx.x; e < n; e += blockDim.x) d[src.idx[at + e] & (kSpLowBins - 1u)] = src.cnt[at + e];
+                }
+            }
+            __syncthreads();
+        }
+    };
+    __device__ __forceinline__ View view(uint32_t* smem) const { return View{*this, smem, {0u, 0u, 0u}, 0}; }
+};
+
+// the staging hook a kernel hands to the entropy helpers: the view itself, or nothing for dense rows
+__device__ __forceinline__ NoStage stager(const DenseRows::View&) { return NoStage{}; }
+__device__ __forceinline__ const SparseRows::View& stager(const SparseRows::View& v) { return v; }
+
+// the staging area of the bounded-error kernels: their dynamic shared memory (the exact kernels place it after
+// their tiles); dense rows have none
+template <class Src>
+__device__ __forceinline__ uint32_t* stage_smem() { return nullptr; }
+template <>
+__device__ __forceinline__ uint32_t* stage_smem<SparseRows>() {
+    extern __shared__ __align__(16) uint32_t sel_stage_smem[];
+    return sel_stage_smem;
+}
+template <class Src>
+__device__ __forceinline__ uint32_t* exact_stage_smem(double* ent_smem) {
+    return Src::kSparse ? reinterpret_cast<uint32_t*>(ent_smem + kEntSmemBytes / sizeof(double)) : nullptr;
+}
+// dynamic shared memory of a kernel that binds `slots` rows (on top of what the dense form uses)
+template <class Src>
+constexpr size_t stage_bytes(int slots) { return Src::kSparse ? (size_t)slots * kStageBytes : 0; }
+
+__device__ __forceinline__ void sum_scalars(const double* __restrict__ H, const unsigned* __restrict__ members, unsigned n,
+                                            int extra_row, unsigned* __restrict__ members_out, SelScal* sc) {
+    double e = 0.0;
+    for (unsigned j = 0; j < n; ++j) e = __dadd_rn(e, H[members[j]]);
+    if (extra_row >= 0) e = __dadd_rn(e, H[extra_row]);
+    unsigned nn = n;
+    if (members_out != members)
+        for (unsigned j = 0; j < n; ++j) members_out[j] = members[j];
+    if (extra_row >= 0) members_out[nn++] = (unsigned)extra_row;
+    sc->E = e;
+    sc->n = nn;
+    sc->panic = 0;
+    sc->panic_total = 0.0;
+    sc->ticket = 0;
+    sc->first_true = kNone;
+    sc->first_panic = kNone;
+    sc->first_unsure = kNone;
+    sc->state_unsure = 0;
+    sc->total_bound = 0.0;
+    sc->exact = 0;
+}
+
 // S[i] = ((0 + f_m0[i]) + f_m1[i]) + ... (+ f_extra[i]);  E likewise  (records.rs:36-42, :129-133)
-__global__ void k_sel_sum(const double* __restrict__ F, const double* __restrict__ H, uint64_t dim,
+// Sparse rows: one CTA per bucket zeroes its 4,096 elements of S and adds the members' entries one member after
+// another, in member order.  An absent entry would add +0.0, which leaves every sum (all >= +0) as it is, so per
+// element these are the same additions in the same order.
+template <class Src>
+__global__ void k_sel_sum(const Src src, const double* __restrict__ H, uint64_t dim,
                           const unsigned* __restrict__ members, unsigned n, int extra_row, double* __restrict__ S,
                           unsigned* __restrict__ members_out, SelScal* sc) {
-    uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < dim) {
-        double s = 0.0;
-        for (unsigned j = 0; j < n; ++j) s = __dadd_rn(s, F[(size_t)members[j] * dim + i]);
-        if (extra_row >= 0) s = __dadd_rn(s, F[(size_t)extra_row * dim + i]);
-        S[i] = s;
-    }
-    if (i == 0) {
-        double e = 0.0;
-        for (unsigned j = 0; j < n; ++j) e = __dadd_rn(e, H[members[j]]);
-        if (extra_row >= 0) e = __dadd_rn(e, H[extra_row]);
-        unsigned nn = n;
-        if (members_out != members)
-            for (unsigned j = 0; j < n; ++j) members_out[j] = members[j];
-        if (extra_row >= 0) members_out[nn++] = (unsigned)extra_row;
-        sc->E = e;
-        sc->n = nn;
-        sc->panic = 0;
-        sc->panic_total = 0.0;
-        sc->ticket = 0;
-        sc->first_true = kNone;
-        sc->first_panic = kNone;
-        sc->first_unsure = kNone;
-        sc->state_unsure = 0;
-        sc->total_bound = 0.0;
-        sc->exact = 0;
+    if constexpr (Src::kSparse) {
+        const uint32_t b = blockIdx.x;
+        double* Sb = S + ((uint64_t)b << kSpLowBits);
+        for (unsigned i = threadIdx.x; i < kSpLowBins; i += blockDim.x) Sb[i] = 0.0;
+        const unsigned nn = n + (extra_row >= 0 ? 1u : 0u);
+        for (unsigned j = 0; j < nn; ++j) {
+            __syncthreads();  // member j - 1 is in
+            const unsigned r = j < n ? members[j] : (unsigned)extra_row;
+            const uint64_t at = src.bucket_at(r, b);
+            const uint32_t m = src.bucket_len(r, b);
+            const FastDiv dv = make_fast_div((double)src.totals[r]);
+            for (uint32_t e = threadIdx.x; e < m; e += blockDim.x) {
+                double* p = Sb + (src.idx[at + e] & (kSpLowBins - 1u));
+                *p = __dadd_rn(*p, div_exact((double)src.cnt[at + e], dv));
+            }
+        }
+        if (b == 0 && threadIdx.x == 0) sum_scalars(H, members, n, extra_row, members_out, sc);
+    } else {
+        const double* F = src.F;
+        uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+        if (i < dim) {
+            double s = 0.0;
+            for (unsigned j = 0; j < n; ++j) s = __dadd_rn(s, F[(size_t)members[j] * dim + i]);
+            if (extra_row >= 0) s = __dadd_rn(s, F[(size_t)extra_row * dim + i]);
+            S[i] = s;
+        }
+        if (i == 0) sum_scalars(H, members, n, extra_row, members_out, sc);
     }
 }
 
 // replace_lowest (records.rs:94-135): drop_lowest + push on summed_kfreqs, elementwise; the LAST
 // CTA to finish then updates the scalars and the member Vec: E -= H_low; E += H_c;
-// Vec::remove(lowest); push(c).
-__global__ void k_sel_replace_vec(const double* __restrict__ F, const double* __restrict__ H, uint64_t dim,
+// Vec::remove(lowest); push(c).  Sparse rows: one CTA per bucket, over every element of S (the clamp too).
+template <class Src>
+__global__ void k_sel_replace_vec(const Src src, const double* __restrict__ H, uint64_t dim,
                                   unsigned* __restrict__ members, uint8_t* __restrict__ is_member, SelScal* sc,
                                   unsigned cand_row, double* __restrict__ S) {
     __shared__ unsigned s_last;
-    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     const unsigned low = sc->lowest;
     const unsigned low_row = members[low];
-    if (i < dim) {
-        double s = __dsub_rn(S[i], F[(size_t)low_row * dim + i]);
-        if (s <= kEps) s = 0.0;
-        S[i] = __dadd_rn(s, F[(size_t)cand_row * dim + i]);
+    if constexpr (Src::kSparse) {
+        auto v = src.view(stage_smem<Src>());
+        const SpRow fl = v.row(0, low_row, dim), fc = v.row(1, cand_row, dim);
+        const uint64_t base = (uint64_t)blockIdx.x << kSpLowBits;
+        v(base);
+        for (unsigned q = threadIdx.x; q < kSpLowBins; q += blockDim.x) {
+            double s = __dsub_rn(S[base + q], fl[q]);
+            if (s <= kEps) s = 0.0;
+            S[base + q] = __dadd_rn(s, fc[q]);
+        }
+    } else {
+        const double* F = src.F;
+        const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+        if (i < dim) {
+            double s = __dsub_rn(S[i], F[(size_t)low_row * dim + i]);
+            if (s <= kEps) s = 0.0;
+            S[i] = __dadd_rn(s, F[(size_t)cand_row * dim + i]);
+        }
     }
     __syncthreads();  // every read of members[]/lowest by this CTA is done
     if (threadIdx.x == 0) {
@@ -182,8 +328,9 @@ __global__ void k_sel_replace_vec(const double* __restrict__ F, const double* __
 // depends on another, only the final scalar arithmetic does, so the last CTA to finish forms
 // total_jsd = H(S/n) - E/n, delta_j = total_jsd - (H(m_j) - (E - H_j)/(n-1)), the strict-<
 // argmin and the mean/std/cov statistics (:153-172) in the reference's order.
+template <class Src>
 __global__ void __launch_bounds__(kEntThreads)
-k_sel_update(const double* __restrict__ F, const double* __restrict__ H, uint64_t dim, const double* __restrict__ S,
+k_sel_update(const Src src, const double* __restrict__ H, uint64_t dim, const double* __restrict__ S,
              const unsigned* __restrict__ members, double* __restrict__ mdelta, SelScal* sc) {
     extern __shared__ __align__(16) double ent_smem[];
     __shared__ unsigned s_last;
@@ -198,14 +345,15 @@ k_sel_update(const double* __restrict__ F, const double* __restrict__ H, uint64_
     } else {
         const unsigned row = members[j];
         const double div = __dsub_rn(nd, 1.0);
-        const double* f = F + (size_t)row * dim;
+        auto v = src.view(exact_stage_smem<Src>(ent_smem));
+        const auto f = v.row(0, row, dim);
         EntropyResult h = block_entropy_exact(
             dim,
             [&](uint64_t i) {
                 double m = __ddiv_rn(__dsub_rn(S[i], f[i]), div);
                 return (m <= kEps) ? 0.0 : m;  // updated_mean_freqs clamp, records.rs:281-284
             },
-            ent_smem);
+            ent_smem, stager(v));
         if (threadIdx.x == 0) {
             const double mean_entropy = __ddiv_rn(__dsub_rn(sc->E, H[row]), div);
             mdelta[j] = __dsub_rn(h.e, mean_entropy);  // jsd without record j; delta formed below
@@ -271,9 +419,11 @@ k_sel_update(const double* __restrict__ F, const double* __restrict__ H, uint64_
     }
 }
 
-// increases_jsd for a window of candidates (records.rs:70-92); one CTA per position
+// increases_jsd for a window of candidates (records.rs:70-92); one CTA per position.  Sparse rows: the candidates
+// are rows of the same source (candF unused).
+template <class Src>
 __global__ void __launch_bounds__(kEntThreads)
-k_sel_scan(const double* __restrict__ F, const double* __restrict__ H, uint64_t dim, const double* __restrict__ S,
+k_sel_scan(const Src src, const double* __restrict__ H, uint64_t dim, const double* __restrict__ S,
            const unsigned* __restrict__ members, SelScal* sc, const double* __restrict__ candF,
            const double* __restrict__ candH, const uint8_t* __restrict__ cand_valid,
            const uint8_t* __restrict__ is_member, const unsigned* __restrict__ order, unsigned pos0,
@@ -286,10 +436,11 @@ k_sel_scan(const double* __restrict__ F, const double* __restrict__ H, uint64_t 
     const unsigned n = sc->n;
     const double nd = (double)n;
     const unsigned low_row = members[sc->lowest];
-    const double* fl = F + (size_t)low_row * dim;
-    const double* fc = candF + (size_t)row * dim;
+    auto v = src.view(exact_stage_smem<Src>(ent_smem));
+    const auto fl = v.row(0, low_row, dim);
+    const auto fc = v.cand_row(candF, 1, row, dim);
     EntropyResult h = block_entropy_exact(
-        dim, [&](uint64_t i) { return __ddiv_rn(__dadd_rn(__dsub_rn(S[i], fl[i]), fc[i]), nd); }, ent_smem);
+        dim, [&](uint64_t i) { return __ddiv_rn(__dadd_rn(__dsub_rn(S[i], fl[i]), fc[i]), nd); }, ent_smem, stager(v));
     if (threadIdx.x == 0) {
         const double mean_entropy = __ddiv_rn(__dadd_rn(__dsub_rn(sc->E, H[low_row]), candH[row]), nd);
         const double d = __dsub_rn(h.e, mean_entropy);
@@ -303,6 +454,8 @@ k_sel_scan(const double* __restrict__ F, const double* __restrict__ H, uint64_t 
 #include "select_fast.cuh"
 #include "select_grow.cuh"
 #include "select_sm.cuh"
+
+static_assert(8 * kFastThreads == (int)kSpLowBins, "a pass of the bounded-error kernels must be one bucket");
 
 constexpr auto k_sel_persist_sm_full = k_sel_persist_sm_t<kFastThreads, 1, kSmMaxN, kSmChunk>;
 
@@ -346,19 +499,35 @@ static int panic_error(const SelScal& h) {
     return DVS_ERR_VALUE;
 }
 
+// the device row source of a record set, and the candidate rows k_sel_scan reads besides it
+inline DenseRows row_source(const dvs_kfreqs* f) { return DenseRows{f->freqs.p}; }
+inline SparseRows row_source(const dvs_ksparse* sp) {
+    return SparseRows{{sp->idx.p, sp->cnt.p, sp->bucket_ptr.p, sp->bucket_nnz.p, sp->offsets.p, sp->totals.p, sp->nb}};
+}
+inline const double* cand_rows(const dvs_kfreqs* q) { return q->freqs.p; }
+inline const double* cand_rows(const dvs_ksparse*) { return nullptr; }
+
+// The launches of the host-driven rounds over one record set: RS is dvs_kfreqs (dense rows) or dvs_ksparse.
+template <class RS>
 struct Selector {
+    using Src = decltype(row_source((const RS*)nullptr));
     dvs_ctx* ctx;
-    const dvs_kfreqs* f;
+    const RS* f;
     uint64_t dim;
     cudaStream_t st;
     SelScal* h_sc;  // pinned
 
+    Src rows() const { return row_source(f); }
     int read(SelState& s) {
         DVS_CUDA_TRY(cudaMemcpyAsync(h_sc, s.sc.p, sizeof(SelScal), cudaMemcpyDeviceToHost, st));
         DVS_CUDA_TRY(cudaStreamSynchronize(st));
         return DVS_OK;
     }
-    unsigned vec_grid() const { return (unsigned)((dim + 255) / 256); }
+    // elementwise kernels (k_sel_sum, k_sel_replace_vec): 256 threads per 256 elements, or per bucket of a sparse row
+    unsigned vec_grid() const {
+        if constexpr (Src::kSparse) return f->nb;
+        else return (unsigned)((dim + 255) / 256);
+    }
     int reset_scan(SelState& s) {
         static_assert(offsetof(SelScal, first_panic) == offsetof(SelScal, first_true) + sizeof(unsigned), "layout");
         DVS_CUDA_TRY(cudaMemsetAsync((char*)s.sc.p + offsetof(SelScal, first_true), 0xFF, 2 * sizeof(unsigned), st));
@@ -366,15 +535,15 @@ struct Selector {
         return DVS_OK;
     }
     int update_fast(SelState& s, unsigned n) {
-        k_sel_update_fast<<<n + 1, kFastThreads, 0, st>>>(f->freqs.p, f->entropy.p, dim, s.S(), s.members(),
-                                                          s.mdelta.p, s.mbound.p, s.sc.p);
+        k_sel_update_fast<<<n + 1, kFastThreads, stage_bytes<Src>(1), st>>>(rows(), f->entropy.p, dim, s.S(), s.members(),
+                                                                          s.mdelta.p, s.mbound.p, s.sc.p);
         DVS_LAUNCHED(ctx);
         return DVS_OK;
     }
     int replace_fast(SelState& s, unsigned n, unsigned cand_row, uint8_t* is_member) {
-        k_sel_replace_update_fast<<<n + 1, kFastThreads, 0, st>>>(f->freqs.p, f->entropy.p, dim, s.S(), s.S_other(),
-                                                                  s.members(), s.members_other(), is_member,
-                                                                  s.mdelta.p, s.mbound.p, s.sc.p, cand_row);
+        k_sel_replace_update_fast<<<n + 1, kFastThreads, stage_bytes<Src>(3), st>>>(
+            rows(), f->entropy.p, dim, s.S(), s.S_other(), s.members(), s.members_other(), is_member, s.mdelta.p,
+            s.mbound.p, s.sc.p, cand_row);
         DVS_LAUNCHED(ctx);
         s.flip();
         return DVS_OK;
@@ -382,63 +551,86 @@ struct Selector {
     // (first_true / first_unsure are re-armed by every update kernel and stay armed after an empty
     // window; the caller resets them explicitly after an exact single-candidate scan)
     int scan_fast(SelState& s, const uint8_t* is_member, const unsigned* d_order, unsigned pos0, unsigned count) {
-        k_sel_scan_fast<<<count, kFastThreads, 0, st>>>(f->freqs.p, f->entropy.p, dim, s.S(), s.members(), s.sc.p,
-                                                         f->valid.p, is_member, d_order, pos0);
+        k_sel_scan_fast<<<count, kFastThreads, stage_bytes<Src>(2), st>>>(rows(), f->entropy.p, dim, s.S(), s.members(),
+                                                                        s.sc.p, f->valid.p, is_member, d_order, pos0);
         DVS_LAUNCHED(ctx);
         return DVS_OK;
     }
     // one candidate row of another kfreqs object, no order / validity / membership filters
     int scan_raw(SelState& s, const double* candF, const double* candH, unsigned row, double* delta_out) {
         DVS_TRY(reset_scan(s));
-        k_sel_scan<<<1, kEntThreads, kEntSmemBytes, st>>>(f->freqs.p, f->entropy.p, dim, s.S(), s.members(), s.sc.p,
-                                                           candF, candH, nullptr, nullptr, nullptr, row, delta_out);
+        k_sel_scan<<<1, kEntThreads, kEntSmemBytes, st>>>(rows(), f->entropy.p, dim, s.S(), s.members(), s.sc.p, candF,
+                                                           candH, nullptr, nullptr, nullptr, row, delta_out);
         DVS_LAUNCHED(ctx);
         return DVS_OK;
     }
 
     // SummedRecords::new over `members` (+ optional pushed row): sums, then total_jsd + member deltas
-    int build(SelState& s, const unsigned* d_members, unsigned n, int extra_row) {
-        k_sel_sum<<<vec_grid(), 256, 0, st>>>(f->freqs.p, f->entropy.p, dim, d_members, n, extra_row, s.S(),
-                                              s.members(), s.sc.p);
+    int sum(SelState& s, const unsigned* d_members, unsigned n, int extra_row) {
+        k_sel_sum<<<vec_grid(), 256, 0, st>>>(rows(), f->entropy.p, dim, d_members, n, extra_row, s.S(), s.members(),
+                                              s.sc.p);
         DVS_LAUNCHED(ctx);
+        return DVS_OK;
+    }
+    int build(SelState& s, const unsigned* d_members, unsigned n, int extra_row) {
+        DVS_TRY(sum(s, d_members, n, extra_row));
         return update(s, n + (extra_row >= 0 ? 1u : 0u));
     }
     // fast SummedRecords::new (+ optional pushed row): exact sums, bounded-error total / deltas / stats
     int build_fast(SelState& s, const unsigned* d_members, unsigned n, int extra_row) {
-        k_sel_sum<<<vec_grid(), 256, 0, st>>>(f->freqs.p, f->entropy.p, dim, d_members, n, extra_row, s.S(),
-                                              s.members(), s.sc.p);
-        DVS_LAUNCHED(ctx);
+        DVS_TRY(sum(s, d_members, n, extra_row));
         return update_fast(s, n + (extra_row >= 0 ? 1u : 0u));
     }
     int update(SelState& s, unsigned n) {
-        k_sel_update<<<n + 1, kEntThreads, kEntSmemBytes, st>>>(f->freqs.p, f->entropy.p, dim, s.S(), s.members(),
-                                                                 s.mdelta.p, s.sc.p);
+        k_sel_update<<<n + 1, kEntThreads, kEntSmemBytes + stage_bytes<Src>(1), st>>>(rows(), f->entropy.p, dim, s.S(),
+                                                                                     s.members(), s.mdelta.p, s.sc.p);
         DVS_LAUNCHED(ctx);
         return DVS_OK;
     }
     int replace(SelState& s, unsigned n, unsigned cand_row, uint8_t* is_member) {
-        k_sel_replace_vec<<<vec_grid(), 256, 0, st>>>(f->freqs.p, f->entropy.p, dim, s.members(), is_member,
-                                                      s.sc.p, cand_row, s.S());
+        k_sel_replace_vec<<<vec_grid(), 256, stage_bytes<Src>(2), st>>>(rows(), f->entropy.p, dim, s.members(), is_member,
+                                                                        s.sc.p, cand_row, s.S());
         DVS_LAUNCHED(ctx);
         return update(s, n);
     }
-    int scan(SelState& s, const dvs_kfreqs* q, const uint8_t* is_member, const unsigned* d_order, unsigned pos0,
+    int scan(SelState& s, const RS* q, const uint8_t* is_member, const unsigned* d_order, unsigned pos0,
              unsigned count, double* delta_out) {
         DVS_TRY(reset_scan(s));  // re-arm the min-index reduction
-        k_sel_scan<<<count, kEntThreads, kEntSmemBytes, st>>>(f->freqs.p, f->entropy.p, dim, s.S(), s.members(),
-                                                               s.sc.p, q->freqs.p, q->entropy.p, q->valid.p,
-                                                               is_member, d_order, pos0, delta_out);
+        k_sel_scan<<<count, kEntThreads, kEntSmemBytes + stage_bytes<Src>(2), st>>>(
+            rows(), f->entropy.p, dim, s.S(), s.members(), s.sc.p, cand_rows(q), q->entropy.p, q->valid.p, is_member,
+            d_order, pos0, delta_out);
         DVS_LAUNCHED(ctx);
         return DVS_OK;
     }
 };
 
+// The sparse forms stage up to 48 KB of rows on top of their own shared memory
+static int sparse_smem_setup() {
+    auto allow = [](auto kernel, size_t bytes) {
+        return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    };
+    cudaError_t e = cudaSuccess;
+    for (cudaError_t x : {allow(k_sel_scan_fast<SparseRows>, 2 * kStageBytes), allow(k_sel_update_fast<SparseRows>, kStageBytes),
+                          allow(k_sel_replace_update_fast<SparseRows>, 3 * kStageBytes),
+                          allow(k_grow_eval<SparseRows>, 2 * kStageBytes), allow(k_sel_replace_vec<SparseRows>, 2 * kStageBytes),
+                          allow(k_sel_update<SparseRows>, kEntSmemBytes + kStageBytes),
+                          allow(k_sel_scan<SparseRows>, kEntSmemBytes + 2 * kStageBytes)})
+        if (x != cudaSuccess && e == cudaSuccess) e = x;
+    if (e != cudaSuccess) {
+        set_error("dvs_select_sparse: shared memory for the staged rows: %s", cudaGetErrorString(e));
+        return DVS_ERR_CUDA;
+    }
+    return DVS_OK;
+}
+
 // One selection call: its arguments, the state and buffers on the device, and where the loop stands.  Each step
-// of the loop in select_core is a function of its own below.
+// of the loop in select_core is a function of its own below.  RS: the record set (dvs_kfreqs or dvs_ksparse).
+template <class RS>
 struct SelRun {
+    using Src = typename Selector<RS>::Src;
     dvs_ctx* ctx;
     dvs_comm* comm;
-    const dvs_kfreqs* f;
+    const RS* f;
     const uint32_t* order;
     uint32_t num;
     int mode;
@@ -459,7 +651,7 @@ struct SelRun {
     unsigned trail_limit = 0;
     std::vector<uint8_t> valid, err;  // validity / panic flags of the records
     std::vector<double> err_total;
-    Selector sel;
+    Selector<RS> sel;
     SelState A, B;
     SelState* cur = &A;
     SelState* alt = &B;
@@ -494,7 +686,8 @@ struct SelRun {
 };
 
 // trailing: wait until every record has been counted
-static int wait_counted(SelRun& r) {
+template <class RS>
+static int wait_counted(SelRun<RS>& r) {
     if (r.trail_limit >= r.num) return DVS_OK;
     DVS_CUDA_TRY(cudaStreamWaitEvent(r.st, r.trail->count_done, 0));
     r.trail_limit = r.num;
@@ -503,8 +696,9 @@ static int wait_counted(SelRun& r) {
 
 // reads the validity / panic flags of the records.  Every record in `order` goes through KmerSeq::new ->
 // entropy(), where a failing sum check panics: checked here for the positions below `upto`.
-static int read_flags(SelRun& r, unsigned upto) {
-    const dvs_kfreqs* f = r.f;
+template <class RS>
+static int read_flags(SelRun<RS>& r, unsigned upto) {
+    const RS* f = r.f;
     if (f->nrec) {
         DVS_CUDA_TRY(cudaMemcpyAsync(r.valid.data(), f->valid.p, f->nrec, cudaMemcpyDeviceToHost, r.st));
         DVS_CUDA_TRY(cudaMemcpyAsync(r.err.data(), f->err.p, f->nrec, cudaMemcpyDeviceToHost, r.st));
@@ -520,11 +714,41 @@ static int read_flags(SelRun& r, unsigned upto) {
     return DVS_OK;
 }
 
+// Sparse rows: the selection state is dense (S double buffered, 4^k f64 each), and `max` keeps two more copies for
+// the grown set and clone().  Fail with the sizes when they do not fit instead of on an allocation.  Memory that the
+// stream-ordered pool holds but does not use counts as free.
+template <class RS>
+static int sparse_state_fits(SelRun<RS>& r) {
+    const bool grow = r.grow_mode;
+    const uint64_t per = 2 * (r.dim * sizeof(double) + (uint64_t)r.cap * (sizeof(unsigned) + 2 * sizeof(double)));
+    const uint64_t need = per * (grow ? 3u : 1u) + (uint64_t)r.f->nrec + (uint64_t)r.num * sizeof(unsigned) +
+                          (grow ? (uint64_t)r.grow_window_max * r.cap * (sizeof(FastSum) + 2 * sizeof(double)) : 0u);
+    size_t free_b = 0, total_b = 0;
+    DVS_CUDA_TRY(cudaMemGetInfo(&free_b, &total_b));
+    uint64_t avail = free_b;
+    cudaMemPool_t pool;
+    if (cudaDeviceGetDefaultMemPool(&pool, r.ctx->device) == cudaSuccess) {
+        uint64_t reserved = 0, used = 0;
+        if (cudaMemPoolGetAttribute(pool, cudaMemPoolAttrReservedMemCurrent, &reserved) == cudaSuccess &&
+            cudaMemPoolGetAttribute(pool, cudaMemPoolAttrUsedMemCurrent, &used) == cudaSuccess && reserved > used)
+            avail += reserved - used;
+    }
+    (void)cudaGetLastError();
+    if (need + (64ull << 20) > avail) {
+        set_error("dvs_select_sparse: the selection state at k=%d needs %.1f MB of device memory (%s), %.1f MB are free",
+                  r.f->k, need / 1e6, grow ? "max: three double-buffered 4^k f64 sums" : "a double-buffered 4^k f64 sum",
+                  avail / 1e6);
+        return DVS_ERR_CUDA;
+    }
+    return DVS_OK;
+}
+
 // argument checks, the panic check over the published positions, the initial set and its state, the buffers,
 // and the round forms this call can use
-static int select_setup(SelRun& r) {
+template <class RS>
+static int select_setup(SelRun<RS>& r) {
     dvs_ctx* ctx = r.ctx;
-    const dvs_kfreqs* f = r.f;
+    const RS* f = r.f;
     const uint32_t* order = r.order;
     const uint32_t num = r.num;
     if (!ctx || !f || (!order && num) || !r.size_out) {
@@ -594,6 +818,7 @@ static int select_setup(SelRun& r) {
     const bool unbounded = r.grow_mode && r.max_size < (uint32_t)init.size();
     r.cap = (unbounded ? num : std::max<unsigned>(std::max(r.min_size, r.max_size), (unsigned)init.size())) + 1;
     r.n = (unsigned)init.size();
+    if constexpr (SelRun<RS>::Src::kSparse) DVS_TRY(sparse_state_fits(r));
     DVS_TRY(r.A.alloc(r.dim, r.cap));
     if (r.grow_mode) DVS_TRY(r.B.alloc(r.dim, r.cap));
     DVS_TRY(r.is_member.alloc(f->nrec));
@@ -605,7 +830,7 @@ static int select_setup(SelRun& r) {
     k_set_members<<<(unsigned)((init.size() + 255) / 256), 256, 0, r.st>>>(r.is_member.p, r.d_init.p, r.n, 1);
     DVS_LAUNCHED(ctx);
     r.pt.emplace(ctx, DVS_PHASE_SELECT);
-    r.sel = Selector{ctx, f, r.dim, r.st, (SelScal*)ctx->pinned};
+    r.sel = Selector<RS>{ctx, f, r.dim, r.st, (SelScal*)ctx->pinned};
     DVS_TRY(r.sel.build(*r.cur, r.d_init.p, r.n, -1));
     r.window_max = std::max(64u, (unsigned)ctx->sm_count * 12u);
     r.cursor = r.min_size;
@@ -616,7 +841,12 @@ static int select_setup(SelRun& r) {
     // DVS_SELECT_PERSIST=0: host-driven rounds, =1: the global-state persistent kernel; default: SM-replicated
     // rounds when the state fits in shared memory.  Host-driven rounds also run where cooperative launches do not.
     // DVS_SELECT_GRID: CTAs of the persistent kernels (tests run several ranks on ONE GPU: their kernels must be
-    // co-resident, so each takes a share of the SMs)
+    // co-resident, so each takes a share of the SMs).  Sparse rows take the host-driven rounds: one evaluation of a
+    // 4^12-element vector is far too long for a round of the persistent kernels to pay off.
+    if constexpr (SelRun<RS>::Src::kSparse) {
+        r.use_persist = r.sm_ok = false;
+        DVS_TRY(sparse_smem_setup());
+    } else {
     const char* grid_env = getenv("DVS_SELECT_GRID");
     const unsigned grid_cap = grid_env && atoi(grid_env) > 0 ? (unsigned)atoi(grid_env) : 0xFFFFFFFFu;
     const char* per_env = getenv("DVS_SELECT_PERSIST");
@@ -641,6 +871,7 @@ static int select_setup(SelRun& r) {
         DVS_TRY(r.d_upart.alloc(kSmMaxN + 1));
         DVS_TRY(r.d_dpart.alloc(3));  // the leader's broadcasts: scan decision (double buffered), update result
     }
+    }
     // batched grow attempts (see k_grow_eval): scratch for a window of candidates; DVS_SELECT_GROW_BATCH=0
     // keeps one host-driven attempt per candidate
     const char* gb_env = getenv("DVS_SELECT_GROW_BATCH");
@@ -659,20 +890,19 @@ static int select_setup(SelRun& r) {
 
 // max while the set grows: evaluate a window of grow attempts on the device and move the cursor to the first
 // candidate that could be adopted (the host path then decides it), past the window when none can
-static int grow_filter(SelRun& r) {
+template <class RS>
+static int grow_filter(SelRun<RS>& r) {
     if (r.filter_bypass > 0) {
         --r.filter_bypass;
         r.single_candidate = true;  // straight to the host path for this candidate
         return DVS_OK;
     }
     dvs_ctx* ctx = r.ctx;
-    const dvs_kfreqs* f = r.f;
+    const RS* f = r.f;
     SelState* cur = r.cur;
     const unsigned n = r.n, cursor = r.cursor, world = r.world;
     if (!r.fresh_valid || r.fresh_n != n || r.fresh_of != cur || r.fresh_which != cur->which) {
-        k_sel_sum<<<r.sel.vec_grid(), 256, 0, r.st>>>(f->freqs.p, f->entropy.p, r.dim, cur->members(), n, -1,
-                                                      r.fresh.S(), r.fresh.members(), r.fresh.sc.p);
-        DVS_LAUNCHED(ctx);
+        DVS_TRY(r.sel.sum(r.fresh, cur->members(), n, -1));
         r.fresh_valid = true;
         r.fresh_n = n;
         r.fresh_of = cur;
@@ -684,9 +914,9 @@ static int grow_filter(SelRun& r) {
     const unsigned gc0 = (r.rank + world - cursor % world) % world;
     const unsigned Wloc = W > gc0 ? (W - gc0 + world - 1) / world : 0;
     if (Wloc) {
-        k_grow_eval<<<dim3(n + 3, Wloc), kFastThreads, 0, r.st>>>(f->freqs.p, r.dim, cur->S(), cur->members(), cur->sc.p,
-                                                                  r.fresh.S(), f->valid.p, r.is_member.p, r.d_order.p,
-                                                                  cursor, r.d_gparts.p, gc0, world);
+        k_grow_eval<<<dim3(n + 3, Wloc), kFastThreads, stage_bytes<typename SelRun<RS>::Src>(2), r.st>>>(
+            r.sel.rows(), r.dim, cur->S(), cur->members(), cur->sc.p, r.fresh.S(), f->valid.p, r.is_member.p, r.d_order.p,
+            cursor, r.d_gparts.p, gc0, world);
         DVS_LAUNCHED(ctx);
         k_grow_decide<<<Wloc, kFastThreads, 0, r.st>>>(f->entropy.p, r.dim, cur->members(), cur->sc.p, r.fresh.sc.p,
                                                        f->valid.p, r.is_member.p, r.d_order.p, cursor, r.d_gparts.p,
@@ -745,9 +975,10 @@ static int write_trace(const unsigned long long* d_trace, size_t len, bool all, 
 // undecided candidate or state, which the host resolves exactly).  The SM-replicated kernel runs while the state
 // fits its shared memory, k_sel_persist otherwise.  Trailing the counting, the SM-replicated kernel takes
 // DVS_TRAIL_SMS whole SMs and returns when everything has been published; anything else waits for the counting.
-static int persist_rounds(SelRun& r, bool& halted) {
+template <class RS>
+static int persist_rounds(SelRun<RS>& r, bool& halted) {
     dvs_ctx* ctx = r.ctx;
-    const dvs_kfreqs* f = r.f;
+    const RS* f = r.f;
     SelState* cur = r.cur;
     const unsigned world = r.world;
     const bool use_sm = r.sm_ok && r.n <= kSmMaxN;
@@ -867,8 +1098,9 @@ static int persist_rounds(SelRun& r, bool& halted) {
 // one host-driven round: score a window of candidates, decide undecided candidates and states exactly, and let
 // the first acceptance replace the lowest record (records.rs:111-118).  While the set grows (max), the accepted
 // candidate is left in `grow_row` for grow_attempt instead, with the scan's scalars in `h`.
-static int host_window(SelRun& r, int& grow_row, SelScal& h) {
-    const dvs_kfreqs* f = r.f;
+template <class RS>
+static int host_window(SelRun<RS>& r, int& grow_row, SelScal& h) {
+    const RS* f = r.f;
     SelState* cur = r.cur;
     grow_row = -1;
     if (!r.use_persist || r.cursor >= r.trail_limit) DVS_TRY(wait_counted(r));  // (host rounds do not trail)
@@ -941,7 +1173,8 @@ static int host_window(SelRun& r, int& grow_row, SelScal& h) {
 // records.rs:434-451: nw = clone(); nw.push(rec); keep whichever has the larger statistic.  First tried with the
 // bounded-error kernels: the comparison is decided from them only when it holds for every admissible error;
 // otherwise both states are evaluated by the exact kernel.  `h`: the scalars of the current state.
-static int grow_attempt(SelRun& r, unsigned row, SelScal h) {
+template <class RS>
+static int grow_attempt(SelRun<RS>& r, unsigned row, SelScal h) {
     const bool use_cov = (r.mode == DVS_MODE_MAX_COV);
     auto adopt = [&]() -> int {
         std::swap(r.cur, r.alt);
@@ -983,7 +1216,8 @@ static int grow_attempt(SelRun& r, unsigned row, SelScal h) {
 
 // the panic check of the records that were not published when a trailing selection started, the exact
 // re-evaluation of the final state (reported numbers are exact), and the copies out
-static int select_finish(SelRun& r) {
+template <class RS>
+static int select_finish(SelRun<RS>& r) {
     dvs_ctx* ctx = r.ctx;
     if (r.trail) {
         DVS_CUDA_TRY(cudaStreamWaitEvent(r.st, r.trail->count_done, 0));
@@ -1017,10 +1251,11 @@ static int select_finish(SelRun& r) {
 // dvs_count_kmers_sharded / dvs_kfreqs_allgather), the same order and the same arguments: the state and
 // every host-side decision are replicated (identical inputs, identical kernels), while the windows of
 // candidates are scored candidate-sharded with an all-reduce(min) of the first interesting position.
-static int select_core(dvs_ctx* ctx, dvs_comm* comm, const dvs_kfreqs* f, const uint32_t* order, uint32_t num, int mode,
+template <class RS>
+static int select_core(dvs_ctx* ctx, dvs_comm* comm, const RS* f, const uint32_t* order, uint32_t num, int mode,
                        uint32_t min_size, uint32_t max_size, uint32_t* sel_idx, double* sel_delta, double* stats5,
                        uint32_t* size_out, const TrailArgs* trail = nullptr) {
-    SelRun r{ctx, comm, f, order, num, mode, min_size, max_size, sel_idx, sel_delta, stats5, size_out, trail};
+    SelRun<RS> r{ctx, comm, f, order, num, mode, min_size, max_size, sel_idx, sel_delta, stats5, size_out, trail};
     DVS_TRY(select_setup(r));
     while (r.cursor < num) {
         const bool growing = r.grow_mode && r.n != r.max_size;  // max below its size: candidates join the set
@@ -1028,11 +1263,13 @@ static int select_core(dvs_ctx* ctx, dvs_comm* comm, const dvs_kfreqs* f, const 
             DVS_TRY(grow_filter(r));  // batched grow attempts isolate the next candidate worth one
             continue;
         }
-        if (!growing && r.use_persist) {  // replacing rounds on the device, until they finish or halt
-            bool halted = false;
-            DVS_TRY(persist_rounds(r, halted));
-            if (!halted) continue;
-            if (r.cursor >= num) break;
+        if constexpr (!SelRun<RS>::Src::kSparse) {  // (sparse rows: host-driven rounds only)
+            if (!growing && r.use_persist) {  // replacing rounds on the device, until they finish or halt
+                bool halted = false;
+                DVS_TRY(persist_rounds(r, halted));
+                if (!halted) continue;
+                if (r.cursor >= num) break;
+            }
         }
         // host-driven: the rounds themselves without persistent kernels (DVS_SELECT_PERSIST=0, exact-only,
         // no cooperative launch), a halted round's exact decision, and every candidate of a growing set
@@ -1077,6 +1314,21 @@ int dvs_select_sharded(dvs_ctx* ctx, dvs_comm* comm, const dvs_kfreqs* f_all, co
     }
     return select_core(ctx, comm->world > 1 ? comm : nullptr, f_all, order, num, mode, min_size, max_size, sel_idx,
                        sel_delta, stats5, size_out);
+}
+
+int dvs_select_sparse(dvs_ctx* ctx, const dvs_ksparse* sp, const uint32_t* order, uint32_t num, int mode,
+                      uint32_t min_size, uint32_t max_size, uint32_t* sel_idx, double* sel_delta, double* stats5,
+                      uint32_t* size_out) {
+    if (sp && !sp->has_entropy) {
+        set_error("dvs_select_sparse: the rows were counted without entropies (dvs_count_kmers_sparse with want_entropy = 0)");
+        return DVS_ERR_ARG;
+    }
+    if (sp && sp->dim % kSpLowBins != 0) {
+        set_error("dvs_select_sparse: 4^k = %llu is not a whole number of %u-bin buckets", (unsigned long long)sp->dim,
+                  kSpLowBins);
+        return DVS_ERR_ARG;
+    }
+    return select_core(ctx, nullptr, sp, order, num, mode, min_size, max_size, sel_idx, sel_delta, stats5, size_out);
 }
 
 int dvs_debug_fast_terms(dvs_ctx* ctx, const double* a, const double* b, double* m, double* l, int32_t* special,
@@ -1140,7 +1392,7 @@ int dvs_summed_create(dvs_ctx* ctx, const dvs_kfreqs* f, const uint32_t* members
             rc = DVS_ERR_CUDA;
         }
     }
-    Selector sel{ctx, f, f->dim, ctx->stream, (SelScal*)ctx->pinned};
+    Selector<dvs_kfreqs> sel{ctx, f, f->dim, ctx->stream, (SelScal*)ctx->pinned};
     if (rc == DVS_OK) rc = sel.build(s->st, d_m.p, n, -1);
     if (rc == DVS_OK) rc = sel.read(s->st);
     if (rc == DVS_OK && sel.h_sc->panic) rc = panic_error(*sel.h_sc);
@@ -1163,7 +1415,7 @@ int dvs_summed_delta_jsd(dvs_ctx* ctx, dvs_summed* s, const dvs_kfreqs* q, uint3
         return DVS_OK;
     }
     DVS_CUDA_TRY(dvs::enter(ctx));
-    Selector sel{ctx, s->f, s->f->dim, ctx->stream, (SelScal*)ctx->pinned};
+    Selector<dvs_kfreqs> sel{ctx, s->f, s->f->dim, ctx->stream, (SelScal*)ctx->pinned};
     DevBuf<double> d_out;
     DVS_TRY(d_out.alloc(1));
     // a window of one candidate at position == row (order == nullptr); validity is the caller's business
@@ -1187,7 +1439,7 @@ int dvs_summed_delta_jsd_batch(dvs_ctx* ctx, dvs_summed* s, const dvs_kfreqs* q,
     const uint32_t nq = q->nrec;
     if (nq == 0) return DVS_OK;
     DVS_CUDA_TRY(dvs::enter(ctx));
-    Selector sel{ctx, s->f, s->f->dim, ctx->stream, (SelScal*)ctx->pinned};
+    Selector<dvs_kfreqs> sel{ctx, s->f, s->f->dim, ctx->stream, (SelScal*)ctx->pinned};
     DevBuf<double> d_out;
     DevBuf<uint8_t> d_mem;
     DVS_TRY(d_out.alloc(nq));
@@ -1199,7 +1451,7 @@ int dvs_summed_delta_jsd_batch(dvs_ctx* ctx, dvs_summed* s, const dvs_kfreqs* q,
     DVS_CUDA_TRY(cudaMemsetAsync(d_out.p, 0, nq * sizeof(double), ctx->stream));
     DVS_TRY(sel.reset_scan(s->st));
     // one CTA per query row; position == row (order == nullptr); invalid / member rows are skipped
-    k_sel_scan<<<nq, kEntThreads, kEntSmemBytes, ctx->stream>>>(s->f->freqs.p, s->f->entropy.p, s->f->dim, s->st.S(),
+    k_sel_scan<<<nq, kEntThreads, kEntSmemBytes, ctx->stream>>>(DenseRows{s->f->freqs.p}, s->f->entropy.p, s->f->dim, s->st.S(),
                                                                  s->st.members(), s->st.sc.p, q->freqs.p,
                                                                  q->entropy.p, q->valid.p, d_mem.p, nullptr, 0u,
                                                                  d_out.p);
@@ -1222,7 +1474,7 @@ int dvs_summed_delta_jsd_batch(dvs_ctx* ctx, dvs_summed* s, const dvs_kfreqs* q,
 int dvs_summed_result(dvs_ctx* ctx, dvs_summed* s, uint32_t* sel_idx, double* sel_delta, double* stats5,
                       uint32_t* size_out, uint32_t* lowest_out) {
     DVS_CUDA_TRY(dvs::enter(ctx));
-    Selector sel{ctx, s->f, s->f->dim, ctx->stream, (SelScal*)ctx->pinned};
+    Selector<dvs_kfreqs> sel{ctx, s->f, s->f->dim, ctx->stream, (SelScal*)ctx->pinned};
     DVS_TRY(sel.read(s->st));
     const SelScal h = *sel.h_sc;
     if (sel_idx)

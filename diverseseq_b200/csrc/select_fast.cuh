@@ -24,9 +24,10 @@ struct FastSum {
     int bad;         // a negative / NaN frequency was seen (reference yields NaN): cannot be bounded
 };
 
-// elements [lo, hi) of a vector (the SM-replicated selection kernel splits one vector over several CTAs)
-template <class Elem>
-__device__ FastSum block_entropy_span(uint64_t lo, uint64_t dim, Elem elem) {
+// elements [lo, hi) of a vector (the SM-replicated selection kernel splits one vector over several CTAs).
+// `stage(base)`: a row source's staging hook, called by every thread before each pass of 8 x kFastThreads elements
+template <class Elem, class Stage = NoStage>
+__device__ FastSum block_entropy_span(uint64_t lo, uint64_t dim, Elem elem, Stage stage = Stage()) {
     __shared__ double s_part[3][kFastThreads / 32];
     __shared__ int s_bad[kFastThreads / 32];
     double e0 = 0.0, e1 = 0.0, t0 = 0.0, t1 = 0.0, a0 = 0.0, a1 = 0.0;
@@ -35,6 +36,7 @@ __device__ FastSum block_entropy_span(uint64_t lo, uint64_t dim, Elem elem) {
     // first log2 so one memory latency is exposed per pass, not one per element
     constexpr int kBatch = 8;
     for (uint64_t base = lo; base < dim; base += (uint64_t)kBatch * kFastThreads) {
+        stage(base);
         double x[kBatch];
 #pragma unroll
         for (int q = 0; q < kBatch; ++q) {
@@ -75,9 +77,9 @@ __device__ FastSum block_entropy_span(uint64_t lo, uint64_t dim, Elem elem) {
     __syncthreads();
     return r;
 }
-template <class Elem>
-__device__ __forceinline__ FastSum block_entropy_fast(uint64_t dim, Elem elem) {
-    return block_entropy_span(0, dim, elem);
+template <class Elem, class Stage = NoStage>
+__device__ __forceinline__ FastSum block_entropy_fast(uint64_t dim, Elem elem, Stage stage = Stage()) {
+    return block_entropy_span(0, dim, elem, stage);
 }
 
 // ---- the same sums with instruction-level parallelism (SM-replicated rounds) ----
@@ -97,14 +99,15 @@ __device__ __forceinline__ bool fast_term_ok(double m) {
     return (uint32_t)__double2hiint(m) - 0x07b00000u < 0x3feea4afu - 0x07b00000u;
 }
 
-template <bool CLAMP, int BATCH, int NT = kFastThreads, class Num>
+template <bool CLAMP, int BATCH, int NT = kFastThreads, class Num, class Stage = NoStage>
 __device__ FastSum block_entropy_ilp(unsigned lo, unsigned hi, Num num, const FastDiv dv,
-                                     const double2* __restrict__ ltab) {
+                                     const double2* __restrict__ ltab, Stage stage = Stage()) {
     __shared__ double s_part[3][NT / 32];
     __shared__ int s_bad[NT / 32];
     double e0 = 0.0, e1 = 0.0, t0 = 0.0, t1 = 0.0, a0 = 0.0, a1 = 0.0;
     bool bad = false;
     for (unsigned base = lo; base < hi; base += BATCH * NT) {
+        stage(base);
         double x[BATCH], l[BATCH];
 #pragma unroll
         for (int q = 0; q < BATCH; ++q) {
@@ -159,19 +162,20 @@ __device__ FastSum block_entropy_ilp(unsigned lo, unsigned hi, Num num, const Fa
 // cooperative kernel, the batched grow attempts — the k >= 7 paths): m_i =
 // num(i) / divisor, optionally clamped (<= EPS -> 0).  Stages the log2 table itself; divisors beyond the
 // range the exact division was verified for, and vectors longer than 2^30, take the one-element-at-a-time
-// form with __ddiv_rn (same values either way).
-template <bool CLAMP, class Num>
-__device__ FastSum block_entropy_div(uint64_t dim, Num num, double divisor) {
+// form with __ddiv_rn (same values either way).  Both forms take passes of 8 x kFastThreads = 4,096 elements, which
+// is one bucket of a sparse row: `stage` is the row source's hook (select.cu).
+template <bool CLAMP, class Num, class Stage = NoStage>
+__device__ FastSum block_entropy_div(uint64_t dim, Num num, double divisor, Stage stage = Stage()) {
     if (dim > (1ull << 30) || !(divisor >= 1.0 && divisor <= 4096.0)) {  // block-uniform
         return block_entropy_fast(dim, [&](uint64_t i) {
             const double m = __ddiv_rn(num(i), divisor);
             return (CLAMP && m <= kEps) ? 0.0 : m;
-        });
+        }, stage);
     }
     __shared__ double2 s_ltab_div[64];
     dvs_log2_stage_table(s_ltab_div);
     __syncthreads();
-    return block_entropy_ilp<CLAMP, 8>(0u, (unsigned)dim, num, make_fast_div(divisor), s_ltab_div);
+    return block_entropy_ilp<CLAMP, 8>(0u, (unsigned)dim, num, make_fast_div(divisor), s_ltab_div, stage);
 }
 
 // Each thread first sums dim/kFastThreads elements sequentially, then the partials are tree-summed:
@@ -328,7 +332,8 @@ struct ScanScal {
 };
 
 // fast increases_jsd of the candidate at position `pos`; first_true / first_unsure by atomicMin
-__device__ __forceinline__ void scan_fast_body(const double* __restrict__ F, const double* __restrict__ H, uint64_t dim,
+template <class Src>
+__device__ __forceinline__ void scan_fast_body(const Src src, const double* __restrict__ H, uint64_t dim,
                                                const double* __restrict__ S, SelScal* sc, const ScanScal& q,
                                                const uint8_t* __restrict__ valid,
                                                const uint8_t* __restrict__ is_member,
@@ -336,10 +341,11 @@ __device__ __forceinline__ void scan_fast_body(const double* __restrict__ F, con
     const unsigned row = order[pos];
     if (!valid[row] || __ldcg(is_member + row)) return;
     const double nd = (double)q.n;
-    const double* fl = F + (size_t)q.low_row * dim;
-    const double* fc = F + (size_t)row * dim;
+    auto v = src.view(stage_smem<Src>());
+    const auto fl = v.row(0, q.low_row, dim);
+    const auto fc = v.row(1, row, dim);
     FastSum h = block_entropy_div<false>(
-        dim, [&](uint64_t i) { return __dadd_rn(__dsub_rn(__ldcg(S + i), fl[i]), fc[i]); }, nd);
+        dim, [&](uint64_t i) { return __dadd_rn(__dsub_rn(__ldcg(S + i), fl[i]), fc[i]); }, nd, stager(v));
     if (threadIdx.x == 0) {
         const double mean_entropy = __ddiv_rn(__dadd_rn(__dsub_rn(q.E, H[q.low_row]), H[row]), nd);
         const double d = h.e - mean_entropy;
@@ -366,17 +372,20 @@ __device__ __forceinline__ ScanScal load_scan_scal(const SelScal* sc, const unsi
 }
 
 // host-driven window: one CTA per position pos0 + blockIdx.x
+template <class Src>
 __global__ void __launch_bounds__(kFastThreads)
-k_sel_scan_fast(const double* __restrict__ F, const double* __restrict__ H, uint64_t dim, const double* __restrict__ S,
+k_sel_scan_fast(const Src src, const double* __restrict__ H, uint64_t dim, const double* __restrict__ S,
                 const unsigned* __restrict__ members, SelScal* sc, const uint8_t* __restrict__ valid,
                 const uint8_t* __restrict__ is_member, const unsigned* __restrict__ order, unsigned pos0) {
-    scan_fast_body(F, H, dim, S, sc, load_scan_scal(sc, members), valid, is_member, order, pos0 + blockIdx.x);
+    const ScanScal q = load_scan_scal(sc, members);
+    scan_fast_body(src, H, dim, S, sc, q, valid, is_member, order, pos0 + blockIdx.x);
 }
 
 // fast total_jsd + get_lowest_record_index: same shape as k_sel_update.  Leaves approximate
 // total_jsd (with total_bound) and mdelta, and lowest_index only if it is certain.
+template <class Src>
 __global__ void __launch_bounds__(kFastThreads)
-k_sel_update_fast(const double* __restrict__ F, const double* __restrict__ H, uint64_t dim,
+k_sel_update_fast(const Src src, const double* __restrict__ H, uint64_t dim,
                   const double* __restrict__ S, const unsigned* __restrict__ members, double* __restrict__ mdelta,
                   double* __restrict__ mbound, SelScal* sc) {
     __shared__ unsigned s_last;
@@ -393,8 +402,9 @@ k_sel_update_fast(const double* __restrict__ F, const double* __restrict__ H, ui
     } else {
         const unsigned row = members[j];
         const double div = __dsub_rn(nd, 1.0);
-        const double* f = F + (size_t)row * dim;
-        FastSum h = block_entropy_div<true>(dim, [&](uint64_t i) { return __dsub_rn(S[i], f[i]); }, div);
+        auto v = src.view(stage_smem<Src>());
+        const auto f = v.row(0, row, dim);
+        FastSum h = block_entropy_div<true>(dim, [&](uint64_t i) { return __dsub_rn(S[i], f[i]); }, div, stager(v));
         if (threadIdx.x == 0) {
             const double mean_entropy = __ddiv_rn(__dsub_rn(sc->E, H[row]), div);
             mdelta[j] = h.e - mean_entropy;
@@ -430,16 +440,18 @@ k_sel_update_fast(const double* __restrict__ F, const double* __restrict__ H, ui
 // operations as k_sel_replace_vec, so S' is bitwise the reference's); CTA n also stores S' and the
 // last CTA to finish stores the new member list / scalars into the other buffer set.
 // dev_pos != kNone: device-driven round; the last CTA also advances cursor / window / accepts / which.
+template <class Src>
 __device__ __forceinline__ void replace_update_fast_body(
-    const double* __restrict__ F, const double* __restrict__ H, uint64_t dim, const double* __restrict__ S_in,
+    const Src src, const double* __restrict__ H, uint64_t dim, const double* __restrict__ S_in,
     double* __restrict__ S_out, const unsigned* __restrict__ m_in, unsigned* __restrict__ m_out,
     uint8_t* __restrict__ is_member, double* __restrict__ mdelta, double* __restrict__ mbound, SelScal* sc,
     unsigned cand_row, unsigned dev_pos, unsigned dev_cursor, unsigned j, unsigned n, unsigned low, double E_old) {
     __shared__ unsigned s_last;
     const double nd = (double)n;
     const unsigned low_row = __ldcg(m_in + low);
-    const double* fl = F + (size_t)low_row * dim;
-    const double* fc = F + (size_t)cand_row * dim;
+    auto v = src.view(stage_smem<Src>());
+    const auto fl = v.row(0, low_row, dim);
+    const auto fc = v.row(1, cand_row, dim);
     const double E_new = __dadd_rn(__dsub_rn(E_old, H[low_row]), H[cand_row]);  // records.rs:101,129
     auto s_new = [&](uint64_t i) {
         double s = __dsub_rn(__ldcg(S_in + i), fl[i]);
@@ -451,7 +463,7 @@ __device__ __forceinline__ void replace_update_fast_body(
             const double s = s_new(i);
             S_out[i] = s;
             return s;
-        }, nd);
+        }, nd, stager(v));
         if (threadIdx.x == 0) {
             const double me = __ddiv_rn(E_new, nd);
             sc->total_jsd = h.e - me;
@@ -462,8 +474,8 @@ __device__ __forceinline__ void replace_update_fast_body(
         // member j of the list after Vec::remove(low) + push(cand)
         const unsigned row = j < low ? __ldcg(m_in + j) : (j + 1 < n ? __ldcg(m_in + j + 1) : cand_row);
         const double div = __dsub_rn(nd, 1.0);
-        const double* f = F + (size_t)row * dim;
-        FastSum h = block_entropy_div<true>(dim, [&](uint64_t i) { return __dsub_rn(s_new(i), f[i]); }, div);
+        const auto f = v.row(2, row, dim);
+        FastSum h = block_entropy_div<true>(dim, [&](uint64_t i) { return __dsub_rn(s_new(i), f[i]); }, div, stager(v));
         if (threadIdx.x == 0) {
             const double mean_entropy = __ddiv_rn(__dsub_rn(E_new, H[row]), div);
             mdelta[j] = h.e - mean_entropy;
@@ -505,13 +517,14 @@ __device__ __forceinline__ void replace_update_fast_body(
     }
 }
 
+template <class Src>
 __global__ void __launch_bounds__(kFastThreads)
-k_sel_replace_update_fast(const double* __restrict__ F, const double* __restrict__ H, uint64_t dim,
+k_sel_replace_update_fast(const Src src, const double* __restrict__ H, uint64_t dim,
                           const double* __restrict__ S_in, double* __restrict__ S_out,
                           const unsigned* __restrict__ m_in, unsigned* __restrict__ m_out,
                           uint8_t* __restrict__ is_member, double* __restrict__ mdelta, double* __restrict__ mbound,
                           SelScal* sc, unsigned cand_row) {
-    replace_update_fast_body(F, H, dim, S_in, S_out, m_in, m_out, is_member, mdelta, mbound, sc, cand_row, kNone, 0u,
+    replace_update_fast_body(src, H, dim, S_in, S_out, m_in, m_out, is_member, mdelta, mbound, sc, cand_row, kNone, 0u,
                              blockIdx.x, sc->n, sc->lowest, sc->E);
 }
 
@@ -724,7 +737,7 @@ k_sel_persist(const double* __restrict__ F, const double* __restrict__ H, uint64
             while (P < kMaxSlices && nloc * P * 2u <= gridDim.x) P *= 2u;
         if (P == 1u) {
             for (unsigned c = woff + world * blockIdx.x; c < count; c += world * gridDim.x)
-                scan_fast_body(F, H, dim, which ? S1 : S0, sc, q, valid, is_member, order, cursor + c);
+                scan_fast_body(DenseRows{F}, H, dim, which ? S1 : S0, sc, q, valid, is_member, order, cursor + c);
         } else if (blockIdx.x < nloc * P) {  // slice s of this GPU's candidate c of the window
             const unsigned c = blockIdx.x / P, s = blockIdx.x % P;
             scan_sliced_body(F, H, dim, which ? S1 : S0, sc, q, valid, is_member, order, cursor + woff + world * c, s, P,
@@ -781,7 +794,7 @@ k_sel_persist(const double* __restrict__ F, const double* __restrict__ H, uint64
             }
             if (Pu == 1u) {
                 for (unsigned j = blockIdx.x; j <= n; j += gridDim.x)
-                    replace_update_fast_body(F, H, dim, which ? S1 : S0, which ? S0 : S1, which ? M1 : M0, which ? M0 : M1,
+                    replace_update_fast_body(DenseRows{F}, H, dim, which ? S1 : S0, which ? S0 : S1, which ? M1 : M0, which ? M0 : M1,
                                              is_member, mdelta, mbound, sc, cand_row, ft, cursor, j, n, rs.lowest, q.E);
             } else {
                 for (unsigned u = blockIdx.x; u < (n + 1u) * Pu; u += gridDim.x) {

@@ -14,8 +14,9 @@
 // does not improve the statistic; the first candidate that is anything else is handed to the existing
 // host path (which adopts it, or decides it exactly).  Decisions are unchanged, only certain discards
 // are taken in bulk.
+template <class Src>
 __global__ void __launch_bounds__(kFastThreads)
-k_grow_eval(const double* __restrict__ F, uint64_t dim, const double* __restrict__ S_cur,
+k_grow_eval(const Src src, uint64_t dim, const double* __restrict__ S_cur,
             const unsigned* __restrict__ members, const SelScal* __restrict__ sc_cur,
             const double* __restrict__ S_fresh, const uint8_t* __restrict__ valid,
             const uint8_t* __restrict__ is_member, const unsigned* __restrict__ order, unsigned cursor,
@@ -24,19 +25,20 @@ k_grow_eval(const double* __restrict__ F, uint64_t dim, const double* __restrict
     const unsigned c = c0 + cstride * blockIdx.y, t = blockIdx.x, n = sc_cur->n;
     const unsigned row = order[cursor + c];
     if (!valid[row] || is_member[row]) return;
-    const double* fc = F + (size_t)row * dim;
+    auto v = src.view(stage_smem<Src>());
+    const auto fc = v.row(0, row, dim);
     const double nd = (double)n;
     FastSum h;
     if (t == 0) {  // increases_jsd against the current state (records.rs:70-92)
-        const double* fl = F + (size_t)members[sc_cur->lowest] * dim;
-        h = block_entropy_div<false>(dim, [&](uint64_t i) { return __dadd_rn(__dsub_rn(S_cur[i], fl[i]), fc[i]); }, nd);
+        const auto fl = v.row(1, members[sc_cur->lowest], dim);
+        h = block_entropy_div<false>(dim, [&](uint64_t i) { return __dadd_rn(__dsub_rn(S_cur[i], fl[i]), fc[i]); }, nd, stager(v));
     } else if (t == 1) {  // total of the grown set: clone() re-sums in member order, push adds the candidate
         const double nd1 = __dadd_rn(nd, 1.0);
-        h = block_entropy_div<false>(dim, [&](uint64_t i) { return __dadd_rn(S_fresh[i], fc[i]); }, nd1);
+        h = block_entropy_div<false>(dim, [&](uint64_t i) { return __dadd_rn(S_fresh[i], fc[i]); }, nd1, stager(v));
     } else {  // leave-one-out of member j of the grown set (j == n: the candidate itself)
         const unsigned j = t - 2;
-        const double* f = j < n ? F + (size_t)members[j] * dim : fc;
-        h = block_entropy_div<true>(dim, [&](uint64_t i) { return __dsub_rn(__dadd_rn(S_fresh[i], fc[i]), f[i]); }, nd);
+        const auto f = v.row(1, j < n ? members[j] : row, dim);
+        h = block_entropy_div<true>(dim, [&](uint64_t i) { return __dsub_rn(__dadd_rn(S_fresh[i], fc[i]), f[i]); }, nd, stager(v));
     }
     if (threadIdx.x == 0) parts[(size_t)c * (n + 3) + t] = h;
 }

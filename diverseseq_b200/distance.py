@@ -74,6 +74,16 @@ def counts_sparse_for_euclidean(k: int, num_states: int) -> bool:
     return num_states == 4 and 10 <= k <= 12
 
 
+def counts_sparse_for_selection(k: int, num_states: int) -> bool:
+    """Whether nmost / max select from sparse k-mer rows (dvs_count_kmers_sparse + dvs_select_sparse) instead of
+    dense frequency rows: for DNA at 10 <= k <= 12.  A dense row takes 12 x 4^k bytes whatever the record's length
+    (201 MB at k = 12), a sparse one 8 bytes per sequence byte; the selection state stays dense either way.  At
+    k = 10 on 1,000 records of 1.5 kbp (B200) nmost n = 100 took 6.1 s from sparse rows against 9.5 s from dense ones,
+    max stdev 124 against 95 ms, with 0.07 against 25 GB of device memory (DESIGN.md §5.12).  k = 9 keeps the dense
+    rows (3 MB each)."""
+    return num_states == 4 and 10 <= k <= 12
+
+
 def euclidean_distances(seq_arrays, k: int, moltype: str = "dna", *, progress=None) -> NamedDistances:
     num_states = seq_arrays[0].num_states if len(seq_arrays) and hasattr(seq_arrays[0], "num_states") else 4
     ctx = _lib.default_context()

@@ -196,6 +196,15 @@ int dvs_euclid_distances_sparse(dvs_ctx* ctx, const dvs_ksparse* sp, uint32_t ro
 int dvs_select(dvs_ctx* ctx, const dvs_kfreqs* f, const uint32_t* order, uint32_t num, int mode,
                uint32_t min_size, uint32_t max_size, uint32_t* sel_idx, double* sel_delta, double* stats5,
                uint32_t* size_out);
+/* dvs_select over sparse rows (dvs_count_kmers_sparse with want_entropy != 0, else DVS_ERR_ARG): the same contract,
+ * errors and results bit for bit as dvs_select over the dense rows of the same records - validity, entropies and
+ * the panic flags come from the sparse counting - without any dense row in memory.  The selection state stays dense
+ * (a double-buffered 4^k f64 sum; three of them for max): a call whose state does not fit the free device memory
+ * fails with DVS_ERR_CUDA and the sizes before allocating anything.  Always host-driven rounds (DESIGN.md §5.12);
+ * DVS_SELECT_EXACT_ONLY and dvs_select_last_accepts / dvs_select_last_exact_evals apply as to dvs_select. */
+int dvs_select_sparse(dvs_ctx* ctx, const dvs_ksparse* sp, const uint32_t* order, uint32_t num, int mode,
+                      uint32_t min_size, uint32_t max_size, uint32_t* sel_idx, double* sel_delta, double* stats5,
+                      uint32_t* size_out);
 /* number of candidates that changed the set during the last dvs_select on this ctx */
 uint32_t dvs_select_last_accepts(dvs_ctx* ctx);
 /* number of exact re-evaluations the bounded-error fast path had to request during the last
