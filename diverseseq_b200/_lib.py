@@ -111,6 +111,10 @@ SIGNATURES = {
     "dvs_euclid_distances_sharded": (_i32, [_vp, _vp, _vp, _vp]),
     "dvs_euclid_distances_sparse_sharded": (_i32, [_vp, _vp, _vp, _vp, _vp]),
     "dvs_select_sharded": (_i32, [_vp, _vp, _vp, _vp, _u32, _i32, _u32, _u32, _vp, _vp, _vp, C.POINTER(_u32)]),
+    "dvs_select_sparse_sharded": (_i32, [_vp, _vp, _vp, _vp, _vp, _u32, _i32, _u32, _u32, _vp, _vp, _vp,
+                                         C.POINTER(_u32)]),
+    "dvs_select_last_rows_fetched": (_u32, [_vp]),
+    "dvs_select_last_bytes_fetched": (_u64, [_vp]),
     "dvs_debug_pack_host": (_i32, [_vp, _u64, _vp, _vp, _vp, _u32, C.POINTER(_u32)]),
     "dvs_debug_log2": (_i32, [_vp, _vp, _vp, _u64]),
     "dvs_debug_fast_terms": (_i32, [_vp, _vp, _vp, _vp, _vp, _vp, _u64]),
@@ -629,6 +633,32 @@ class KSparse(_Handle):
                                               ptr(stats), C.byref(size)))
         n = size.value
         return idx[:n].copy(), delta[:n].copy(), stats
+
+    def select_sharded(self, comm: "Comm", nrec_per_rank, order, mode: int, min_size: int, max_size: int = 0):
+        """nmost / max over the sparse rows of ALL ranks, each rank passing its own (collective,
+        dvs_select_sparse_sharded): `order` indexes the rank-major rows of all ranks; every rank gets the
+        (row indices, delta_jsd, stats5) `select` gives over the union of the records"""
+        npr = np.ascontiguousarray(nrec_per_rank, dtype=np.uint32)
+        assert npr.size == comm.world
+        order = np.ascontiguousarray(order, dtype=np.uint32)
+        cap = max(int(min_size), int(max_size), 1) + 1
+        if int(mode) != MODE_NMOST and int(max_size) < int(min_size):
+            cap = order.size + 1  # the set can grow without bound (dvs_b200.h, dvs_select)
+        idx = np.zeros(cap, dtype=np.uint32)
+        delta = np.zeros(cap, dtype=np.float64)
+        stats = np.zeros(5, dtype=np.float64)
+        size = _u32(0)
+        check(self.ctx._lib.dvs_select_sparse_sharded(self.ctx.handle, comm.handle, self.handle, ptr(npr),
+                                                      ptr(order) if order.size else None, order.size, int(mode),
+                                                      int(min_size), int(max_size), ptr(idx), ptr(delta), ptr(stats),
+                                                      C.byref(size)))
+        n = size.value
+        return idx[:n].copy(), delta[:n].copy(), stats
+
+    def rows_fetched(self) -> tuple[int, int]:
+        """(rows, bytes) this rank copied in from peers during the last `select_sharded` on this context"""
+        lib, h = self.ctx._lib, self.ctx.handle
+        return int(lib.dvs_select_last_rows_fetched(h)), int(lib.dvs_select_last_bytes_fetched(h))
 
     def dense_rows(self, rows) -> np.ndarray:
         """frequency rows `rows` as one [len(rows), num_states^k] f64 array, formed on the host from the downloaded

@@ -118,6 +118,8 @@ struct dvs_ctx {
     uint32_t last_trail_launches = 0, last_trail_sms = 0;  // trailing kernel launches / fewest distinct SMs one sat on
     uint32_t last_trail_accepts = 0;  // of those, made while the counting was still running (dvs_count_select)
     uint32_t last_exact_evals = 0;  // exact re-evaluations forced by the fast path's error bound
+    uint32_t last_rows_fetched = 0;   // peer rows copied in by the last dvs_select_sparse_sharded on this rank
+    uint64_t last_bytes_fetched = 0;
     uint64_t last_upload_wire_bytes = 0;
     uint32_t last_euclid_fallback_pairs = 0;  // pairs the Gram-form Euclid kernel handed to the difference form
     double euclid_rows_ms = -1.0;  // peer row copies of the last dvs_euclid_distances_sparse_sharded (timing on)

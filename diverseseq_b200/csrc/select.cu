@@ -20,6 +20,7 @@
 #include <algorithm>
 #include <limits>
 #include <optional>
+#include <type_traits>
 
 #include <cooperative_groups.h>
 
@@ -140,11 +141,30 @@ struct SparseRowsData {
         return offsets[r] + bucket_ptr[(size_t)r * (nb + 1) + b];
     }
     __device__ __forceinline__ uint32_t bucket_len(unsigned r, uint32_t b) const { return bucket_nnz[(size_t)r * nb + b]; }
+    // the arrays that hold record r, and r's row in them: these
+    __device__ __forceinline__ const SparseRowsData& part(unsigned&) const { return *this; }
 };
-struct SparseRows : SparseRowsData {
+
+// dvs_select_sparse_sharded: the rows a rank reads are its own (`local`) or peer rows copied into its member-row
+// cache (`cache`, one row per slot); where[r] tells which for global row r.  Totals are indexed by global row.
+constexpr uint32_t kCachedRow = 0x80000000u;  // where[r]: cache slot (low bits) instead of a local row
+constexpr uint32_t kAbsentRow = 0xFFFFFFFFu;  // where[r]: neither (never read)
+struct ShardRowsData {
+    SparseRowsData local, cache;
+    const uint32_t* where;
+    const uint64_t* totals;
+    __device__ __forceinline__ SparseRowsData part(unsigned& r) const {
+        const uint32_t w = where[r];
+        r = w & ~kCachedRow;
+        return (w & kCachedRow) ? cache : local;
+    }
+};
+
+template <class D>
+struct SparseRowsT : D {
     static constexpr bool kSparse = true;
     struct View {
-        SparseRowsData src;
+        D src;
         uint32_t* smem;  // kStageSlots x 4,096 counts
         unsigned rows[kStageSlots];
         int nbound;
@@ -164,10 +184,12 @@ struct SparseRows : SparseRowsData {
 #pragma unroll
             for (int q = 0; q < kStageSlots; ++q) {
                 if (q < nbound) {
-                    const uint64_t at = src.bucket_at(rows[q], b);
-                    const uint32_t n = src.bucket_len(rows[q], b);
+                    unsigned r = rows[q];
+                    const auto& p = src.part(r);
+                    const uint64_t at = p.bucket_at(r, b);
+                    const uint32_t n = p.bucket_len(r, b);
                     uint32_t* d = smem + (size_t)q * kSpLowBins;
-                    for (uint32_t e = threadIdx.x; e < n; e += blockDim.x) d[src.idx[at + e] & (kSpLowBins - 1u)] = src.cnt[at + e];
+                    for (uint32_t e = threadIdx.x; e < n; e += blockDim.x) d[p.idx[at + e] & (kSpLowBins - 1u)] = p.cnt[at + e];
                 }
             }
             __syncthreads();
@@ -175,10 +197,13 @@ struct SparseRows : SparseRowsData {
     };
     __device__ __forceinline__ View view(uint32_t* smem) const { return View{*this, smem, {0u, 0u, 0u}, 0}; }
 };
+struct SparseRows : SparseRowsT<SparseRowsData> {};
+struct ShardRows : SparseRowsT<ShardRowsData> {};
 
 // the staging hook a kernel hands to the entropy helpers: the view itself, or nothing for dense rows
 __device__ __forceinline__ NoStage stager(const DenseRows::View&) { return NoStage{}; }
 __device__ __forceinline__ const SparseRows::View& stager(const SparseRows::View& v) { return v; }
+__device__ __forceinline__ const ShardRows::View& stager(const ShardRows::View& v) { return v; }
 
 // the staging area of the bounded-error kernels: their dynamic shared memory (the exact kernels place it after
 // their tiles); dense rows have none
@@ -186,6 +211,11 @@ template <class Src>
 __device__ __forceinline__ uint32_t* stage_smem() { return nullptr; }
 template <>
 __device__ __forceinline__ uint32_t* stage_smem<SparseRows>() {
+    extern __shared__ __align__(16) uint32_t sel_stage_smem[];
+    return sel_stage_smem;
+}
+template <>
+__device__ __forceinline__ uint32_t* stage_smem<ShardRows>() {
     extern __shared__ __align__(16) uint32_t sel_stage_smem[];
     return sel_stage_smem;
 }
@@ -235,12 +265,14 @@ __global__ void k_sel_sum(const Src src, const double* __restrict__ H, uint64_t 
         for (unsigned j = 0; j < nn; ++j) {
             __syncthreads();  // member j - 1 is in
             const unsigned r = j < n ? members[j] : (unsigned)extra_row;
-            const uint64_t at = src.bucket_at(r, b);
-            const uint32_t m = src.bucket_len(r, b);
+            unsigned pr = r;
+            const auto& d = src.part(pr);
+            const uint64_t at = d.bucket_at(pr, b);
+            const uint32_t m = d.bucket_len(pr, b);
             const FastDiv dv = make_fast_div((double)src.totals[r]);
             for (uint32_t e = threadIdx.x; e < m; e += blockDim.x) {
-                double* p = Sb + (src.idx[at + e] & (kSpLowBins - 1u));
-                *p = __dadd_rn(*p, div_exact((double)src.cnt[at + e], dv));
+                double* p = Sb + (d.idx[at + e] & (kSpLowBins - 1u));
+                *p = __dadd_rn(*p, div_exact((double)d.cnt[at + e], dv));
             }
         }
         if (b == 0 && threadIdx.x == 0) sum_scalars(H, members, n, extra_row, members_out, sc);
@@ -499,13 +531,79 @@ static int panic_error(const SelScal& h) {
     return DVS_ERR_VALUE;
 }
 
+// The record set of dvs_select_sparse_sharded on one rank (DESIGN.md §5.13).  The per-record scalars of ALL
+// records are gathered once per call and indexed by global (rank-major) row, as the kernels and read_flags expect.
+// The rows are this rank's own (`local`) plus a cache of peer rows: the members of the set and the candidate being
+// decided, copied in from their owner's window outbox.  `owned` (valid and held here) is the validity mask the
+// candidate scans and the grow filter see, so each rank scores exactly the candidates whose rows it holds.
+struct SparseShard {
+    dvs_comm* comm = nullptr;
+    const dvs_ksparse* local = nullptr;
+    uint32_t nrec = 0, nb = 0;
+    int k = 0;
+    uint64_t dim = 0;
+    std::vector<uint32_t> rank_base;  // [world + 1]: global row of each rank's first record
+    std::vector<uint64_t> lens;       // slots of every record's region (its byte length)
+    DevBuf<uint8_t> valid, err, owned;
+    DevBuf<double> err_total, entropy;
+    DevBuf<uint64_t> totals;
+    // member-row cache: slot s holds one peer row in entries [s * slot_len, (s + 1) * slot_len) and bucket tables
+    uint64_t slot_len = 0;
+    mutable DevBuf<uint32_t> c_idx, c_cnt, c_bp, c_nnz;  // (allocated by the call once it knows the set's size)
+    mutable DevBuf<uint64_t> c_off;
+    DevBuf<uint32_t> where;
+    uint64_t outbox = 0;  // heap offset of this rank's outbox in its window
+    // host bookkeeping, identical on every rank (each step is taken on all ranks with the same arguments)
+    mutable std::vector<uint32_t> h_where;
+    mutable std::vector<unsigned> refs;  // references to each row: members (a row may repeat) + the candidate
+    mutable std::vector<unsigned> free_slots;
+    mutable uint32_t fetched = 0;
+    mutable uint64_t fetched_bytes = 0;
+    unsigned owner_of(unsigned row) const {
+        return (unsigned)(std::upper_bound(rank_base.begin(), rank_base.end(), row) - rank_base.begin()) - 1u;
+    }
+};
+
+// byte layout of one row in an outbox
+struct ShardRowLayout {
+    uint64_t cnt, bp, nnz, bytes;
+};
+static uint64_t ss_align(uint64_t b) { return (b + 255) & ~255ull; }
+static ShardRowLayout shard_row_layout(uint64_t slot_len, uint32_t nb) {
+    ShardRowLayout L;
+    L.cnt = ss_align(slot_len * 4);
+    L.bp = 2 * L.cnt;
+    L.nnz = L.bp + ss_align((nb + 1ull) * 4);
+    L.bytes = std::max<uint64_t>(L.nnz + ss_align((uint64_t)nb * 4), 256);
+    return L;
+}
+// window bytes dvs_select_sparse_sharded needs (shard.window_bytes_for_sparse_select): control words + the larger
+// of the staging of the per-record scalars (8 bytes a record at most) and the outbox of one row
+static uint64_t shard_window_need(uint64_t nrec_total, uint64_t slot_len, uint32_t nb) {
+    return kCommCtrlBytes + std::max(std::max<uint64_t>(ss_align(nrec_total * 8), 256), shard_row_layout(slot_len, nb).bytes);
+}
+
 // the device row source of a record set, and the candidate rows k_sel_scan reads besides it
 inline DenseRows row_source(const dvs_kfreqs* f) { return DenseRows{f->freqs.p}; }
 inline SparseRows row_source(const dvs_ksparse* sp) {
-    return SparseRows{{sp->idx.p, sp->cnt.p, sp->bucket_ptr.p, sp->bucket_nnz.p, sp->offsets.p, sp->totals.p, sp->nb}};
+    return SparseRows{{{sp->idx.p, sp->cnt.p, sp->bucket_ptr.p, sp->bucket_nnz.p, sp->offsets.p, sp->totals.p, sp->nb}}};
+}
+inline ShardRows row_source(const SparseShard* s) {
+    const dvs_ksparse* l = s->local;
+    ShardRows r;
+    r.local = SparseRowsData{l->idx.p, l->cnt.p, l->bucket_ptr.p, l->bucket_nnz.p, l->offsets.p, l->totals.p, s->nb};
+    r.cache = SparseRowsData{s->c_idx.p, s->c_cnt.p, s->c_bp.p, s->c_nnz.p, s->c_off.p, nullptr, s->nb};
+    r.where = s->where.p;
+    r.totals = s->totals.p;
+    return r;
 }
 inline const double* cand_rows(const dvs_kfreqs* q) { return q->freqs.p; }
 inline const double* cand_rows(const dvs_ksparse*) { return nullptr; }
+inline const double* cand_rows(const SparseShard*) { return nullptr; }
+// the validity mask of the candidates this GPU scores
+inline const uint8_t* cand_valid(const dvs_kfreqs* q) { return q->valid.p; }
+inline const uint8_t* cand_valid(const dvs_ksparse* q) { return q->valid.p; }
+inline const uint8_t* cand_valid(const SparseShard* q) { return q->owned.p; }
 
 // The launches of the host-driven rounds over one record set: RS is dvs_kfreqs (dense rows) or dvs_ksparse.
 template <class RS>
@@ -552,7 +650,7 @@ struct Selector {
     // window; the caller resets them explicitly after an exact single-candidate scan)
     int scan_fast(SelState& s, const uint8_t* is_member, const unsigned* d_order, unsigned pos0, unsigned count) {
         k_sel_scan_fast<<<count, kFastThreads, stage_bytes<Src>(2), st>>>(rows(), f->entropy.p, dim, s.S(), s.members(),
-                                                                        s.sc.p, f->valid.p, is_member, d_order, pos0);
+                                                                        s.sc.p, cand_valid(f), is_member, d_order, pos0);
         DVS_LAUNCHED(ctx);
         return DVS_OK;
     }
@@ -597,7 +695,7 @@ struct Selector {
              unsigned count, double* delta_out) {
         DVS_TRY(reset_scan(s));  // re-arm the min-index reduction
         k_sel_scan<<<count, kEntThreads, kEntSmemBytes + stage_bytes<Src>(2), st>>>(
-            rows(), f->entropy.p, dim, s.S(), s.members(), s.sc.p, cand_rows(q), q->entropy.p, q->valid.p, is_member,
+            rows(), f->entropy.p, dim, s.S(), s.members(), s.sc.p, cand_rows(q), q->entropy.p, cand_valid(q), is_member,
             d_order, pos0, delta_out);
         DVS_LAUNCHED(ctx);
         return DVS_OK;
@@ -614,7 +712,12 @@ static int sparse_smem_setup() {
                           allow(k_sel_replace_update_fast<SparseRows>, 3 * kStageBytes),
                           allow(k_grow_eval<SparseRows>, 2 * kStageBytes), allow(k_sel_replace_vec<SparseRows>, 2 * kStageBytes),
                           allow(k_sel_update<SparseRows>, kEntSmemBytes + kStageBytes),
-                          allow(k_sel_scan<SparseRows>, kEntSmemBytes + 2 * kStageBytes)})
+                          allow(k_sel_scan<SparseRows>, kEntSmemBytes + 2 * kStageBytes),
+                          allow(k_sel_scan_fast<ShardRows>, 2 * kStageBytes), allow(k_sel_update_fast<ShardRows>, kStageBytes),
+                          allow(k_sel_replace_update_fast<ShardRows>, 3 * kStageBytes),
+                          allow(k_grow_eval<ShardRows>, 2 * kStageBytes), allow(k_sel_replace_vec<ShardRows>, 2 * kStageBytes),
+                          allow(k_sel_update<ShardRows>, kEntSmemBytes + kStageBytes),
+                          allow(k_sel_scan<ShardRows>, kEntSmemBytes + 2 * kStageBytes)})
         if (x != cudaSuccess && e == cudaSuccess) e = x;
     if (e != cudaSuccess) {
         set_error("dvs_select_sparse: shared memory for the staged rows: %s", cudaGetErrorString(e));
@@ -694,6 +797,141 @@ static int wait_counted(SelRun<RS>& r) {
     return DVS_OK;
 }
 
+// ---- dvs_select_sparse_sharded: rows stay with their owner (DESIGN.md §5.13) ------------------------------------
+// Every rank runs the same host loop over the same replicated state; these steps are taken on all ranks with the same
+// arguments, so the barriers and all-reduces below line up.
+template <class RS>
+constexpr bool kByOwner = std::is_same_v<RS, SparseShard>;
+constexpr const char* kShardName = "dvs_select_sparse_sharded";
+
+// device memory of the peer-row cache (cap + 1 slots) and of the gathered per-record scalars
+template <class RS>
+static uint64_t shard_bytes(const SelRun<RS>& r) {
+    if constexpr (kByOwner<RS>) {
+        const SparseShard& s = *r.f;
+        return (r.cap + 1ull) * (s.slot_len * 2 * sizeof(uint32_t) + (2ull * s.nb + 1) * sizeof(uint32_t) + sizeof(uint64_t)) +
+               (uint64_t)s.nrec * (3 * sizeof(uint8_t) + 3 * sizeof(double) + sizeof(uint32_t));
+    } else {
+        return 0;
+    }
+}
+
+// every rank returns the worst status of any rank (a CUDA failure before a bad argument before a value error); a
+// rank whose own status is the worst keeps its own message
+static int agree_status(dvs_ctx* ctx, dvs_comm* c, int rc) {
+    enum : uint32_t { kCuda = 0, kArg = 1, kValue = 2, kOk = 3 };
+    const uint32_t mine = rc == DVS_OK ? kOk : rc == DVS_ERR_VALUE ? kValue : rc == DVS_ERR_ARG ? kArg : kCuda;
+    uint32_t* h = reinterpret_cast<uint32_t*>(reinterpret_cast<char*>(ctx->pinned) + sizeof(SelScal) + 16);
+    DevBuf<uint32_t> d;
+    DVS_TRY(d.alloc(1));
+    *h = mine;
+    DVS_CUDA_TRY(cudaMemcpyAsync(d.p, h, sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+    DVS_TRY(comm_barrier(ctx, c));
+    DVS_TRY(comm_min_u32(ctx, c, d.p, d.p));
+    DVS_CUDA_TRY(cudaMemcpyAsync(h, d.p, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+    DVS_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    const uint32_t all = *h;
+    DVS_TRY(comm_check_error(ctx, c, kShardName));
+    if (all == kOk) return DVS_OK;
+    if (all != mine)
+        set_error("%s: the call failed on another rank (%s)", kShardName,
+                  all == kValue ? "value error" : all == kArg ? "bad argument" : "CUDA error");
+    return all == kValue ? DVS_ERR_VALUE : all == kArg ? DVS_ERR_ARG : DVS_ERR_CUDA;
+}
+
+// the scan results of this rank's candidates -> the first interesting positions over all ranks
+template <class RS>
+static int agree_scan(SelRun<RS>& r) {
+    if constexpr (kByOwner<RS>) {
+        char* sc = reinterpret_cast<char*>(r.cur->sc.p);
+        for (size_t off : {offsetof(SelScal, first_true), offsetof(SelScal, first_panic), offsetof(SelScal, first_unsure)}) {
+            uint32_t* w = reinterpret_cast<uint32_t*>(sc + off);
+            DVS_TRY(comm_min_u32(r.ctx, r.comm, w, w));
+        }
+    }
+    return DVS_OK;
+}
+
+// A row enters the state (a member of the initial set, a replacing candidate, a grow attempt).  Its owner copies it
+// into its window outbox; every other rank pulls it into a free cache slot (fetch and replicate).  The first barrier
+// means every rank has pulled the previous row, so the outbox may be overwritten; the second, that this row is in it.
+// A cache slot is written only by its own rank, on its stream, so every kernel that read the slot's previous row has
+// finished before the copy starts.
+template <class RS>
+static int take_row(SelRun<RS>& r, unsigned row) {
+    if constexpr (kByOwner<RS>) {
+        const SparseShard& s = *r.f;
+        if (s.refs[row]++ > 0) return DVS_OK;  // already here (a row that repeats in the set)
+        dvs_comm* c = s.comm;
+        const unsigned owner = s.owner_of(row), me = (unsigned)c->rank;
+        const uint64_t len = s.lens[row];
+        const uint32_t nb = s.nb;
+        const ShardRowLayout L = shard_row_layout(s.slot_len, nb);
+        cudaStream_t st = r.st;
+        DVS_TRY(comm_barrier(r.ctx, c));
+        if (owner == me) {
+            const dvs_ksparse* l = s.local;
+            const uint32_t lr = row - s.rank_base[me];
+            const uint64_t at = l->h_offsets[lr];
+            uint8_t* ob = c->window + s.outbox;
+            if (len) {
+                DVS_CUDA_TRY(cudaMemcpyAsync(ob, l->idx.p + at, len * 4, cudaMemcpyDeviceToDevice, st));
+                DVS_CUDA_TRY(cudaMemcpyAsync(ob + L.cnt, l->cnt.p + at, len * 4, cudaMemcpyDeviceToDevice, st));
+            }
+            DVS_CUDA_TRY(cudaMemcpyAsync(ob + L.bp, l->bucket_ptr.p + (size_t)lr * (nb + 1), (nb + 1ull) * 4,
+                                         cudaMemcpyDeviceToDevice, st));
+            DVS_CUDA_TRY(cudaMemcpyAsync(ob + L.nnz, l->bucket_nnz.p + (size_t)lr * nb, nb * 4ull, cudaMemcpyDeviceToDevice, st));
+        }
+        DVS_TRY(comm_barrier(r.ctx, c));
+        if (owner != me) {
+            if (s.free_slots.empty()) {
+                set_error("%s: no free slot in the row cache for record %u", kShardName, row);
+                return DVS_ERR_CUDA;
+            }
+            const unsigned slot = s.free_slots.back();
+            s.free_slots.pop_back();
+            const uint8_t* ob = c->peer[owner] + s.outbox;
+            if (len) {
+                DVS_CUDA_TRY(cudaMemcpyAsync(s.c_idx.p + slot * s.slot_len, ob, len * 4, cudaMemcpyDeviceToDevice, st));
+                DVS_CUDA_TRY(cudaMemcpyAsync(s.c_cnt.p + slot * s.slot_len, ob + L.cnt, len * 4, cudaMemcpyDeviceToDevice, st));
+            }
+            DVS_CUDA_TRY(cudaMemcpyAsync(s.c_bp.p + (size_t)slot * (nb + 1), ob + L.bp, (nb + 1ull) * 4,
+                                         cudaMemcpyDeviceToDevice, st));
+            DVS_CUDA_TRY(cudaMemcpyAsync(s.c_nnz.p + (size_t)slot * nb, ob + L.nnz, nb * 4ull, cudaMemcpyDeviceToDevice, st));
+            s.h_where[row] = kCachedRow | slot;
+            DVS_CUDA_TRY(cudaMemcpyAsync(s.where.p + row, &s.h_where[row], sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+            ++s.fetched;
+            s.fetched_bytes += len * 8 + (2ull * nb + 1) * 4;
+        }
+    }
+    return DVS_OK;
+}
+
+// a row leaves the state (the replaced lowest member, a discarded grow candidate): its slot is free once nothing
+// refers to it.  (where[] on the device keeps the old slot: a row that is neither member nor candidate is never read.)
+template <class RS>
+static void drop_row(SelRun<RS>& r, unsigned row) {
+    if constexpr (kByOwner<RS>) {
+        const SparseShard& s = *r.f;
+        if (--s.refs[row] > 0) return;
+        const uint32_t w = s.h_where[row];
+        if (w != kAbsentRow && (w & kCachedRow)) {
+            s.free_slots.push_back(w & ~kCachedRow);
+            s.h_where[row] = kAbsentRow;
+        }
+    }
+}
+
+// the row of member `j` of the current state
+template <class RS>
+static int member_row(SelRun<RS>& r, unsigned j, unsigned& row) {
+    unsigned* h = reinterpret_cast<unsigned*>(reinterpret_cast<char*>(r.ctx->pinned) + sizeof(SelScal) + 16);
+    DVS_CUDA_TRY(cudaMemcpyAsync(h, r.cur->members() + j, sizeof(unsigned), cudaMemcpyDeviceToHost, r.st));
+    DVS_CUDA_TRY(cudaStreamSynchronize(r.st));
+    row = *h;
+    return DVS_OK;
+}
+
 // reads the validity / panic flags of the records.  Every record in `order` goes through KmerSeq::new ->
 // entropy(), where a failing sum check panics: checked here for the positions below `upto`.
 template <class RS>
@@ -722,7 +960,8 @@ static int sparse_state_fits(SelRun<RS>& r) {
     const bool grow = r.grow_mode;
     const uint64_t per = 2 * (r.dim * sizeof(double) + (uint64_t)r.cap * (sizeof(unsigned) + 2 * sizeof(double)));
     const uint64_t need = per * (grow ? 3u : 1u) + (uint64_t)r.f->nrec + (uint64_t)r.num * sizeof(unsigned) +
-                          (grow ? (uint64_t)r.grow_window_max * r.cap * (sizeof(FastSum) + 2 * sizeof(double)) : 0u);
+                          (grow ? (uint64_t)r.grow_window_max * r.cap * (sizeof(FastSum) + 2 * sizeof(double)) : 0u) +
+                          shard_bytes(r);
     size_t free_b = 0, total_b = 0;
     DVS_CUDA_TRY(cudaMemGetInfo(&free_b, &total_b));
     uint64_t avail = free_b;
@@ -735,11 +974,38 @@ static int sparse_state_fits(SelRun<RS>& r) {
     }
     (void)cudaGetLastError();
     if (need + (64ull << 20) > avail) {
-        set_error("dvs_select_sparse: the selection state at k=%d needs %.1f MB of device memory (%s), %.1f MB are free",
+        set_error("dvs_select_sparse: the selection state at k=%d needs %.1f MB of device memory (%s%s), %.1f MB are free",
                   r.f->k, need / 1e6, grow ? "max: three double-buffered 4^k f64 sums" : "a double-buffered 4^k f64 sum",
-                  avail / 1e6);
+                  shard_bytes(r) ? ", the peer-row cache and every record's scalars" : "", avail / 1e6);
         return DVS_ERR_CUDA;
     }
+    return DVS_OK;
+}
+
+// after the argument checks: the memory check and the cache on every rank (all fail together), then the rows of the
+// initial set
+static int shard_prepare(SelRun<SparseShard>& r, const std::vector<unsigned>& init) {
+    const SparseShard& s = *r.f;
+    const unsigned slots = r.cap + 1;
+    int rc = sparse_state_fits(r);
+    if (rc == DVS_OK) rc = s.c_idx.alloc((size_t)slots * s.slot_len);
+    if (rc == DVS_OK) rc = s.c_cnt.alloc((size_t)slots * s.slot_len);
+    if (rc == DVS_OK) rc = s.c_bp.alloc((size_t)slots * (s.nb + 1));
+    if (rc == DVS_OK) rc = s.c_nnz.alloc((size_t)slots * s.nb);
+    if (rc == DVS_OK) rc = s.c_off.alloc(slots);
+    if (rc == DVS_OK) {
+        std::vector<uint64_t> off(slots);
+        for (unsigned q = 0; q < slots; ++q) off[q] = (uint64_t)q * s.slot_len;
+        if (cudaMemcpyAsync(s.c_off.p, off.data(), slots * sizeof(uint64_t), cudaMemcpyHostToDevice, r.st) != cudaSuccess ||
+            cudaStreamSynchronize(r.st) != cudaSuccess) {
+            set_error("%s: setting up the row cache failed", kShardName);
+            rc = DVS_ERR_CUDA;
+        }
+    }
+    s.free_slots.clear();
+    for (unsigned q = slots; q-- > 0;) s.free_slots.push_back(q);
+    DVS_TRY(agree_status(r.ctx, r.comm, rc));
+    for (unsigned row : init) DVS_TRY(take_row(r, row));
     return DVS_OK;
 }
 
@@ -818,7 +1084,8 @@ static int select_setup(SelRun<RS>& r) {
     const bool unbounded = r.grow_mode && r.max_size < (uint32_t)init.size();
     r.cap = (unbounded ? num : std::max<unsigned>(std::max(r.min_size, r.max_size), (unsigned)init.size())) + 1;
     r.n = (unsigned)init.size();
-    if constexpr (SelRun<RS>::Src::kSparse) DVS_TRY(sparse_state_fits(r));
+    if constexpr (kByOwner<RS>) DVS_TRY(shard_prepare(r, init));
+    else if constexpr (SelRun<RS>::Src::kSparse) DVS_TRY(sparse_state_fits(r));
     DVS_TRY(r.A.alloc(r.dim, r.cap));
     if (r.grow_mode) DVS_TRY(r.B.alloc(r.dim, r.cap));
     DVS_TRY(r.is_member.alloc(f->nrec));
@@ -833,6 +1100,7 @@ static int select_setup(SelRun<RS>& r) {
     r.sel = Selector<RS>{ctx, f, r.dim, r.st, (SelScal*)ctx->pinned};
     DVS_TRY(r.sel.build(*r.cur, r.d_init.p, r.n, -1));
     r.window_max = std::max(64u, (unsigned)ctx->sm_count * 12u);
+    if constexpr (kByOwner<RS>) r.window_max *= r.world;  // each rank scores its share of the window
     r.cursor = r.min_size;
     // DVS_SELECT_EXACT_ONLY=1 disables the bounded-error fast path (tests compare both)
     const char* exact_env = getenv("DVS_SELECT_EXACT_ONLY");
@@ -876,7 +1144,9 @@ static int select_setup(SelRun<RS>& r) {
     // keeps one host-driven attempt per candidate
     const char* gb_env = getenv("DVS_SELECT_GROW_BATCH");
     r.use_grow_batch = r.use_fast && r.grow_mode && !(gb_env && gb_env[0] == '0');
-    r.grow_window_max = 64 * r.world;
+    // (rows scored by their owner: the filter's windows stay those of one GPU, because where they end decides which
+    // candidates the filter hands to the host path, and with that the exact evaluations)
+    r.grow_window_max = kByOwner<RS> ? 64u : 64 * r.world;
     if (r.use_grow_batch && r.n != r.max_size) {
         DVS_TRY(r.fresh.alloc(r.dim, r.cap));
         DVS_TRY(r.d_gparts.alloc((size_t)r.grow_window_max * (r.cap + 3)));
@@ -910,18 +1180,20 @@ static int grow_filter(SelRun<RS>& r) {
     }
     const unsigned W = std::min(r.grow_window, r.num - cursor);
     DVS_CUDA_TRY(cudaMemsetAsync(r.d_ginteresting.p, 0xFF, sizeof(unsigned), r.st));
-    // candidate-sharded: this GPU evaluates the window candidates c with (cursor + c) % world == rank
-    const unsigned gc0 = (r.rank + world - cursor % world) % world;
-    const unsigned Wloc = W > gc0 ? (W - gc0 + world - 1) / world : 0;
+    // candidate-sharded: this GPU evaluates the window candidates c with (cursor + c) % world == rank; with rows kept
+    // by their owner, every candidate of the window whose row it holds (the mask cand_valid)
+    const unsigned cw = kByOwner<RS> ? 1u : world;
+    const unsigned gc0 = kByOwner<RS> ? 0u : (r.rank + world - cursor % world) % world;
+    const unsigned Wloc = W > gc0 ? (W - gc0 + cw - 1) / cw : 0;
     if (Wloc) {
         k_grow_eval<<<dim3(n + 3, Wloc), kFastThreads, stage_bytes<typename SelRun<RS>::Src>(2), r.st>>>(
-            r.sel.rows(), r.dim, cur->S(), cur->members(), cur->sc.p, r.fresh.S(), f->valid.p, r.is_member.p, r.d_order.p,
-            cursor, r.d_gparts.p, gc0, world);
+            r.sel.rows(), r.dim, cur->S(), cur->members(), cur->sc.p, r.fresh.S(), cand_valid(f), r.is_member.p, r.d_order.p,
+            cursor, r.d_gparts.p, gc0, cw);
         DVS_LAUNCHED(ctx);
         k_grow_decide<<<Wloc, kFastThreads, 0, r.st>>>(f->entropy.p, r.dim, cur->members(), cur->sc.p, r.fresh.sc.p,
-                                                       f->valid.p, r.is_member.p, r.d_order.p, cursor, r.d_gparts.p,
+                                                       cand_valid(f), r.is_member.p, r.d_order.p, cursor, r.d_gparts.p,
                                                        r.d_gmd.p, r.d_gmb.p, r.cap, r.d_gscratch.p, r.d_ginteresting.p,
-                                                       r.mode == DVS_MODE_MAX_COV ? 1 : 0, gc0, world);
+                                                       r.mode == DVS_MODE_MAX_COV ? 1 : 0, gc0, cw);
         DVS_LAUNCHED(ctx);
     }
     if (world > 1) DVS_TRY(comm_min_u32(ctx, r.comm, r.d_ginteresting.p, r.d_ginteresting.p));
@@ -1109,6 +1381,7 @@ static int host_window(SelRun<RS>& r, int& grow_row, SelScal& h) {
     unsigned pos = kNone;
     if (r.use_fast) {
         DVS_TRY(r.sel.scan_fast(*cur, r.is_member.p, r.d_order.p, r.cursor, count));
+        DVS_TRY(agree_scan(r));
         DVS_TRY(r.sel.read(*cur));
         h = *r.sel.h_sc;
         if (h.panic) return panic_error(h);
@@ -1123,7 +1396,8 @@ static int host_window(SelRun<RS>& r, int& grow_row, SelScal& h) {
             // an undecided candidate comes before the first certain acceptance: decide it exactly
             const unsigned pu = h.first_unsure;
             if (!h.exact) DVS_TRY(r.sel.update(*cur, r.n));
-            DVS_TRY(r.sel.scan(*cur, f, r.is_member.p, r.d_order.p, pu, 1, nullptr));
+            DVS_TRY(r.sel.scan(*cur, f, r.is_member.p, r.d_order.p, pu, 1, nullptr));  // (decided by its owner)
+            DVS_TRY(agree_scan(r));
             DVS_TRY(r.sel.read(*cur));
             h = *r.sel.h_sc;
             ++r.exact_evals;
@@ -1143,6 +1417,7 @@ static int host_window(SelRun<RS>& r, int& grow_row, SelScal& h) {
         }
     } else {
         DVS_TRY(r.sel.scan(*cur, f, r.is_member.p, r.d_order.p, r.cursor, count, nullptr));
+        DVS_TRY(agree_scan(r));
         DVS_TRY(r.sel.read(*cur));
         h = *r.sel.h_sc;
         if (h.panic) return panic_error(h);
@@ -1165,7 +1440,13 @@ static int host_window(SelRun<RS>& r, int& grow_row, SelScal& h) {
         grow_row = (int)row;
         return DVS_OK;
     }
+    unsigned low_row = 0;
+    if constexpr (kByOwner<RS>) {
+        DVS_TRY(take_row(r, row));
+        DVS_TRY(member_row(r, h.lowest, low_row));
+    }
     DVS_TRY(r.use_fast ? r.sel.replace_fast(*cur, r.n, row, r.is_member.p) : r.sel.replace(*cur, r.n, row, r.is_member.p));
+    drop_row(r, low_row);
     ++r.accepts;
     return DVS_OK;
 }
@@ -1185,6 +1466,11 @@ static int grow_attempt(SelRun<RS>& r, unsigned row, SelScal h) {
         DVS_CUDA_TRY(cudaStreamSynchronize(r.st));
         return DVS_OK;
     };
+    auto discard = [&]() -> int {
+        drop_row(r, row);
+        return r.sel.reset_scan(*r.cur);  // re-arm the min-index reduction of `cur`
+    };
+    DVS_TRY(take_row(r, row));
     if (r.use_fast && !h.state_unsure) {
         DVS_TRY(r.sel.build_fast(*r.alt, r.cur->members(), r.n, (int)row));
         DVS_TRY(r.sel.read(*r.alt));
@@ -1194,7 +1480,7 @@ static int grow_attempt(SelRun<RS>& r, unsigned row, SelScal h) {
             const double sa_f = use_cov ? h.cov : h.stdv, ba = h.exact ? 0.0 : (use_cov ? h.cov_bound : h.std_bound);
             const double sb_f = use_cov ? hf.cov : hf.stdv, bb = use_cov ? hf.cov_bound : hf.std_bound;
             if (sb_f - bb > sa_f + ba) return adopt();
-            if (sb_f + bb < sa_f - ba) return r.sel.reset_scan(*r.cur);  // candidate discarded
+            if (sb_f + bb < sa_f - ba) return discard();
         }
     }
     if (r.use_fast) ++r.exact_evals;
@@ -1211,7 +1497,7 @@ static int grow_attempt(SelRun<RS>& r, unsigned row, SelScal h) {
     const double sa = use_cov ? h.cov : h.stdv;
     const double sb = use_cov ? hb.cov : hb.stdv;
     if (sb > sa) return adopt();
-    return r.sel.reset_scan(*r.cur);  // candidate discarded: re-arm the min-index reduction of `cur`
+    return discard();
 }
 
 // the panic check of the records that were not published when a trailing selection started, the exact
@@ -1331,6 +1617,135 @@ int dvs_select_sparse(dvs_ctx* ctx, const dvs_ksparse* sp, const uint32_t* order
     return select_core(ctx, nullptr, sp, order, num, mode, min_size, max_size, sel_idx, sel_delta, stats5, size_out);
 }
 
+int dvs_select_sparse_sharded(dvs_ctx* ctx, dvs_comm* c, const dvs_ksparse* local, const uint32_t* nrec_per_rank,
+                              const uint32_t* order, uint32_t num, int mode, uint32_t min_size, uint32_t max_size,
+                              uint32_t* sel_idx, double* sel_delta, double* stats5, uint32_t* size_out) {
+    if (ctx) {
+        ctx->last_rows_fetched = 0;
+        ctx->last_bytes_fetched = 0;
+    }
+    if (!ctx || !c || !local || !nrec_per_rank || !c->connected) {
+        set_error("%s: bad argument / communicator not connected", kShardName);
+        return DVS_ERR_ARG;
+    }
+    if (c->world == 1)
+        return dvs_select_sparse(ctx, local, order, num, mode, min_size, max_size, sel_idx, sel_delta, stats5, size_out);
+    DVS_CUDA_TRY(dvs::enter(ctx));
+    cudaStream_t st = ctx->stream;
+    const int W = c->world, me = c->rank;
+    // 1. what every rank tells the others; the checks below see the same data everywhere, so all return the same status
+    struct Meta {
+        uint64_t nrec, k, has_entropy, max_len, npr[kCommMaxWorld];
+    };
+    std::vector<Meta> m(W);
+    {
+        Meta x;
+        memset(&x, 0, sizeof x);
+        x.nrec = local->nrec;
+        x.k = (uint64_t)local->k;
+        x.has_entropy = (local->has_entropy || local->nrec == 0) ? 1 : 0;  // (no records: no entropy pass to ask for)
+        for (uint32_t q = 0; q < local->nrec; ++q)
+            x.max_len = std::max(x.max_len, local->h_offsets[q + 1] - local->h_offsets[q]);
+        for (int q = 0; q < W; ++q) x.npr[q] = nrec_per_rank[q];
+        DevBuf<Meta> d_in, d_all;
+        DVS_TRY(d_in.alloc(1));
+        DVS_TRY(d_all.alloc(W));
+        DVS_CUDA_TRY(cudaMemcpyAsync(d_in.p, &x, sizeof x, cudaMemcpyHostToDevice, st));
+        std::vector<uint64_t> bytes(W, sizeof(Meta));
+        DVS_TRY(dvs_comm_allgatherv(ctx, c, d_in.p, bytes.data(), d_all.p));
+        DVS_CUDA_TRY(cudaMemcpyAsync(m.data(), d_all.p, W * sizeof(Meta), cudaMemcpyDeviceToHost, st));
+        DVS_CUDA_TRY(cudaStreamSynchronize(st));
+    }
+    SparseShard s;
+    s.comm = c;
+    s.local = local;
+    s.k = local->k;
+    s.dim = local->dim;
+    s.nb = local->nb;
+    s.rank_base.assign(W + 1, 0);
+    uint64_t n64 = 0;
+    for (int r = 0; r < W; ++r) {
+        if (!m[r].has_entropy) {
+            set_error("%s: rank %d counted its rows without entropies (dvs_count_kmers_sparse with want_entropy = 0)",
+                      kShardName, r);
+            return DVS_ERR_ARG;
+        }
+        if (m[r].k != m[0].k) {
+            set_error("%s: rank %d counted k=%llu, rank 0 k=%llu", kShardName, r, (unsigned long long)m[r].k,
+                      (unsigned long long)m[0].k);
+            return DVS_ERR_ARG;
+        }
+        for (int q = 0; q < W; ++q)
+            if (m[q].npr[r] != m[r].nrec) {
+                set_error("%s: rank %d passed nrec_per_rank[%d] = %llu, but rank %d holds %llu records", kShardName, q, r,
+                          (unsigned long long)m[q].npr[r], r, (unsigned long long)m[r].nrec);
+                return DVS_ERR_ARG;
+            }
+        s.rank_base[r] = (uint32_t)n64;
+        n64 += m[r].nrec;
+        s.slot_len = std::max(s.slot_len, m[r].max_len);
+    }
+    if (n64 >= (1ull << 31)) {
+        set_error("%s: %llu records are too many", kShardName, (unsigned long long)n64);
+        return DVS_ERR_ARG;
+    }
+    s.nrec = (uint32_t)n64;
+    s.rank_base[W] = s.nrec;
+    const uint64_t need = shard_window_need(s.nrec, s.slot_len, s.nb);
+    if (need > c->window_bytes) {
+        set_error("%s: the per-record scalars of %u records and the outbox of one row of up to %llu entries need a window "
+                  "of %llu bytes, the window has %llu (shard.window_bytes_for_sparse_select)",
+                  kShardName, s.nrec, (unsigned long long)s.slot_len, (unsigned long long)need,
+                  (unsigned long long)c->window_bytes);
+        return DVS_ERR_ARG;
+    }
+    // 2. the per-record scalars of every record, in rank-major order; the owned mask; where the rows live
+    {
+        const uint32_t nl = local->nrec, base = s.rank_base[me];
+        DVS_TRY(s.valid.alloc(s.nrec));
+        DVS_TRY(s.err.alloc(s.nrec));
+        DVS_TRY(s.owned.alloc(s.nrec));
+        DVS_TRY(s.err_total.alloc(s.nrec));
+        DVS_TRY(s.entropy.alloc(s.nrec));
+        DVS_TRY(s.totals.alloc(s.nrec));
+        DVS_TRY(s.where.alloc(s.nrec));
+        DevBuf<uint64_t> d_len, d_lens;
+        DVS_TRY(d_len.alloc(nl));
+        DVS_TRY(d_lens.alloc(s.nrec));
+        std::vector<uint64_t> len(nl);
+        for (uint32_t q = 0; q < nl; ++q) len[q] = local->h_offsets[q + 1] - local->h_offsets[q];
+        DVS_CUDA_TRY(cudaMemcpyAsync(d_len.p, len.data(), nl * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
+        std::vector<uint64_t> b1(W), b8(W);
+        for (int r = 0; r < W; ++r) {
+            b1[r] = m[r].nrec;
+            b8[r] = m[r].nrec * 8;
+        }
+        DVS_TRY(dvs_comm_allgatherv(ctx, c, local->valid.p, b1.data(), s.valid.p));
+        DVS_TRY(dvs_comm_allgatherv(ctx, c, local->err.p, b1.data(), s.err.p));
+        DVS_TRY(dvs_comm_allgatherv(ctx, c, local->err_total.p, b8.data(), s.err_total.p));
+        DVS_TRY(dvs_comm_allgatherv(ctx, c, local->entropy.p, b8.data(), s.entropy.p));
+        DVS_TRY(dvs_comm_allgatherv(ctx, c, local->totals.p, b8.data(), s.totals.p));
+        DVS_TRY(dvs_comm_allgatherv(ctx, c, d_len.p, b8.data(), d_lens.p));
+        s.lens.resize(s.nrec);
+        DVS_CUDA_TRY(cudaMemcpyAsync(s.lens.data(), d_lens.p, s.nrec * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+        DVS_CUDA_TRY(cudaMemsetAsync(s.owned.p, 0, s.nrec, st));
+        if (nl) DVS_CUDA_TRY(cudaMemcpyAsync(s.owned.p + base, local->valid.p, nl, cudaMemcpyDeviceToDevice, st));
+        s.h_where.assign(s.nrec, kAbsentRow);
+        for (uint32_t q = 0; q < nl; ++q) s.h_where[base + q] = q;
+        DVS_CUDA_TRY(cudaMemcpyAsync(s.where.p, s.h_where.data(), s.nrec * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+        DVS_CUDA_TRY(cudaStreamSynchronize(st));
+        s.refs.assign(s.nrec, 0);
+    }
+    // 3. the outbox (symmetric heap: the same size on every rank), the selection, the status of all ranks
+    DVS_TRY(comm_heap_alloc(c, shard_row_layout(s.slot_len, s.nb).bytes, &s.outbox));
+    const int rc = select_core(ctx, c, &s, order, num, mode, min_size, max_size, sel_idx, sel_delta, stats5, size_out);
+    ctx->last_rows_fetched = s.fetched;
+    ctx->last_bytes_fetched = s.fetched_bytes;
+    const int all = agree_status(ctx, c, rc);  // (also: no rank still pulls from an outbox)
+    comm_heap_free(c, s.outbox);
+    return all;
+}
+
 int dvs_debug_fast_terms(dvs_ctx* ctx, const double* a, const double* b, double* m, double* l, int32_t* special,
                          uint64_t n) {
     if (n == 0) return DVS_OK;
@@ -1355,6 +1770,8 @@ int dvs_debug_fast_terms(dvs_ctx* ctx, const double* a, const double* b, double*
 
 uint32_t dvs_select_last_accepts(dvs_ctx* ctx) { return ctx->last_accepts; }
 uint32_t dvs_select_last_exact_evals(dvs_ctx* ctx) { return ctx->last_exact_evals; }
+uint32_t dvs_select_last_rows_fetched(dvs_ctx* ctx) { return ctx->last_rows_fetched; }
+uint64_t dvs_select_last_bytes_fetched(dvs_ctx* ctx) { return ctx->last_bytes_fetched; }
 uint32_t dvs_select_last_trail_accepts(dvs_ctx* ctx) { return ctx->last_trail_accepts; }
 uint32_t dvs_select_last_trail_launches(dvs_ctx* ctx) { return ctx->last_trail_launches; }
 uint32_t dvs_select_last_trail_sms(dvs_ctx* ctx) { return ctx->last_trail_launches ? ctx->last_trail_sms : 0; }

@@ -13,6 +13,8 @@ library's own peer windows (include/dvs_b200.h, dvs_comm_*): no NCCL and no torc
   mash, 128 x 128 tiles for Euclid) and every kernel stores its results straight into every peer's copy
   of the matrix.  Sparse k-mer rows (k = 9..12) are not gathered: each rank keeps its own and copies one peer's
   at a time (`sharded_euclidean_sparse`).
+* nmost / max from sparse rows (k = 10..12): `select_sparse_sharded`.  Each rank keeps its own rows and scores the
+  candidates it holds; only rows that enter the set (and `max`'s grow candidates) are copied to the other ranks.
 
 The only host-side exchange is the rendezvous below (window handles and a few integers over TCP on
 MASTER_ADDR:MASTER_PORT+1, or in-process for ranks that are threads of one process).
@@ -190,6 +192,18 @@ def window_bytes_for_sparse(nrec_per_rank, bases_per_rank, k: int, extra: int = 
     return 64 * 1024 + stage + max(align(n * n * 8), 256) + int(extra)
 
 
+def window_bytes_for_sparse_select(max_record_len: int, k: int, nrec_total: int, extra: int = 0) -> int:
+    """the window `select_sparse_sharded` needs (the formula dvs_select_sparse_sharded checks): control words and the
+    larger of the staging of the per-record scalars (8 bytes a record) and the outbox of one row - one slot per byte of
+    the longest record of any rank, so known before counting - plus `extra` bytes of other objects.  The member-row
+    cache is ordinary device memory, not window memory, so the size of the set does not enter."""
+    def align(b):
+        return (int(b) + 255) // 256 * 256
+    nb = 4 ** (int(k) - 6)  # buckets per record (csrc/sparse.cu)
+    outbox = max(2 * align(int(max_record_len) * 4) + align((nb + 1) * 4) + align(nb * 4), 256)
+    return 64 * 1024 + max(align(int(nrec_total) * 8), 256, outbox) + int(extra)
+
+
 # --------------------------------------------------------------------------------- counting ----
 def count_sharded(ctx, comm, seqset_local, k: int, num_states: int = 4):
     """(kfreqs with the rows of ALL ranks in rank-major order, records per rank)"""
@@ -216,6 +230,18 @@ def interleaved_order(local_orders, nrec_per_rank) -> np.ndarray:
 def select_sharded(ctx, comm, kf_all, order, mode: int, min_size: int, max_size: int = 0):
     """single-pass selection over all rows, candidate-sharded (identical result on every rank)"""
     return kf_all.select_sharded(comm, order, mode, min_size, max_size)
+
+
+def select_sparse_sharded(ctx, comm, ks_local, order, mode: int, min_size: int, max_size: int = 0):
+    """single-pass nmost / max over the sparse rows of all ranks, each rank passing its own (KSparse.count with
+    want_entropy=True): identical result on every rank, bitwise KSparse.select over the union of the records.
+
+    `order` indexes the rank-major rows of all ranks.  Any placement of the records gives the same result; the one that
+    balances the work deals the shuffled seqids round-robin - rank r takes positions r, r + W, ... of the shuffled list,
+    in that order - and rebuilds the global order with `interleaved_order(local orders, nrec)`, so that every window of
+    candidates falls evenly on the ranks.  The window: `window_bytes_for_sparse_select`."""
+    nrec = comm.rv.allgather(int(ks_local.nrec))
+    return ks_local.select_sharded(comm, nrec, order, mode, min_size, max_size)
 
 
 def chunked_select(ctx, comm, kf_local, local_order, mode: int, min_size: int, max_size: int):

@@ -350,6 +350,28 @@ int dvs_euclid_distances_sparse_sharded(dvs_ctx* ctx, dvs_comm* c, const dvs_ksp
 int dvs_select_sharded(dvs_ctx* ctx, dvs_comm* c, const dvs_kfreqs* f_all, const uint32_t* order, uint32_t num,
                        int mode, uint32_t min_size, uint32_t max_size, uint32_t* sel_idx, double* sel_delta,
                        double* stats5, uint32_t* size_out);
+/* dvs_select_sparse over the sparse rows of ALL ranks, each rank keeping its own (DESIGN.md §5.13).  Collective.
+ * Each rank passes ITS OWN dvs_count_kmers_sparse result (want_entropy != 0); global rows are rank-major, as in
+ * dvs_euclid_distances_sparse_sharded, and `order` indexes them.  Every rank passes the same order and arguments and
+ * receives the same result: bit for bit dvs_select_sparse over the union of the records (sel_idx, sel_delta, stats5,
+ * size, and dvs_select_last_accepts / dvs_select_last_exact_evals), with the reference's single-pass semantics
+ * (numprocs = 1).  The per-record scalars of all records are gathered once; a candidate is scored only by the rank
+ * that holds its row, and the first interesting position is all-reduced.  A row that enters the set (initial members,
+ * an accepted candidate, a grow attempt of `max`) is copied to every other rank's member-row cache through its
+ * owner's window outbox; all ranks then decide identically.  A rank therefore holds, besides its own rows, only the
+ * members' and the candidate's.  The window must hold the larger of 8 bytes per record and one row's outbox
+ * (shard.window_bytes_for_sparse_select).  Errors: the value errors of dvs_select_sparse, with its texts; rows counted
+ * without entropies on any rank, a different k on some rank, an nrec_per_rank that disagrees with any rank's records
+ * or a window too small for the call are DVS_ERR_ARG on every rank; the memory check of dvs_select_sparse includes the
+ * cache.  When ranks fail differently, all return the worst class (DVS_ERR_CUDA before DVS_ERR_ARG before
+ * DVS_ERR_VALUE).  With world == 1 this is dvs_select_sparse. */
+int dvs_select_sparse_sharded(dvs_ctx* ctx, dvs_comm* c, const dvs_ksparse* local, const uint32_t* nrec_per_rank,
+                              const uint32_t* order, uint32_t num, int mode, uint32_t min_size, uint32_t max_size,
+                              uint32_t* sel_idx, double* sel_delta, double* stats5, uint32_t* size_out);
+/* rows this rank copied in from peers during the last dvs_select_sparse_sharded on this ctx, and their bytes (0 with
+ * one rank) */
+uint32_t dvs_select_last_rows_fetched(dvs_ctx* ctx);
+uint64_t dvs_select_last_bytes_fetched(dvs_ctx* ctx);
 
 /* dvs_count_kmers + dvs_select in one call with the two OVERLAPPED on one GPU (the `dvs prep` -> `dvs nmost` flow of
  * BASELINE.json configs[1]; reference: src/lib.rs nmost() over the records src/record.rs KmerSeq::new builds).
